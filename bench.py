@@ -15,7 +15,9 @@ before the closing timestamp.
     python bench.py --gpus 1 --steps K --warmup W          # our arm
     python bench.py --impl reference ...                   # the reference's own CPU code path
 
-A "step" is one pass of the hot path over one query batch.  Prints ONE JSON line (rank 0).
+A "step" is one pass of the hot path over one query batch.  Prints ONE JSON line (rank 0).  ``--dump-outputs DIR``
+also writes the scores and ids of the last timed step as .npy files; the inputs depend only on the arguments, so two
+builds run with the same arguments can be compared output for output.
 
 Reference arm: the reference's OWN batched entry point, ``core.FAISSRetriever.build_index`` + ``.search``
 (core.py:758-930), imported unmodified from ``oracle/_ref`` (tools/make_ref.py) and run on every host core of
@@ -59,6 +61,7 @@ GEN_CHUNK = 500_000              # rows generated per step; shard boundaries are
 N_CENTRES = 4096
 CHECK_QUERIES = 256              # queries verified against an exact fp32 scan of the whole DB
 TOL = 1e-3                       # north_star: ids identical except ties within 1e-3 of the k-th score
+DUMP_BYTES = 64 << 20            # --dump-outputs: at most this much on disk
 
 
 def parse_args():
@@ -83,7 +86,16 @@ def parse_args():
                    help="N > 1: fraction of a shard every rank also stores from either neighbour (elastic boundaries)")
     p.add_argument("--no-extras", action="store_true",
                    help="skip the informational legs (BASELINE configs A, B, C, the production-shaped cell)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the top-k of the last timed step to DIR: scores.npy (float32 [m,k]), ids.npy (float64 "
+                        "[m,k]) and query_rows.npy (float64 [m], the query of each row; a fixed sample when all nq "
+                        "rows would exceed 64 MB)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def workload_config(args):
@@ -320,6 +332,20 @@ def time_host(fn, reps=20, warm=3):
     for _ in range(reps):
         fn()
     return (time.perf_counter() - t0) / reps
+
+
+def dump_outputs(out_dir, D, I):
+    """Writes what a caller of the timed path receives -- scores [nq,k] and global row ids [nq,k] -- so that two builds
+    can be compared output for output.  Ids go out as float64 (exact below 2**53).  When every query row would not
+    fit in DUMP_BYTES, a sample of query rows drawn with a fixed seed is written instead."""
+    D, I = D.cpu().numpy(), I.cpu().numpy()
+    nq, k = D.shape
+    m = min(nq, (DUMP_BYTES - 4096) // (4 * k + 8 * k + 8))          # 4 KB: room for the three .npy headers
+    rows = np.arange(nq) if m == nq else np.sort(np.random.default_rng(0).choice(nq, m, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), D[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "ids.npy"), I[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
 
 
 def run_extras(args, dev, peaks):
@@ -595,18 +621,19 @@ def run_ours(args):
     def run_steps(n):
         """n searches back to back.  Sharded: two in flight -- the exchange + merge of search i run on the index's
         side stream while search i+1 is being scored (ShardedFlatIP.search_async); every result is complete and
-        ordered into the timing stream before the closing event."""
+        ordered into the timing stream before the closing event.  Returns the (D, I) of the last search."""
+        out = None
         if not index:
             for _ in range(n):
-                local.search_tensor(q_dev, k)
-            return
+                out = local.search_tensor(q_dev, k)
+            return out
         prev = None
         for _ in range(n):
             h = index.search_async(q_dev, k)
             if prev is not None:
                 prev.result(copy=False)
             prev = h
-        prev.result(copy=False)
+        return prev.result(copy=False)
 
     def barrier():
         if world > 1:
@@ -637,10 +664,13 @@ def run_ours(args):
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    run_steps(args.steps)
+    last = run_steps(args.steps)
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                          # before later searches can reuse the result buffers
+        dump_outputs(args.dump_outputs, *last)
+    del last
     ms_total = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms_total, op=dist.ReduceOp.MAX)

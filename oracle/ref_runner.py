@@ -7,8 +7,6 @@ under them is whatever the caller injects:
 * ``oracle.flat_ip_mt.faiss_module()``  -> the reference's CPU path (bench.py ``--impl reference`` / ``cpu_baseline``):
   FAISS itself is an un-vendored, absent dependency, so the flat search UNDER the reference's wrappers is the
   oracle's multi-threaded restatement of its contract; everything above it is reference code.
-* ``ivr_b200.faiss_compat``             -> the drop-in proof (tests/test_dropin_gpu.py): the same unmodified
-  classes running on the B200 kernels.
 
 Reference constructors read ``utils.Config`` / create log directories; the objects are therefore assembled the
 way tests/golden/make_golden.py does it (``__new__`` + the attributes ``__init__`` would set: core.py:700-734).

@@ -4,8 +4,7 @@ TEST / BENCH INFRASTRUCTURE ONLY.  Used by tests/golden/make_golden*.py to produ
 vectors from the unmodified reference at /root/reference, and -- through the byte-for-byte,
 git-ignored copy ``oracle/_ref`` that tools/make_ref.py makes at build time and that travels
 to the GPU box with the snapshot -- by ``bench.py``'s CPU arm (the reference's own wrappers
-and filter.py timed on the host cores) and by tests/test_dropin_gpu.py (the reference's own
-classes running on top of ``faiss_compat``).  No reference source enters the git history.
+and filter.py timed on the host cores).  No reference source enters the git history.
 
 What is shimmed and why (SURVEY.md section 0, fact 4):
   * ``transformers``  -- filter.py:46-48 calls ``from_pretrained`` at import

@@ -3,6 +3,8 @@ loudly (no CPU fallback) when there is no GPU."""
 import ctypes
 import os
 import re
+import shutil
+import subprocess
 
 import numpy as np
 import pytest
@@ -27,11 +29,21 @@ def test_header_and_library_agree():
     assert sorted(nat.PROTOTYPES) == syms, "ctypes PROTOTYPES out of sync with the header"
 
 
+def _cuobjdump():
+    """cuobjdump on PATH, else next to the nvcc the library was built with (NVCC, as in __graft_entry__.build())."""
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    for cand in (shutil.which("cuobjdump"), os.path.join(os.path.dirname(nvcc), "cuobjdump")):
+        if cand and os.access(cand, os.X_OK):
+            return cand
+    return None
+
+
 def test_library_is_sm100a_native():
     """The .so carries sm_100a SASS (no PTX-JIT for other archs, no multi-backend)."""
-    out = os.popen(f"cuobjdump -lelf '{nat.LIB_PATH}' 2>/dev/null").read()
-    if not out:
+    tool = _cuobjdump()
+    if tool is None:
         pytest.skip("cuobjdump not available")
+    out = subprocess.run([tool, "-lelf", nat.LIB_PATH], capture_output=True, text=True, check=True).stdout
     assert "sm_100a" in out
     assert not re.search(r"sm_(7|8|9)\d", out)
 

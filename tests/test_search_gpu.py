@@ -488,6 +488,8 @@ def test_wrappers_against_reference_golden(search_golden):
     ref.add(sg["xb"])
     for key, want in sg["results"]["search_vectors"].items():
         if key == "k20_q0_even":
+            got = u.search_vectors(sg["xq"][0], k=20, filter_func=lambda m: m["frame_id"] % 2 == 0)
+            assert all(g["metadata"]["frame_id"] % 2 == 0 for g in got) and abs(len(got) - len(want)) <= 1
             continue
         k, q = key.split("_")
         k, qi = int(k[1:]), int(q[1:])
@@ -502,11 +504,14 @@ def test_wrappers_against_reference_golden(search_golden):
         assert not bad, (key, bad)
         for g in got:
             assert g["metadata"] is sg["meta"][g["index"]]
+    assert u.faiss_index.last_timing()["path"] in ("stream", "mma")    # it really ran on the device
     b = ivr_b200.UnifiedBuilderIntegration(system=None)
     b.unified_index = u
     for key, want in sg["results"]["search_unified_fast"].items():
         got = b.search_unified_fast(sg["xq"][1], k=30, similarity_threshold=float(key[3:]))
         assert abs(len(got) - len(want)) <= 1                               # threshold on 1-ip, 1e-3 band
+        for g, w in zip(got, want):
+            assert abs(g["similarity_score"] - w[1]) < 2 * TOL
         for g in got:
             assert g["similarity_score"] >= float(key[3:]) and g["temporal_context"] == []
             assert type(g["metadata"]).__name__ == "KeyframeMetadata"
@@ -552,6 +557,7 @@ def test_faiss_retriever_on_gpu(search_golden):
            for i, m in enumerate(sg["meta"])]
     fr = ivr_b200.FAISSRetriever()
     fr.build_index(raw, kms, validate_consistency=False)
+    assert fr.index.ntotal == sg["results"]["ntotal"]
     out = fr.search(sg["xq"][:3] * np.float32(1.7), k=12)
     want = sg["results"]["faiss_retriever_search"]
     assert len(out) == len(want) == 36
@@ -564,6 +570,13 @@ def test_faiss_retriever_on_gpu(search_golden):
         assert len(common) >= 11
         for key in common:
             assert abs(g[key] - w[key]) < 1e-6
+    one = fr.search(sg["xq"][4], k=5)
+    assert [(r.metadata.folder_name, r.metadata.image_name, r.rank) for r in one] == \
+        [(w[0], w[1], w[3]) for w in sg["results"]["faiss_retriever_search_1d"]]
+    by_id = sg["results"]["faiss_retriever_search_by_id"]
+    hits = fr.search_by_id(by_id["key"], k=7)
+    assert [(r.metadata.folder_name, r.metadata.image_name) for r in hits][:1] == [tuple(by_id["hits"][0][:2])]
+    assert len(hits) == len(by_id["hits"])
 
 
 def test_similarity_relationships_vs_oracle():

@@ -1,4 +1,4 @@
-"""Recipe for ``oracle/_ref/``: an UNMODIFIED copy of the reference files the CPU baseline and the drop-in tests run.
+"""Recipe for ``oracle/_ref/``: an UNMODIFIED copy of the reference files the CPU baseline runs.
 
     python tools/make_ref.py            (called by __graft_entry__.build() whenever /root/reference is present)
 
@@ -6,12 +6,11 @@ Why a copy: the reference is pure Python (nothing to compile) and has no setup.p
 --target baseline/_ref /root/reference`` fails: "neither 'setup.py' nor 'pyproject.toml' found"), yet
 ``/root/reference`` does not exist on the GPU box.  ``oracle/_ref/`` is git-ignored (it never enters the history)
 but not gpurun-ignored, so it travels with the snapshot exactly like the built ``.so``.  Files are copied byte for
-byte; ``MANIFEST.json`` records their SHA-256 so a test can prove nothing was edited.
+byte; ``MANIFEST.json`` records their SHA-256.
 
 TEST / BENCH INFRASTRUCTURE ONLY: the product never imports anything from here.  Consumers:
 ``bench.py --impl reference`` and ``cpu_baseline`` (the reference's own FAISSRetriever / UnifiedIndex / filter.py
-code timed on the host cores), and ``tests/test_dropin_gpu.py`` (the reference's own wrappers running on top of
-``faiss_compat`` on a B200).
+code timed on the host cores).
 """
 from __future__ import annotations
 
