@@ -105,6 +105,23 @@ IVR_API int ivr_index_search_device(ivr_index* idx, const float* q_dev, int64_t 
 IVR_API int ivr_index_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, int k,
                                  uint64_t* keys_dev, int64_t id_offset, int path, void* stream);
 
+/* Replaces lims, D, I = index.range_search(x, radius) of faiss.IndexFlatIP (not called by the reference): every
+ * stored row whose inner product with the query is strictly greater than `radius`.
+ *   lims   int64   [nq + 1]  the hits of query i are D[lims[i] : lims[i+1]], I[lims[i] : lims[i+1]]
+ *   D      float32 [capacity] scores, descending within a query (ties -> lower id)
+ *   I      int64   [capacity] row ids + id_offset
+ * lims always receives nq + 1 entries.  When lims[nq] > capacity only lims[nq] (the exact total) is meaningful and
+ * D / I are untouched: retry with capacity >= lims[nq] (the max_hits convention of ivr_sequence_similarity).
+ * Scores, ids and the search window are those of ivr_index_search.  A NaN radius is IVR_EINVAL; capacity above
+ * 2^31-1, padded dim above 4096 and indexes of 2^32 rows or more are IVR_EUNSUPPORTED.  The device variant never
+ * blocks the host; its scratch grows the handle's workspace by about 28 bytes per capacity entry.  The host variant
+ * stages through the handle's pinned buffer. */
+IVR_API int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, float radius, int64_t capacity,
+                                   int64_t* lims_host, float* D_host, int64_t* I_host);
+IVR_API int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius,
+                                          int64_t capacity, int64_t* lims_dev, float* D_dev, int64_t* I_dev,
+                                          int64_t id_offset, void* stream);
+
 /* Search window: until cleared (count < 0) every search on this handle scores only the stored rows
  * [first, first + count) -- ids are still "stored row + id_offset", k > count pads as usual, a window reaching beyond
  * ntotal fails the search with IVR_EINVAL.  No data moves: this is how a row shard that also holds a replica of its

@@ -2,6 +2,7 @@
 #include "index.cuh"
 
 #include <algorithm>
+#include <climits>
 #include <cstdarg>
 #include <cstring>
 #include <new>
@@ -379,6 +380,26 @@ struct RowWindow {
     ~RowWindow() { idx->rows = rows; idx->ntotal = ntotal; idx->capacity = capacity; }
 };
 
+// The preamble of every query over the stored rows: runs body(id_offset) on the rows of the handle's search window
+// (ivr_index_set_window; ids stay "stored row + id_offset") after the rows added on other streams.  `who` prefixes
+// the error message.
+template <class Body>
+static int with_search_window(ivr_index* idx, int64_t id_offset, cudaStream_t st, const char* who, Body&& body) {
+    if (idx->win_count >= 0) {
+        if (idx->win_first + idx->win_count > idx->ntotal) {
+            set_error("%s: the window [%lld, +%lld) reaches beyond the %lld rows of the index", who,
+                      static_cast<long long>(idx->win_first), static_cast<long long>(idx->win_count),
+                      static_cast<long long>(idx->ntotal));
+            return IVR_EINVAL;
+        }
+        id_offset += idx->win_first;
+    }
+    RowWindow window(idx);
+    IVR_CUDA(cudaSetDevice(idx->device));
+    if (idx->rows_ready_set) IVR_CUDA(cudaStreamWaitEvent(st, idx->rows_ready, 0));   // rows added on another stream
+    return body(id_offset);
+}
+
 // D_dev == nullptr selects the packed-key output: I_dev then receives uint64 keys [nq, k]
 // (order_preserving(score) << 32 | ~(row + id_offset), 0 = padding) instead of int64 ids.
 static int search_device_impl(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,
@@ -386,36 +407,56 @@ static int search_device_impl(ivr_index* idx, const float* q_dev, int64_t nq, in
     if (k <= 0) { set_error("search: k must be positive (got %d)", k); return IVR_EINVAL; }
     if (k > IVR_MAX_K) { set_error("search: k=%d exceeds IVR_MAX_K=%d", k, IVR_MAX_K); return IVR_EUNSUPPORTED; }
     if (nq == 0) return IVR_OK;
-    if (idx->win_count >= 0) {
-        if (idx->win_first + idx->win_count > idx->ntotal) {
-            set_error("search: the window [%lld, +%lld) reaches beyond the %lld rows of the index",
-                      static_cast<long long>(idx->win_first), static_cast<long long>(idx->win_count),
-                      static_cast<long long>(idx->ntotal));
-            return IVR_EINVAL;
+    return with_search_window(idx, id_offset, st, "search", [&](int64_t id_offset) {
+        idx->launches[0] = idx->launches[1] = idx->launches[2] = 0;
+        idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = false;
+        if (idx->ntotal == 0) {
+            const int64_t n = nq * k;
+            fill_empty_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(D_dev, I_dev, n);
+            IVR_CUDA(cudaGetLastError());
+            idx->last_path = 0;
+            return IVR_OK;
         }
-        id_offset += idx->win_first;                 // ids stay "stored row + id_offset"
+        const int use = choose_path(idx, nq, k, path);
+        if (use < 0) return use;
+        if (use == IVR_PATH_MMA) {
+            idx->last_path = IVR_PATH_MMA;
+            return search_mma(idx, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+        }
+        idx->last_path = IVR_PATH_STREAM;
+        idx->last_kernel = "search_stream_kernel";
+        return search_stream(idx, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+    });
+}
+
+// Checks of ivr_index_range_search*(), in an order that needs no device.
+static int range_args(const ivr_index* idx, const void* q, int64_t nq, float radius, int64_t capacity,
+                      const void* lims, const void* D, const void* I) {
+    if (nq < 0) { set_error("range_search: nq must be >= 0 (got %lld)", static_cast<long long>(nq)); return IVR_EINVAL; }
+    if (capacity < 0) {
+        set_error("range_search: capacity must be >= 0 (got %lld)", static_cast<long long>(capacity));
+        return IVR_EINVAL;
     }
-    RowWindow window(idx);
-    IVR_CUDA(cudaSetDevice(idx->device));
-    if (idx->rows_ready_set) IVR_CUDA(cudaStreamWaitEvent(st, idx->rows_ready, 0));   // rows added on another stream
-    idx->launches[0] = idx->launches[1] = idx->launches[2] = 0;
-    idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = false;
-    if (idx->ntotal == 0) {
-        const int64_t n = nq * k;
-        fill_empty_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(D_dev, I_dev, n);
-        IVR_CUDA(cudaGetLastError());
-        idx->last_path = 0;
-        return IVR_OK;
+    if (radius != radius) { set_error("range_search: radius is NaN"); return IVR_EINVAL; }
+    if (!idx || !lims || (nq > 0 && !q) || (capacity > 0 && (!D || !I))) {
+        set_error("range_search: bad argument (NULL index or buffer)");
+        return IVR_EINVAL;
     }
-    const int use = choose_path(idx, nq, k, path);
-    if (use < 0) return use;
-    if (use == IVR_PATH_MMA) {
-        idx->last_path = IVR_PATH_MMA;
-        return search_mma(idx, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+    if (capacity > INT_MAX || nq >= INT_MAX) {
+        set_error("range_search: at most 2^31-1 hits and queries per call (capacity %lld, nq %lld)",
+                  static_cast<long long>(capacity), static_cast<long long>(nq));
+        return IVR_EUNSUPPORTED;
     }
-    idx->last_path = IVR_PATH_STREAM;
-    idx->last_kernel = "search_stream_kernel";
-    return search_stream(idx, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+    if (small_range_chunk(idx) < 16) {
+        set_error("range_search: dim %d is wider than the small-batch kernel holds (padded dim <= 4096)", idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    if (idx->ntotal >= (1ll << 32)) {
+        set_error("range_search: the hit key holds a 32-bit row; the index has %lld rows",
+                  static_cast<long long>(idx->ntotal));
+        return IVR_EUNSUPPORTED;
+    }
+    return IVR_OK;
 }
 
 }  // namespace ivr
@@ -477,6 +518,58 @@ int ivr_index_search(ivr_index* idx, const float* q_host, int64_t nq, int k, flo
     IVR_CUDA(cudaStreamSynchronize(st));
     memcpy(D_host, pin + up(qb), db);
     memcpy(I_host, pin + up(qb) + up(db), ib);
+    return IVR_OK;
+}
+
+int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                                  int64_t* lims_dev, float* D_dev, int64_t* I_dev, int64_t id_offset, void* stream) {
+    IVR_TRY(range_args(idx, q_dev, nq, radius, capacity, lims_dev, D_dev, I_dev));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);       // NULL = the legacy default stream, as in CUDA
+    if (nq == 0) {
+        IVR_CUDA(cudaSetDevice(idx->device));
+        IVR_CUDA(cudaMemsetAsync(lims_dev, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return with_search_window(idx, id_offset, st, "range_search", [&](int64_t id_offset) {
+        return range_search_device(idx, q_dev, nq, radius, capacity, lims_dev, D_dev, I_dev, id_offset, st);
+    });
+}
+
+int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, float radius, int64_t capacity,
+                           int64_t* lims_host, float* D_host, int64_t* I_host) {
+    IVR_TRY(range_args(idx, q_host, nq, radius, capacity, lims_host, D_host, I_host));
+    if (nq == 0) { lims_host[0] = 0; return IVR_OK; }
+    IVR_CUDA(cudaSetDevice(idx->device));
+    cudaStream_t st = idx->stream;
+    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
+    const size_t qb = static_cast<size_t>(nq) * idx->dim * sizeof(float);
+    const size_t lb = static_cast<size_t>(nq + 1) * sizeof(int64_t);
+    const size_t db = static_cast<size_t>(capacity) * sizeof(float), ib = static_cast<size_t>(capacity) * sizeof(int64_t);
+    IVR_TRY(ensure_pin(idx, up(qb) + up(lb)));
+    IVR_TRY(ensure_io(idx, up(qb) + up(lb) + up(db) + up(ib)));
+    char* pin = static_cast<char*>(idx->pin);
+    char* io = static_cast<char*>(idx->io);
+    float* dq = reinterpret_cast<float*>(io);
+    int64_t* dl = reinterpret_cast<int64_t*>(io + up(qb));
+    float* dd = reinterpret_cast<float*>(io + up(qb) + up(lb));
+    int64_t* di = reinterpret_cast<int64_t*>(io + up(qb) + up(lb) + up(db));
+    memcpy(pin, q_host, qb);
+    IVR_CUDA(cudaMemcpyAsync(dq, pin, qb, cudaMemcpyHostToDevice, st));
+    IVR_TRY(ivr_index_range_search_device(idx, dq, nq, radius, capacity, dl, dd, di, 0, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + up(qb), dl, lb, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaStreamSynchronize(st));
+    memcpy(lims_host, pin + up(qb), lb);
+    const int64_t total = lims_host[nq];
+    if (total == 0 || total > capacity) return IVR_OK;              // nothing to copy / the caller retries
+    // the hits, through the pinned buffer sized to what was found
+    const size_t hd = static_cast<size_t>(total) * sizeof(float), hi = static_cast<size_t>(total) * sizeof(int64_t);
+    IVR_TRY(ensure_pin(idx, up(hd) + up(hi)));
+    pin = static_cast<char*>(idx->pin);
+    IVR_CUDA(cudaMemcpyAsync(pin, dd, hd, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + up(hd), di, hi, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaStreamSynchronize(st));
+    staged_memcpy(D_host, pin, hd);
+    staged_memcpy(I_host, pin + up(hd), hi);
     return IVR_OK;
 }
 

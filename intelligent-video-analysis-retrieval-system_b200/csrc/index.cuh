@@ -63,6 +63,10 @@ int search_mma(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_d
                int64_t* I_dev, int64_t id_offset, cudaStream_t st);
 bool mma_supported(const ivr_index* idx, int64_t nq, int k);
 bool mma_small_supported(const ivr_index* idx, int64_t nq, int k);   // small-batch kernel (search_mma_small.cu)
+int  small_range_chunk(const ivr_index* idx);    // queries per range launch of that kernel; 0 = dimension too wide
+// lims, D, I = range_search(q, radius) on the current rows (range_search.cu); capacity <= INT_MAX
+int  range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                         int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st);
 
 // Generic list merge.  For query q, list l lives at entries + l*list_stride + q*q_stride
 // (64-bit keys) and holds counts[l*cnt_list_stride + q*cnt_q_stride] entries (or

@@ -372,5 +372,10 @@ int launch_seed_tau(const uint64_t* keys, const int* counts, uint32_t* tau_g, in
 // small-batch kernel (search_mma_small.cu)
 int  search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,
                       int64_t id_offset, cudaStream_t st);
+// its range epilogue: one launch of <= small_range_chunk() queries that appends every (row, query) with
+// score > radius to the hit pool of range_search.cu
+int  search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
+                            float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
+                            cudaStream_t st);
 
 }  // namespace ivr

@@ -1,0 +1,131 @@
+// range_search.cu -- exact range search: every stored row whose inner product with a query is > radius.
+//
+// Replaces lims, D, I = index.range_search(x, radius) of faiss.IndexFlatIP (not called by the reference).
+//   1. queries -> fp16, scaled by a power of two (launch_queries_to_f16), one chunk of <= small_range_chunk() queries
+//      at a time;
+//   2. one K1s launch per chunk in RANGE mode (search_mma_small.cu): every hit goes to one pool of
+//      (packed key, query) pairs; the 64-bit cursor counts every hit, also those past the pool's capacity;
+//   3. if the pool held them all: histogram by query, exclusive scan into lims, scatter into the query segments,
+//      segmented sort descending (the key order: score descending, then lower row), unpack to D / I.
+// Step 3 reads the cursor on the device, so nothing here waits for the GPU.  Algorithmic bytes:
+// ntotal * dpad * 2 per query chunk, plus 12 bytes per hit in the pool and 12 in the output.
+#include "mma_common.cuh"
+
+#include <climits>
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
+
+namespace ivr {
+
+__device__ __forceinline__ int64_t stored_hits(const unsigned long long* cursor, int64_t capacity) {
+    const unsigned long long total = *cursor;
+    return total > static_cast<unsigned long long>(capacity) ? 0 : static_cast<int64_t>(total);
+}
+
+__global__ void range_histogram_kernel(const uint32_t* __restrict__ qidx, const unsigned long long* __restrict__ cursor,
+                                       int64_t capacity, unsigned long long* __restrict__ counts) {
+    const int64_t n = stored_hits(cursor, capacity);
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+        atomicAdd(counts + qidx[i], 1ull);
+}
+
+__global__ void range_scatter_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ qidx,
+                                     const unsigned long long* __restrict__ cursor, int64_t capacity,
+                                     const int64_t* __restrict__ lims, unsigned long long* __restrict__ fill,
+                                     uint64_t* __restrict__ out) {
+    const int64_t n = stored_hits(cursor, capacity);
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const uint32_t q = qidx[i];
+        out[lims[q] + static_cast<int64_t>(atomicAdd(fill + q, 1ull))] = keys[i];
+    }
+}
+
+// D = score * q_scale[q], I = row + id_offset; the query of position i is found by bisection of lims
+__global__ void range_unpack_kernel(const uint64_t* __restrict__ keys, const unsigned long long* __restrict__ cursor,
+                                    int64_t capacity, const int64_t* __restrict__ lims, int64_t nq,
+                                    const float* __restrict__ q_scale, int64_t id_offset, float* __restrict__ D,
+                                    int64_t* __restrict__ I) {
+    const int64_t n = stored_hits(cursor, capacity);
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        int64_t lo = 0, hi = nq - 1;                     // the q with lims[q] <= i < lims[q + 1]
+        while (lo < hi) {
+            const int64_t mid = (lo + hi + 1) >> 1;
+            if (lims[mid] <= i) lo = mid; else hi = mid - 1;
+        }
+        const uint64_t key = keys[i];
+        D[i] = key_score(key) * q_scale[lo];
+        I[i] = static_cast<int64_t>(key_row(key)) + id_offset;
+    }
+}
+
+int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                        int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st) {
+    if (idx->ntotal == 0) {
+        IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    const int chunk = small_range_chunk(idx);
+    const int64_t n_chunks = (nq + chunk - 1) / chunk;
+    const int items = static_cast<int>(capacity);        // the caller checked capacity <= INT_MAX
+
+    size_t scan_bytes = 0, sort_bytes = 0;
+    IVR_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<const int64_t*>(nullptr),
+                                           static_cast<int64_t*>(nullptr), static_cast<int>(nq + 1), st));
+    IVR_CUDA(cub::DeviceSegmentedSort::SortKeysDescending(nullptr, sort_bytes, static_cast<const uint64_t*>(nullptr),
+                                                          static_cast<uint64_t*>(nullptr), items, static_cast<int>(nq),
+                                                          static_cast<const int64_t*>(nullptr),
+                                                          static_cast<const int64_t*>(nullptr), st));
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t o_q   = carve(static_cast<size_t>(chunk) * idx->dpad * 2);
+    const size_t o_sc  = carve(static_cast<size_t>(n_chunks) * chunk * 4);
+    const size_t o_tg  = carve(static_cast<size_t>(chunk) * 4);
+    const size_t zero_bytes = (1 + 2 * static_cast<size_t>(nq) + 1) * 8;   // cursor, counts [nq + 1], fill [nq]
+    const size_t o_z   = carve(zero_bytes);
+    const size_t o_k   = carve(static_cast<size_t>(capacity) * 8);
+    const size_t o_qi  = carve(static_cast<size_t>(capacity) * 4);
+    const size_t o_seg = carve(static_cast<size_t>(capacity) * 8);
+    const size_t o_srt = carve(static_cast<size_t>(capacity) * 8);
+    const size_t o_tmp = carve(std::max(scan_bytes, sort_bytes));
+    IVR_TRY(ensure_ws(idx, off));
+    char* ws = static_cast<char*>(idx->ws);
+    __half* q_h = reinterpret_cast<__half*>(ws + o_q);
+    float* q_scale = reinterpret_cast<float*>(ws + o_sc);
+    uint32_t* tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
+    unsigned long long* cursor = reinterpret_cast<unsigned long long*>(ws + o_z);
+    unsigned long long* counts = cursor + 1;
+    unsigned long long* fill = counts + nq + 1;
+    uint64_t* keys = reinterpret_cast<uint64_t*>(ws + o_k);
+    uint32_t* qidx = reinterpret_cast<uint32_t*>(ws + o_qi);
+    uint64_t* seg = reinterpret_cast<uint64_t*>(ws + o_seg);
+    uint64_t* sorted = reinterpret_cast<uint64_t*>(ws + o_srt);
+    void* tmp = ws + o_tmp;
+
+    IVR_CUDA(cudaMemsetAsync(cursor, 0, zero_bytes, st));
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        const int64_t q0 = c * chunk, m = std::min<int64_t>(chunk, nq - q0);
+        IVR_TRY(launch_queries_to_f16(q_dev + q0 * idx->dim, q_h, q_scale + q0, tau_g, m, (m + 15) / 16 * 16, idx->dim,
+                                      idx->dpad, st));
+        IVR_TRY(search_mma_small_range(idx, q_h, q_scale + q0, m, q0, radius, cursor, keys, qidx, capacity, st));
+    }
+    const int grid = idx->sm_count * 4, threads = 256;
+    range_histogram_kernel<<<grid, threads, 0, st>>>(qidx, cursor, capacity, counts);
+    IVR_CUDA(cudaGetLastError());
+    IVR_CUDA(cub::DeviceScan::ExclusiveSum(tmp, scan_bytes, reinterpret_cast<const int64_t*>(counts), lims,
+                                           static_cast<int>(nq + 1), st));
+    range_scatter_kernel<<<grid, threads, 0, st>>>(keys, qidx, cursor, capacity, lims, fill, seg);
+    IVR_CUDA(cudaGetLastError());
+    if (items > 0)
+        IVR_CUDA(cub::DeviceSegmentedSort::SortKeysDescending(tmp, sort_bytes, seg, sorted, items, static_cast<int>(nq),
+                                                              lims, lims + 1, st));
+    range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset, D, I);
+    IVR_CUDA(cudaGetLastError());
+    // lims[nq] = the true total: equal to the scan's when the pool held every hit, the size to retry with otherwise
+    IVR_CUDA(cudaMemcpyAsync(lims + nq, cursor, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    return IVR_OK;
+}
+
+}  // namespace ivr

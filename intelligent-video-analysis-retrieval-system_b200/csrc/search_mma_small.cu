@@ -26,6 +26,8 @@
 // next launch, so that lists almost never need compaction (the cold start of 4 x 148 lists per
 // query would otherwise cost more than the streaming itself).
 // The per-(CTA, warp) survivors are folded by topk_merge.cu.
+// A third epilogue, with a fixed threshold, runs in its own __global__ (search_mma_small_range_kernel) for the exact
+// range search of range_search.cu; it shares the producer and MMA code below.
 //
 // Replaces D, I = index.search(x, k) for small batches (unified_index.py:503, core.py:891).
 // Algorithmic bytes: ntotal * dpad * 2 per search.
@@ -76,38 +78,101 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&v)[32])
         : "r"(taddr) : "memory");
 }
 
+// Shared-memory layout of every K1s kernel: [query tile | row ring | aux]; aux holds the mbarriers, the TMEM address
+// slot and (from byte 512) the per-query thresholds.
+struct SmallSmem {
+    uint8_t* gen_base;              // generic address of smem_q
+    uint32_t smem_q, smem_a, aux;
+    uint32_t q_block, q_bytes;      // one k-block of the query matrix; all of it
+    __device__ __forceinline__ SmallSmem(uint8_t* smem_raw, int npad, int kblocks, int stages) {
+        smem_q = (smem_u32(smem_raw) + 1023u) & ~1023u;
+        gen_base = smem_raw + (smem_q - smem_u32(smem_raw));
+        q_block = static_cast<uint32_t>(npad) * 128u;
+        q_bytes = kblocks * q_block;
+        smem_a = smem_q + q_bytes;
+        aux = smem_a + stages * kSmallStageBytes;
+    }
+    __device__ __forceinline__ uint32_t full_bar(int s) const   { return aux + 8u * s; }
+    __device__ __forceinline__ uint32_t empty_bar(int s) const  { return aux + 8u * (16 + s); }
+    __device__ __forceinline__ uint32_t q_full() const          { return aux + 8u * 32; }
+    __device__ __forceinline__ uint32_t tfull_bar(int a) const  { return aux + 8u * (34 + a); }
+    __device__ __forceinline__ uint32_t tempty_bar(int a) const { return aux + 8u * (42 + a); }
+    __device__ __forceinline__ uint32_t tmem_slot() const       { return aux + 8u * 50; }
+    __device__ __forceinline__ float* tau_s() const { return reinterpret_cast<float*>(gen_base + (aux - smem_q) + 512); }
+};
+
+// Prologue shared by the K1s kernels, before their __syncthreads: barriers, descriptor prefetch, TMEM allocation.
+__device__ __forceinline__ void small_setup(const SmallSmem& sm, const CUtensorMap* tmap_q, const CUtensorMap* tmap_x,
+                                            int stages, int nbuf, int warp, int lane) {
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < stages; ++s) { mbar_init(sm.full_bar(s), 1); mbar_init(sm.empty_bar(s), 1); }
+        mbar_init(sm.q_full(), 1);
+        for (int a = 0; a < nbuf; ++a) { mbar_init(sm.tfull_bar(a), 1); mbar_init(sm.tempty_bar(a), 4); }
+        fence_barrier_init();
+    }
+    if (warp == 0 && lane == 0) { tma_prefetch_desc(tmap_q); tma_prefetch_desc(tmap_x); }
+    if (warp == 1) tmem_alloc<1>(sm.tmem_slot(), 512);
+}
+
+// Warp 0, one lane: the query tile once, then row tiles [j0, j1) through the ring.
+__device__ __forceinline__ void small_produce(const SmallSmem& sm, const CUtensorMap* tmap_q, const CUtensorMap* tmap_x,
+                                              int kblocks, int stages, int64_t tile0, int64_t j0, int64_t j1,
+                                              uint64_t row_policy) {
+    mbar_expect_tx(sm.q_full(), sm.q_bytes);
+    for (int kb = 0; kb < kblocks; ++kb)
+        tma_load_2d<1>(sm.smem_q + kb * sm.q_block, tmap_q, sm.q_full(), kb * kKBlock, 0, kL2EvictLast);
+    int stage = 0; uint32_t phase = 0;
+    for (int64_t j = j0; j < j1; ++j) {
+        const int row0 = static_cast<int>((tile0 + j) * kSmallTileRows);
+        for (int kb = 0; kb < kblocks; ++kb) {
+            mbar_wait(sm.empty_bar(stage), phase ^ 1);
+            mbar_expect_tx(sm.full_bar(stage), kSmallStageBytes);
+            tma_load_2d<1>(sm.smem_a + stage * kSmallStageBytes, tmap_x, sm.full_bar(stage), kb * kKBlock, row0, row_policy);
+            if (++stage == stages) { stage = 0; phase ^= 1; }
+        }
+    }
+}
+
+// Warp 1, one lane: D[128 rows, npad queries] of each row tile into the next of the nbuf TMEM accumulators.
+__device__ __forceinline__ void small_mma(const SmallSmem& sm, uint32_t tmem_base, int npad, int kblocks, int stages,
+                                          int nbuf, int buf_cols, int64_t j0, int64_t j1) {
+    const uint32_t idesc = make_idesc(kSmallTileRows, npad);
+    mbar_wait(sm.q_full(), 0);
+    tc_fence_after();
+    int stage = 0; uint32_t phase = 0; int buf = 0; uint32_t bphase = 0;
+    for (int64_t j = j0; j < j1; ++j) {
+        mbar_wait(sm.tempty_bar(buf), bphase ^ 1);                  // epilogue drained this accumulator
+        tc_fence_after();
+        const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(buf * buf_cols);
+        for (int kb = 0; kb < kblocks; ++kb) {
+            mbar_wait(sm.full_bar(stage), phase);
+            tc_fence_after();
+            const uint32_t a0 = sm.smem_a + stage * kSmallStageBytes;   // A: streamed rows (M)
+            const uint32_t b0 = sm.smem_q + kb * sm.q_block;            // B: resident queries (N)
+#pragma unroll
+            for (int k4 = 0; k4 < kKBlock / 16; ++k4)
+                umma_f16<1>(tmem_d, make_smem_desc(a0 + k4 * 32), make_smem_desc(b0 + k4 * 32), idesc,
+                            (kb | k4) ? 1u : 0u);
+            umma_commit<1>(sm.empty_bar(stage));                    // ring slot free when these MMAs retire
+            if (++stage == stages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit<1>(sm.tfull_bar(buf));
+        if (++buf == nbuf) { buf = 0; bphase ^= 1; }
+    }
+}
+
 __global__ void __launch_bounds__(kSmallThreads, 1)
 search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
                         const SmallParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
-    const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    uint8_t* const gen_base = smem_raw + (smem_base - smem_u32(smem_raw));
+    const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    const uint32_t q_block = static_cast<uint32_t>(p.npad) * 128u;   // one k-block of the query matrix
-    const uint32_t q_bytes = p.kblocks * q_block;
-    const uint32_t smem_q = smem_base;
-    const uint32_t smem_a = smem_q + q_bytes;
-    const uint32_t aux = smem_a + p.stages * kSmallStageBytes;
-    auto full_bar   = [&](int s) { return aux + 8u * s; };
-    auto empty_bar  = [&](int s) { return aux + 8u * (16 + s); };
-    const uint32_t q_full = aux + 8u * 32;
-    auto tfull_bar  = [&](int a) { return aux + 8u * (34 + a); };
-    auto tempty_bar = [&](int a) { return aux + 8u * (42 + a); };
-    const uint32_t tmem_slot = aux + 8u * 50;
-    float* const tau_s = reinterpret_cast<float*>(gen_base + (aux - smem_base) + 512);   // [128]
-    int*   const cnt_s = reinterpret_cast<int*>(gen_base + (aux - smem_base) + 1024);    // [4][128]
+    float* const tau_s = sm.tau_s();                                                          // [128]
+    int*   const cnt_s = reinterpret_cast<int*>(sm.gen_base + (sm.aux - sm.smem_q) + 1024);   // [4][128]
 
     const int64_t j0 = p.nt * blockIdx.x / gridDim.x, j1 = p.nt * (blockIdx.x + 1) / gridDim.x;   // owned row tiles
 
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < p.stages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-        mbar_init(q_full, 1);
-        for (int a = 0; a < p.nbuf; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 4); }
-        fence_barrier_init();
-    }
-    if (warp == 0 && lane == 0) { tma_prefetch_desc(&tmap_q); tma_prefetch_desc(&tmap_x); }
-    if (warp == 1) tmem_alloc<1>(tmem_slot, 512);
+    small_setup(sm, &tmap_q, &tmap_x, p.stages, p.nbuf, warp, lane);
     for (int i = threadIdx.x; i < 4 * kSmallMaxQ; i += kSmallThreads) cnt_s[i] = 0;
     for (int i = threadIdx.x; i < kSmallMaxQ; i += kSmallThreads)      // padded queries admit nothing
         tau_s[i] = (i < p.nq) ? ord2f(__ldcg(p.tau_g + i)) : __int_as_float(0x7f800000);
@@ -115,48 +180,12 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     __syncthreads();
     tc_fence_after();
     uint32_t tmem_base;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
 
     if (warp == 0 && lane == 0) {
-        // ============================ TMA producer ============================
-        mbar_expect_tx(q_full, q_bytes);
-        for (int kb = 0; kb < p.kblocks; ++kb)
-            tma_load_2d<1>(smem_q + kb * q_block, &tmap_q, q_full, kb * kKBlock, 0, kL2EvictLast);
-        int stage = 0; uint32_t phase = 0;
-        for (int64_t j = j0; j < j1; ++j) {
-            const int row0 = static_cast<int>((p.tile0 + j) * kSmallTileRows);
-            for (int kb = 0; kb < p.kblocks; ++kb) {
-                mbar_wait(empty_bar(stage), phase ^ 1);
-                mbar_expect_tx(full_bar(stage), kSmallStageBytes);
-                tma_load_2d<1>(smem_a + stage * kSmallStageBytes, &tmap_x, full_bar(stage), kb * kKBlock, row0, p.row_policy);
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-        }
+        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, p.tile0, j0, j1, p.row_policy);
     } else if (warp == 1 && lane == 0) {
-        // ============================ MMA issuer ==============================
-        const uint32_t idesc = make_idesc(kSmallTileRows, p.npad);
-        mbar_wait(q_full, 0);
-        tc_fence_after();
-        int stage = 0; uint32_t phase = 0; int buf = 0; uint32_t bphase = 0;
-        for (int64_t j = j0; j < j1; ++j) {
-            mbar_wait(tempty_bar(buf), bphase ^ 1);                  // epilogue drained this accumulator
-            tc_fence_after();
-            const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(buf * p.buf_cols);
-            for (int kb = 0; kb < p.kblocks; ++kb) {
-                mbar_wait(full_bar(stage), phase);
-                tc_fence_after();
-                const uint32_t a0 = smem_a + stage * kSmallStageBytes;   // A: streamed rows (M)
-                const uint32_t b0 = smem_q + kb * q_block;               // B: resident queries (N)
-#pragma unroll
-                for (int k4 = 0; k4 < kKBlock / 16; ++k4)
-                    umma_f16<1>(tmem_d, make_smem_desc(a0 + k4 * 32), make_smem_desc(b0 + k4 * 32), idesc,
-                                (kb | k4) ? 1u : 0u);
-                umma_commit<1>(empty_bar(stage));                    // ring slot free when these MMAs retire
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-            umma_commit<1>(tfull_bar(buf));
-            if (++buf == p.nbuf) { buf = 0; bphase ^= 1; }
-        }
+        small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, j0, j1);
     } else if (warp >= 2) {
         // ============================ epilogue: fused top-k ====================
         const int quarter = warp & 3;                              // the TMEM lanes this warp may read
@@ -189,7 +218,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
                 const int64_t grp = tile * p.n_groups / p.n_tiles;
                 const int64_t row = tile * kSmallTileRows + quarter * 32 + lane;
                 const bool valid = row < p.n_rows;
-                mbar_wait(tfull_bar(buf), bphase);
+                mbar_wait(sm.tfull_bar(buf), bphase);
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
                                        static_cast<uint32_t>(buf * p.buf_cols);
@@ -202,7 +231,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
                     if (c0 + 32 >= p.npad) {                            // accumulator fully read: hand it back
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) mbar_arrive_local(tempty_bar(buf));
+                        if (lane == 0) mbar_arrive_local(sm.tempty_bar(buf));
                     }
 #pragma unroll
                     for (int i = 0; i < 32; ++i) {
@@ -236,7 +265,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
             __syncwarp();
             const uint32_t row = static_cast<uint32_t>((p.tile0 + j) * kSmallTileRows + quarter * 32 + lane);
             const bool valid = static_cast<int64_t>(row) < p.n_rows;
-            mbar_wait(tfull_bar(buf), bphase);
+            mbar_wait(sm.tfull_bar(buf), bphase);
             tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
                                    static_cast<uint32_t>(buf * p.buf_cols);
@@ -253,7 +282,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
                 if (c0 + 32 >= p.npad) {                            // accumulator fully read: hand it back
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) mbar_arrive_local(tempty_bar(buf));
+                    if (lane == 0) mbar_arrive_local(sm.tempty_bar(buf));
                 }
                 unsigned m = 0;
                 const float4* t4 = reinterpret_cast<const float4*>(tau_s + c0);
@@ -296,23 +325,151 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
 }
 
+// RANGE mode: the same producer and MMA warps; the epilogue compares every score with a threshold that never moves
+// (radius / q_scale[q]: q_scale is a power of two, so the division is exact and "score > radius" survives it, except
+// at the ends of the float range) and appends the survivors to ONE hit pool shared by all CTAs and launches.  One
+// 64-bit cursor reservation per warp and 32-query chunk, no lists, no compaction, no counts.  Writes at or past
+// `capacity` are dropped, but the cursor still advances, so the true total is always known.
+struct SmallRangeParams {
+    int64_t  n_rows;
+    int      nq, npad, kblocks, stages, nbuf, buf_cols;
+    int64_t  nt;                       // row tiles (the whole index: one launch per query chunk)
+    uint64_t row_policy;
+    float        radius;
+    const float* q_scale;              // [nq] power-of-two query scales of this launch
+    uint32_t     q_base;               // global index of this launch's first query
+    unsigned long long* cursor;        // hits reserved so far, by every launch of the search
+    uint64_t*    keys;                 // [capacity] make_key(score in the kernel's domain, row)
+    uint32_t*    qidx;                 // [capacity] global query index of each key
+    unsigned long long capacity;
+};
+
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
+                              const SmallRangeParams p) {
+    extern __shared__ __align__(1024) uint8_t smem_raw[];
+    const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float* const tau_s = sm.tau_s();                                   // [128]
+    const int64_t j0 = p.nt * blockIdx.x / gridDim.x, j1 = p.nt * (blockIdx.x + 1) / gridDim.x;
+
+    small_setup(sm, &tmap_q, &tmap_x, p.stages, p.nbuf, warp, lane);
+    for (int i = threadIdx.x; i < kSmallMaxQ; i += kSmallThreads)      // padded queries admit nothing
+        tau_s[i] = (i < p.nq) ? p.radius / p.q_scale[i] : __int_as_float(0x7f800000);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    uint32_t tmem_base;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
+
+    if (warp == 0 && lane == 0) {
+        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, 0, j0, j1, p.row_policy);
+    } else if (warp == 1 && lane == 0) {
+        small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, j0, j1);
+    } else if (warp >= 2) {
+        // ============================ epilogue: fixed-threshold filter ========
+        const int quarter = warp & 3;                              // the TMEM lanes this warp may read
+        int buf = 0; uint32_t bphase = 0;
+        for (int64_t j = j0; j < j1; ++j) {
+            const int64_t row64 = j * kSmallTileRows + quarter * 32 + lane;
+            const bool valid = row64 < p.n_rows;
+            const uint32_t row = static_cast<uint32_t>(row64);
+            mbar_wait(sm.tfull_bar(buf), bphase);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
+                                   static_cast<uint32_t>(buf * p.buf_cols);
+            for (int c0 = 0; c0 < p.npad; c0 += 32) {
+                uint32_t v[32];
+                if (p.npad - c0 >= 32) {
+                    tmem_ld_32x32(taddr + c0, v);
+                } else {                                            // npad is a multiple of 16: a 16-column tail
+#pragma unroll
+                    for (int i = 16; i < 32; ++i) v[i] = 0xff800000u;
+                    tmem_ld_32x16(taddr + c0, v);
+                }
+                tmem_wait_ld(v);
+                if (c0 + 32 >= p.npad) {                            // accumulator fully read: hand it back
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_local(sm.tempty_bar(buf));
+                }
+                unsigned m = 0;
+                const float4* t4 = reinterpret_cast<const float4*>(tau_s + c0);
+#pragma unroll
+                for (int i4 = 0; i4 < 8; ++i4) {
+                    const float4 t = t4[i4];
+                    m |= (__uint_as_float(v[4 * i4 + 0]) > t.x ? 1u : 0u) << (4 * i4 + 0);
+                    m |= (__uint_as_float(v[4 * i4 + 1]) > t.y ? 1u : 0u) << (4 * i4 + 1);
+                    m |= (__uint_as_float(v[4 * i4 + 2]) > t.z ? 1u : 0u) << (4 * i4 + 2);
+                    m |= (__uint_as_float(v[4 * i4 + 3]) > t.w ? 1u : 0u) << (4 * i4 + 3);
+                }
+                if (!valid) m = 0;                                  // rows past the end (TMA zero fill)
+                // one reservation for the warp's hits, each lane's slots from an inclusive prefix sum
+                const int cnt = __popc(m);
+                int incl = cnt;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += t;
+                }
+                const int total = __shfl_sync(0xffffffffu, incl, 31);
+                if (total == 0) continue;                           // warp-uniform
+                unsigned long long slot = 0;
+                if (lane == 0) slot = atomicAdd(p.cursor, static_cast<unsigned long long>(total));
+                slot = __shfl_sync(0xffffffffu, slot, 0) + static_cast<unsigned long long>(incl - cnt);
+#pragma unroll
+                for (int i = 0; i < 32; ++i) {
+                    if (!((m >> i) & 1u)) continue;
+                    if (slot < p.capacity) {
+                        p.keys[slot] = make_key(__uint_as_float(v[i]), row);
+                        p.qidx[slot] = p.q_base + static_cast<uint32_t>(c0 + i);
+                    }
+                    ++slot;
+                }
+            }
+            if (++buf == p.nbuf) { buf = 0; bphase ^= 1; }
+        }
+    }
+
+    // ------------------------------------------------------------------ teardown ----
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
+}
+
 // ------------------------------------------------------------------ host side ----
 struct SmallShape { int npad, stages, nbuf, buf_cols, C; size_t smem; };
 
-static bool small_shape(const ivr_index* idx, int64_t nq, int k, SmallShape* s) {
-    if (k < 1 || k > IVR_MAX_K || nq < 1 || nq > kSmallMaxQ) return false;
+// Pipeline shape of a K1s launch over nq queries: false when the resident query tile does not fit.
+static bool pipe_shape(const ivr_index* idx, int64_t nq, SmallShape* s) {
+    if (nq < 1 || nq > kSmallMaxQ) return false;
     const int npad = static_cast<int>((nq + 15) / 16 * 16);
-    const int C = 2 * kcap_for(k);
-    if (static_cast<size_t>(4 * idx->sm_count) * npad * C * 8 > kSmallMaxListBytes) return false;   // huge k x many queries
     const int64_t q_bytes = static_cast<int64_t>(npad) * idx->dpad * 2;
     if (q_bytes > 128 * 1024) return false;
     const int stages = std::min<int64_t>(12, (kSmemBudget - 1024 - kSmallAuxBytes - q_bytes) / kSmallStageBytes);
     if (stages < 4) return false;
-    s->npad = npad; s->stages = stages; s->C = C;
+    s->npad = npad; s->stages = stages; s->C = 0;
     s->buf_cols = std::max(npad, 32);
     s->nbuf = std::min(kSmallMaxBuf, 512 / s->buf_cols);
     s->smem = 1024 + static_cast<size_t>(q_bytes) + static_cast<size_t>(stages) * kSmallStageBytes + kSmallAuxBytes;
     return true;
+}
+
+static bool small_shape(const ivr_index* idx, int64_t nq, int k, SmallShape* s) {
+    if (k < 1 || k > IVR_MAX_K || !pipe_shape(idx, nq, s)) return false;
+    const int C = 2 * kcap_for(k);
+    if (static_cast<size_t>(4 * idx->sm_count) * s->npad * C * 8 > kSmallMaxListBytes) return false;   // huge k x many queries
+    s->C = C;
+    return true;
+}
+
+// The TMA descriptor of the (windowed) row matrix in 128-row boxes, cached on the handle.
+static int small_row_tmap(ivr_index* idx) {
+    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != kSmallTileRows) {
+        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, kSmallTileRows));
+        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = kSmallTileRows;
+    }
+    return IVR_OK;
 }
 
 bool mma_small_supported(const ivr_index* idx, int64_t nq, int k) {
@@ -353,10 +510,7 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
 
     CUtensorMap tmq;
     IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
-    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != kSmallTileRows) {
-        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, kSmallTileRows));
-        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = kSmallTileRows;
-    }
+    IVR_TRY(small_row_tmap(idx));
     const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
     IVR_CUDA(cudaFuncSetAttribute(search_mma_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(sh.smem)));
@@ -449,10 +603,7 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
 
     CUtensorMap tmq;
     IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
-    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != kSmallTileRows) {
-        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, kSmallTileRows));
-        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = kSmallTileRows;
-    }
+    IVR_TRY(small_row_tmap(idx));
     const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
     IVR_CUDA(cudaFuncSetAttribute(search_mma_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(sh.smem)));
@@ -504,6 +655,37 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
         idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
     }
     idx->last_kernel = "search_mma_small_kernel";
+    return IVR_OK;
+}
+
+int small_range_chunk(const ivr_index* idx) {
+    return std::min(kSmallMaxQ, 65536 / idx->dpad / 16 * 16);
+}
+
+int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
+                           float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
+                           cudaStream_t st) {
+    SmallShape sh;
+    if (nq > small_range_chunk(idx) || !pipe_shape(idx, nq, &sh)) {
+        set_error("range_search: %lld queries of dim %d do not fit one query tile", static_cast<long long>(nq), idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    CUtensorMap tmq;
+    IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
+    IVR_TRY(small_row_tmap(idx));
+    const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    IVR_CUDA(cudaFuncSetAttribute(search_mma_small_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(sh.smem)));
+    SmallRangeParams p{};
+    p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad;
+    p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
+    p.nt = (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
+    p.row_policy = kL2EvictFirst;                                    // each launch reads every row once
+    p.radius = radius; p.q_scale = q_scale; p.q_base = static_cast<uint32_t>(q_base);
+    p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
+    const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(p.nt, 1)));
+    search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
+    IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }
 

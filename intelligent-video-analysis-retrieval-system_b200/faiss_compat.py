@@ -39,7 +39,7 @@ class IndexFlatIP:
     """Exact inner-product index; rows live in HBM as fp16, ids are insertion order.
 
     ``add`` / ``search`` / ``ntotal`` / ``d`` / ``is_trained`` / ``train`` / ``reset`` follow
-    ``faiss.IndexFlatIP`` as used by the reference.
+    ``faiss.IndexFlatIP`` as used by the reference; ``range_search`` follows FAISS's flat-index range query.
     """
 
     metric_type = METRIC_INNER_PRODUCT
@@ -171,6 +171,52 @@ class IndexFlatIP:
                 self._handle(), q.data_ptr(), nq, k, out.data_ptr(), int(id_offset),
                 self.search_path if path is None else path, st))
         return out
+
+    def range_search(self, x, radius: float):
+        """lims, D, I = index.range_search(x, radius): every stored row whose inner product with the query is
+        strictly greater than ``radius``.  Query i's hits are ``D[lims[i]:lims[i+1]]`` (float32, descending, ties ->
+        lower id) and ``I[lims[i]:lims[i+1]]`` (int64).  A CUDA tensor ``x`` runs ``range_search_tensor``."""
+        if _is_cuda_tensor(x):
+            return self.range_search_tensor(x, radius)
+        q = _as_f32_2d(x, self.d, "range_search(x)")
+        radius = _radius(radius)
+        nq = q.shape[0]
+        lims = np.zeros(nq + 1, np.int64)
+        cap = _range_capacity(nq, self.ntotal)
+        while True:                                     # at most twice: the first call reports the exact total
+            D = np.empty(cap, np.float32)
+            I = np.empty(cap, np.int64)
+            nat.check(nat.lib.ivr_index_range_search(self._handle(), q.ctypes.data, nq, radius, cap,
+                                                     lims.ctypes.data, D.ctypes.data, I.ctypes.data))
+            total = int(lims[nq])
+            if total <= cap:
+                return lims, D[:total].copy(), I[:total].copy()
+            cap = total
+
+    def range_search_tensor(self, q, radius: float, id_offset: int = 0):
+        """Device-resident range search on torch's current stream; returns CUDA tensors (lims, D, I), ids =
+        stored row + ``id_offset``.  Sizing the outputs reads ``lims[nq]`` back to the host once (twice when more
+        hits than the first guess of the capacity turn up), so this call waits for the search to finish."""
+        import torch
+        if q.dim() != 2 or q.shape[1] != self.d:
+            raise ValueError(f"range_search(x): expected [nq,{self.d}], got {tuple(q.shape)}")
+        q = q.to(dtype=torch.float32).contiguous()
+        _check_device(q, self.device)
+        radius = _radius(radius)
+        nq = q.shape[0]
+        lims = torch.zeros(nq + 1, dtype=torch.int64, device=q.device)
+        cap = _range_capacity(nq, self.ntotal)
+        st = torch.cuda.current_stream(q.device).cuda_stream
+        while True:
+            D = torch.empty(cap, dtype=torch.float32, device=q.device)
+            I = torch.empty(cap, dtype=torch.int64, device=q.device)
+            nat.check(nat.lib.ivr_index_range_search_device(self._handle(), q.data_ptr(), nq, radius, cap,
+                                                            lims.data_ptr(), D.data_ptr(), I.data_ptr(),
+                                                            int(id_offset), st))
+            total = int(lims[nq].item())
+            if total <= cap:
+                return lims, D[:total], I[:total]
+            cap = total
 
     # -- instrumentation ---------------------------------------------------
     def set_timing(self, enable: bool = True):
@@ -329,6 +375,18 @@ def read_index(path, flags: int = 0, device: int | None = None) -> IndexFlatIP:
         _add_payload(index, payload, ntotal, d)
         del payload
     return index
+
+
+def _radius(radius) -> float:
+    r = float(radius)
+    if r != r:
+        raise ValueError("range_search: radius is NaN")
+    return r
+
+
+def _range_capacity(nq: int, ntotal: int) -> int:
+    """First guess of a range search's hit count: 1024 per query (at least 1 M), never more than nq * ntotal."""
+    return min(nq * ntotal, max(nq * 1024, 1 << 20), (1 << 31) - 1)
 
 
 def _is_cuda_tensor(x) -> bool:
