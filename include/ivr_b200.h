@@ -121,6 +121,15 @@ IVR_API int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t 
 IVR_API int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius,
                                           int64_t capacity, int64_t* lims_dev, float* D_dev, int64_t* I_dev,
                                           int64_t id_offset, void* stream);
+/* The same range search, hits left as PACKED exchange keys (the format of ivr_index_search_keys_device):
+ *   keys   uint64  [capacity] make_key(score, row + id_offset); query i's hits are keys[lims[i] : lims[i+1]], in the
+ *                             order of D / I above (score descending, then lower id), so unsigned key descending
+ * Same contract as ivr_index_range_search_device (capacity, the exact total in lims[nq], the search window, the
+ * argument checks before any device call); in addition id_offset + ntotal > 2^32 is IVR_EUNSUPPORTED.  The per-rank
+ * step of ShardedFlatIP.range_search: the runs of all ranks are merged by ivr_range_merge_keys_device. */
+IVR_API int ivr_index_range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius,
+                                               int64_t capacity, int64_t* lims_dev, uint64_t* keys_dev,
+                                               int64_t id_offset, void* stream);
 
 /* Search window: until cleared (count < 0) every search on this handle scores only the stored rows
  * [first, first + count) -- ids are still "stored row + id_offset", k > count pads as usual, a window reaching beyond
@@ -151,6 +160,19 @@ IVR_API int ivr_topk_merge_device(int device, const float* D_parts, const int64_
  * (device; the all-gather output), n_parts <= 64.  No scratch, no allocation, one kernel launch. */
 IVR_API int ivr_topk_merge_keys_device(int device, const uint64_t* keys_parts, int n_parts, int64_t nq, int k,
                                float* D_out, int64_t* I_out, void* stream);
+/* Merge of per-part range results (the runs of ivr_index_range_search_keys_device after one all-gather), device:
+ *   keys_parts uint64 [n_parts, part_stride]: part p holds query q's hits, sorted (unsigned key descending), at
+ *              [lims_parts[p][q], lims_parts[p][q+1])
+ *   lims_parts int64  [n_parts, nq + 1]
+ * Out: lims int64 [nq + 1], lims[q] = sum over p of lims_parts[p][q]; D float32 / I int64 [lims[nq]] in key order
+ * (score descending, then lower id; I = the key's 32-bit id).  An equal key in two parts is placed after the one of
+ * the lower part, so the output stays a permutation of the input.  n_parts in 1..64, nq >= 0; keys_parts, D and I
+ * may be NULL only when part_stride == 0; else IVR_EINVAL before any device call.  The caller promises
+ * part_stride >= lims_parts[p][nq] for every p and monotone lims_parts (they live on the device and are not read
+ * back).  Two kernel launches, no atomics, no scratch, no allocation, deterministic. */
+IVR_API int ivr_range_merge_keys_device(int device, const uint64_t* keys_parts, int64_t part_stride,
+                                        const int64_t* lims_parts, int n_parts, int64_t nq, int64_t* lims, float* D,
+                                        int64_t* I, void* stream);
 
 /* ---- K7: cross-shard hit exchange over NVLink / NVSwitch peer memory ------------------------
  * Replaces the "collect every shard's hit list" step of _search_with_remote_index (system.py:1721-1746) for

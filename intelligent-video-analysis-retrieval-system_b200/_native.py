@@ -52,6 +52,8 @@ PROTOTYPES = {
                                          C.c_void_p, C.c_void_p]),
     "ivr_index_range_search_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_int64,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "ivr_index_range_search_keys_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_int64,
+                                                     C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "ivr_index_set_window": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64]),
     "ivr_index_set_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "ivr_index_last_timing": (C.c_int, [C.c_void_p, _c_f32p, _c_intp]),
@@ -61,6 +63,8 @@ PROTOTYPES = {
                                         C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ivr_topk_merge_keys_device": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_void_p,
                                              C.c_void_p, C.c_void_p]),
+    "ivr_range_merge_keys_device": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int64,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ivr_exchange_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_void_p)]),
     "ivr_exchange_destroy": (C.c_int, [C.c_void_p]),
     "ivr_exchange_base": (C.c_void_p, [C.c_void_p]),

@@ -535,6 +535,25 @@ int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq
     });
 }
 
+int ivr_index_range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                                       int64_t* lims_dev, uint64_t* keys_dev, int64_t id_offset, void* stream) {
+    IVR_TRY(range_args(idx, q_dev, nq, radius, capacity, lims_dev, keys_dev, keys_dev));
+    if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
+        set_error("range_search_keys: global row ids must stay below 2^32 (offset %lld + %lld rows)",
+                  static_cast<long long>(id_offset), static_cast<long long>(idx->ntotal));
+        return IVR_EUNSUPPORTED;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (nq == 0) {
+        IVR_CUDA(cudaSetDevice(idx->device));
+        IVR_CUDA(cudaMemsetAsync(lims_dev, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return with_search_window(idx, id_offset, st, "range_search_keys", [&](int64_t id_offset) {
+        return range_search_keys_device(idx, q_dev, nq, radius, capacity, lims_dev, keys_dev, id_offset, st);
+    });
+}
+
 int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, float radius, int64_t capacity,
                            int64_t* lims_host, float* D_host, int64_t* I_host) {
     IVR_TRY(range_args(idx, q_host, nq, radius, capacity, lims_host, D_host, I_host));
@@ -644,6 +663,25 @@ int ivr_topk_merge_keys_device(int device, const uint64_t* keys_parts, int n_par
     in.list_stride = nq * k; in.q_stride = k;
     in.n_lists = n_parts; in.fixed_count = k;
     return merge_lists_final(in, nq, k, D_out, I_out, 0, nullptr, nullptr, static_cast<cudaStream_t>(stream), nullptr);
+}
+
+int ivr_range_merge_keys_device(int device, const uint64_t* keys_parts, int64_t part_stride, const int64_t* lims_parts,
+                                int n_parts, int64_t nq, int64_t* lims, float* D, int64_t* I, void* stream) {
+    if (n_parts < 1 || n_parts > 64 || nq < 0 || part_stride < 0 || !lims_parts || !lims ||
+        (part_stride > 0 && (!keys_parts || !D || !I))) {
+        set_error("range_merge_keys: bad argument (n_parts %d of 1..64, nq %lld, part_stride %lld, or a NULL buffer)",
+                  n_parts, static_cast<long long>(nq), static_cast<long long>(part_stride));
+        return IVR_EINVAL;
+    }
+    if (part_stride > INT64_MAX / n_parts || nq >= INT64_MAX / 64) {
+        set_error("range_merge_keys: n_parts * part_stride or n_parts * (nq + 1) overflows");
+        return IVR_EINVAL;
+    }
+    static thread_local int checked_device = -1;       // the capability probe is done once per thread and device
+    if (checked_device != device) { IVR_TRY(require_device(device)); checked_device = device; }
+    else IVR_CUDA(cudaSetDevice(device));
+    return range_merge_keys_device(keys_parts, part_stride, lims_parts, n_parts, nq, lims, D, I,
+                                   static_cast<cudaStream_t>(stream));
 }
 
 // ------------------------------------------------------------ normalise ----

@@ -61,8 +61,30 @@ __global__ void range_unpack_kernel(const uint64_t* __restrict__ keys, const uns
     }
 }
 
-int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
-                        int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st) {
+// keys[i] = make_key(score * q_scale[q], row + id_offset), the exchange key of ivr_index_search_keys_device.  q_scale
+// is a power of two, so the rescaled keys keep the segmented sort's order (score descending, then lower row).
+__global__ void range_pack_keys_kernel(const uint64_t* __restrict__ sorted,
+                                       const unsigned long long* __restrict__ cursor, int64_t capacity,
+                                       const int64_t* __restrict__ lims, int64_t nq, const float* __restrict__ q_scale,
+                                       int64_t id_offset, uint64_t* __restrict__ keys) {
+    const int64_t n = stored_hits(cursor, capacity);
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        int64_t lo = 0, hi = nq - 1;
+        while (lo < hi) {
+            const int64_t mid = (lo + hi + 1) >> 1;
+            if (lims[mid] <= i) lo = mid; else hi = mid - 1;
+        }
+        const uint64_t key = sorted[i];
+        keys[i] = make_key(key_score(key) * q_scale[lo], key_row(key) + static_cast<uint32_t>(id_offset));
+    }
+}
+
+// The body shared by both range entry points: score, group and sort every hit into lims / the sorted pool, then
+// finish(sorted, cursor, q_scale, grid, threads) queues the last step, which writes the caller's output.
+template <class Finish>
+static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                               int64_t* lims, cudaStream_t st, Finish&& finish) {
     if (idx->ntotal == 0) {
         IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t), st));
         return IVR_OK;
@@ -121,10 +143,100 @@ int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float ra
     if (items > 0)
         IVR_CUDA(cub::DeviceSegmentedSort::SortKeysDescending(tmp, sort_bytes, seg, sorted, items, static_cast<int>(nq),
                                                               lims, lims + 1, st));
-    range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset, D, I);
-    IVR_CUDA(cudaGetLastError());
+    IVR_TRY(finish(static_cast<const uint64_t*>(sorted), static_cast<const unsigned long long*>(cursor),
+                   static_cast<const float*>(q_scale), grid, threads));
     // lims[nq] = the true total: equal to the scan's when the pool held every hit, the size to retry with otherwise
     IVR_CUDA(cudaMemcpyAsync(lims + nq, cursor, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    return IVR_OK;
+}
+
+int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                        int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st) {
+    return range_search_sorted(idx, q_dev, nq, radius, capacity, lims, st,
+                               [&](const uint64_t* sorted, const unsigned long long* cursor, const float* q_scale,
+                                   int grid, int threads) {
+        range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset, D, I);
+        IVR_CUDA(cudaGetLastError());
+        return IVR_OK;
+    });
+}
+
+int range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                             int64_t* lims, uint64_t* keys, int64_t id_offset, cudaStream_t st) {
+    return range_search_sorted(idx, q_dev, nq, radius, capacity, lims, st,
+                               [&](const uint64_t* sorted, const unsigned long long* cursor, const float* q_scale,
+                                   int grid, int threads) {
+        range_pack_keys_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset,
+                                                         keys);
+        IVR_CUDA(cudaGetLastError());
+        return IVR_OK;
+    });
+}
+
+// ---- merge of per-rank range runs (ShardedFlatIP.range_search) ----
+
+// lims[q] = sum over parts of lims_parts[p][q]
+__global__ void range_merge_lims_kernel(const int64_t* __restrict__ lims_parts, int n_parts, int64_t nq,
+                                        int64_t* __restrict__ lims) {
+    for (int64_t q = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; q <= nq;
+         q += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        int64_t s = 0;
+        for (int p = 0; p < n_parts; ++p) s += lims_parts[p * (nq + 1) + q];
+        lims[q] = s;
+    }
+}
+
+// One thread per input hit (p, j).  Its query q comes from bisecting lims_parts[p]; its output slot is
+//   sum_s lims_parts[s][q]  +  (j - lims_parts[p][q])  +  sum_{s != p} |{keys of run (s, q) that come before it}|,
+// the count found by binary search in each other (descending) run: keys greater than it, and in a lower part also
+// keys equal to it.  This is the rank of (key, part, position) in one total order, so the slots are a permutation of
+// query q's output range, also when two parts hold the same key.  Every slot stays inside [lims[q], lims[q + 1]).
+__global__ void range_merge_keys_kernel(const uint64_t* __restrict__ keys_parts, int64_t part_stride,
+                                        const int64_t* __restrict__ lims_parts, int n_parts, int64_t nq,
+                                        float* __restrict__ D, int64_t* __restrict__ I) {
+    const int64_t n = static_cast<int64_t>(n_parts) * part_stride;
+    for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < n;
+         t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int p = static_cast<int>(t / part_stride);
+        const int64_t j = t - p * part_stride;
+        const int64_t* lp = lims_parts + p * (nq + 1);
+        if (j >= lp[nq]) continue;
+        int64_t lo = 0, hi = nq - 1;                     // the q with lp[q] <= j < lp[q + 1]
+        while (lo < hi) {
+            const int64_t mid = (lo + hi + 1) >> 1;
+            if (lp[mid] <= j) lo = mid; else hi = mid - 1;
+        }
+        const int64_t q = lo;
+        const uint64_t key = keys_parts[t];
+        int64_t slot = j - lp[q];
+        for (int s = 0; s < n_parts; ++s) {
+            const int64_t* ls = lims_parts + s * (nq + 1);
+            const int64_t b = ls[q], e = ls[q + 1];
+            slot += b;
+            if (s == p) continue;
+            const uint64_t* run = keys_parts + s * part_stride;
+            int64_t a = b, z = e;                        // first position in [b, e) that comes after `key`
+            if (s < p) { while (a < z) { const int64_t m = (a + z) >> 1; if (run[m] >= key) a = m + 1; else z = m; } }
+            else       { while (a < z) { const int64_t m = (a + z) >> 1; if (run[m] > key) a = m + 1; else z = m; } }
+            slot += a - b;
+        }
+        D[slot] = key_score(key);
+        I[slot] = static_cast<int64_t>(key_row(key));
+    }
+}
+
+int range_merge_keys_device(const uint64_t* keys_parts, int64_t part_stride, const int64_t* lims_parts, int n_parts,
+                            int64_t nq, int64_t* lims, float* D, int64_t* I, cudaStream_t st) {
+    const int threads = 256;
+    const int64_t grid_cap = 2048;                       // grid-stride beyond that: enough blocks to fill 148 SMs
+    const int g_lims = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((nq + threads) / threads, grid_cap)));
+    range_merge_lims_kernel<<<g_lims, threads, 0, st>>>(lims_parts, n_parts, nq, lims);
+    IVR_CUDA(cudaGetLastError());
+    const int64_t n = static_cast<int64_t>(n_parts) * part_stride;
+    if (n == 0) return IVR_OK;
+    const int g = static_cast<int>(std::min<int64_t>((n + threads - 1) / threads, grid_cap));
+    range_merge_keys_kernel<<<g, threads, 0, st>>>(keys_parts, part_stride, lims_parts, n_parts, nq, D, I);
+    IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }
 

@@ -198,6 +198,37 @@ class IndexFlatIP:
         stored row + ``id_offset``.  Sizing the outputs reads ``lims[nq]`` back to the host once (twice when more
         hits than the first guess of the capacity turn up), so this call waits for the search to finish."""
         import torch
+
+        def call(q, radius, cap, lims, st):
+            D = torch.empty(cap, dtype=torch.float32, device=q.device)
+            I = torch.empty(cap, dtype=torch.int64, device=q.device)
+            nat.check(nat.lib.ivr_index_range_search_device(self._handle(), q.data_ptr(), q.shape[0], radius, cap,
+                                                            lims.data_ptr(), D.data_ptr(), I.data_ptr(),
+                                                            int(id_offset), st))
+            return D, I
+        lims, total, (D, I) = self._range_device(q, radius, call)
+        return lims, D[:total], I[:total]
+
+    def range_search_keys_tensor(self, q, radius: float, id_offset: int = 0):
+        """``range_search_tensor`` with the hits left as packed 64-bit keys: returns CUDA int64 tensors (lims, keys),
+        query i's hits are ``keys[lims[i]:lims[i+1]]`` holding ``order_preserving(score) << 32 | ~(row + id_offset)``
+        in descending unsigned order (score descending, then lower id).  The per-rank step of
+        ``ShardedFlatIP.range_search``; global ids must stay below 2^32."""
+        import torch
+
+        def call(q, radius, cap, lims, st):
+            keys = torch.empty(cap, dtype=torch.int64, device=q.device)
+            nat.check(nat.lib.ivr_index_range_search_keys_device(self._handle(), q.data_ptr(), q.shape[0], radius,
+                                                                 cap, lims.data_ptr(), keys.data_ptr(),
+                                                                 int(id_offset), st))
+            return (keys,)
+        lims, total, (keys,) = self._range_device(q, radius, call)
+        return lims, keys[:total]
+
+    def _range_device(self, q, radius, call):
+        """Checks, then ``call(q, radius, capacity, lims, stream)`` with the first capacity guess and once more with
+        the exact total when that overflowed.  Returns (lims, total hits, the outputs of the last call)."""
+        import torch
         if q.dim() != 2 or q.shape[1] != self.d:
             raise ValueError(f"range_search(x): expected [nq,{self.d}], got {tuple(q.shape)}")
         q = q.to(dtype=torch.float32).contiguous()
@@ -208,14 +239,10 @@ class IndexFlatIP:
         cap = _range_capacity(nq, self.ntotal)
         st = torch.cuda.current_stream(q.device).cuda_stream
         while True:
-            D = torch.empty(cap, dtype=torch.float32, device=q.device)
-            I = torch.empty(cap, dtype=torch.int64, device=q.device)
-            nat.check(nat.lib.ivr_index_range_search_device(self._handle(), q.data_ptr(), nq, radius, cap,
-                                                            lims.data_ptr(), D.data_ptr(), I.data_ptr(),
-                                                            int(id_offset), st))
+            out = call(q, radius, cap, lims, st)
             total = int(lims[nq].item())
             if total <= cap:
-                return lims, D[:total], I[:total]
+                return lims, total, out
             cap = total
 
     # -- instrumentation ---------------------------------------------------

@@ -131,6 +131,23 @@ def _cuda_merge(device: int):
     return merge
 
 
+def _cuda_range_merge(keys_parts, lims_parts, total: int):
+    """ivr_range_merge_keys_device on the current stream: keys_parts int64 [world, stride] (the all-gathered padded
+    runs), lims_parts int64 [world, nq + 1], total = the sum of lims_parts[:, nq].  Returns (lims, D, I)."""
+    import torch
+    from . import _native as nat
+    dev = lims_parts.device
+    n_parts, stride = keys_parts.shape
+    nq = lims_parts.shape[1] - 1
+    lims = torch.empty(nq + 1, dtype=torch.int64, device=dev)
+    D = torch.empty(total, dtype=torch.float32, device=dev)
+    I = torch.empty(total, dtype=torch.int64, device=dev)
+    nat.check(nat.lib.ivr_range_merge_keys_device(dev.index, keys_parts.data_ptr(), stride, lims_parts.data_ptr(),
+                                                  n_parts, nq, lims.data_ptr(), D.data_ptr(), I.data_ptr(),
+                                                  torch.cuda.current_stream(dev).cuda_stream))
+    return lims, D, I
+
+
 class _PeerExchange:
     """The mailbox of ``csrc/exchange.cu`` for one rank (ctypes over ``ivr_exchange_*``)."""
 
@@ -210,12 +227,15 @@ class ShardedFlatIP:
 
     ``local_index`` / ``merge`` can be injected (the CPU ``gloo`` tests exercise the
     partition / offset / gather logic with a stand-in backend that speaks the same packed-key
-    protocol: ``search_keys_tensor(q, k, id_offset, out)`` and ``merge(keys [world, nq, k], k)``);
-    by default they are the CUDA index and the CUDA merge kernel and fail loudly without a GPU.
+    protocol: ``search_keys_tensor(q, k, id_offset, out)`` and ``merge(keys [world, nq, k], k)``; for
+    ``range_search`` also ``range_search_tensor`` / ``range_search_keys_tensor(q, radius, id_offset)`` and
+    ``range_merge(keys [world, stride], lims [world, nq + 1], total)``); by default they are the CUDA index and the
+    CUDA merge kernels and fail loudly without a GPU.
     """
 
     def __init__(self, d: int, group=None, device: Optional[int] = None,
-                 local_index=None, merge: Optional[Callable] = None, exchange: Optional[str] = None):
+                 local_index=None, merge: Optional[Callable] = None, exchange: Optional[str] = None,
+                 range_merge: Optional[Callable] = None):
         import os
         import torch.distributed as dist
         self.d = int(d)
@@ -233,6 +253,7 @@ class ShardedFlatIP:
             self.device = device
         self.local = local_index
         self._merge = merge
+        self._range_merge = range_merge or _cuda_range_merge
         self.id_offset = 0
         self.ntotal_global = 0
         self._keys = None          # [nq, k] local keys and [world, nq, k] gathered keys, reused across searches
@@ -348,10 +369,14 @@ class ShardedFlatIP:
         return self._elastic_window(i)
 
     def _elastic_window(self, i: int) -> int:
-        first = int(self._bounds[self.rank]) - self.id_offset
-        self.local.set_window(first, int(self._bounds[self.rank + 1] - self._bounds[self.rank]))
+        self._set_window()
         self._timer.start(i)
         return i
+
+    def _set_window(self) -> None:
+        """The local index scores the rows [bounds[r], bounds[r+1]) of the current elastic boundaries."""
+        first = int(self._bounds[self.rank]) - self.id_offset
+        self.local.set_window(first, int(self._bounds[self.rank + 1] - self._bounds[self.rank]))
 
     @property
     def ntotal(self) -> int:
@@ -405,6 +430,74 @@ class ShardedFlatIP:
         dist.all_gather_into_tensor(self._gathered.view(self.world * nq, k), self._keys, group=self.group)
         D, I = self._merge(self._gathered, k)
         return PendingSearch(D, I, None, None)
+
+    def range_search(self, q, radius: float):
+        """Exact range search over the rows of every rank: every row whose inner product with a query is strictly
+        greater than ``radius``.  q: [nq, d] tensor, the same on every rank (as for ``search``).  Returns tensors
+        (lims int64 [nq + 1], D float32, I int64 global ids) on q's device, identical on every rank; query i's hits
+        are ``D[lims[i]:lims[i+1]]``, descending, ties -> lower id.  Collective: every rank must call it.
+
+        Each rank scores the rows it would score in a search (the current elastic boundaries, or its block) and keeps
+        its hits as sorted packed keys (``range_search_keys_tensor``).  One all-gather carries every rank's ``lims``
+        with a status, nq and the radius, so every rank learns every run length -- and raises the same error when any
+        rank failed or was called with a different radius.  A second all-gather carries the runs, padded to the
+        longest; ``ivr_range_merge_keys_device`` merges them on the current stream.  A range search is not a timed
+        search: it leaves the elastic controller and ``balance_log`` alone.
+
+        The exchange always uses these collectives over ``group``, never the peer mailboxes (their slots are sized
+        for nq * k and pipelined).  So ``range_search`` may be called between ``search_async`` calls: its scoring
+        queues on the current stream behind theirs, it blocks the host until its run lengths are known, it takes no
+        mailbox slot, and the pending searches still complete in issue order."""
+        import torch
+        import torch.distributed as dist
+        if self._bounds is not None:
+            self._set_window()
+        if self.world == 1:
+            return self.local.range_search_tensor(q, radius, id_offset=self.id_offset)
+        nq, dev = q.shape[0], q.device
+        if nq == 0:                                      # replicated queries: every rank takes this branch
+            return (torch.zeros(1, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.float32, device=dev),
+                    torch.empty(0, dtype=torch.int64, device=dev))
+        # every rank reaches both collectives whatever happens locally: a local failure travels as a status
+        err, rbits = None, 0
+        try:
+            rbits = int(np.float32(radius).view(np.int32))
+            lims, keys = self.local.range_search_keys_tensor(q, radius, id_offset=self.id_offset)
+        except Exception as e:
+            err = e
+            lims, keys = torch.zeros(nq + 1, dtype=torch.int64, device=dev), None
+        # a batch of another size would also change the row length: queries must be replicated, as for search
+        row = torch.cat([lims, torch.tensor([0 if err is None else 1, nq, rbits], dtype=torch.int64, device=dev)])
+        rows = torch.empty((self.world, nq + 4), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(rows.view(-1), row, group=self.group)
+        host = rows.cpu().numpy()
+        failed = np.nonzero(host[:, nq + 1])[0]
+        if failed.size:
+            raise RuntimeError(f"range_search failed on rank {int(failed[0])}") from err
+        differ = np.nonzero((host[:, nq + 2] != host[0, nq + 2]) | (host[:, nq + 3] != host[0, nq + 3]))[0]
+        if differ.size:
+            def call(r):
+                return f"nq={int(host[r, nq + 2])} radius={float(np.int32(host[r, nq + 3]).view(np.float32))}"
+            raise ValueError(f"range_search: rank {int(differ[0])} was called with {call(int(differ[0]))}, "
+                             f"rank 0 with {call(0)}")
+        totals = host[:, nq]
+        stride = int(totals.max())
+        gathered = torch.empty((self.world, 0), dtype=torch.int64, device=dev)
+        if stride > 0:                                   # every rank knows stride: all skip or all gather
+            fail = self.world
+            try:
+                gathered = torch.empty((self.world, stride), dtype=torch.int64, device=dev)
+                mine = torch.empty(stride, dtype=torch.int64, device=dev)
+                mine[:keys.numel()] = keys
+            except RuntimeError:                         # torch.OutOfMemoryError included
+                fail = self.rank
+            flag = torch.tensor([fail], dtype=torch.int64, device=dev)
+            dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
+            if int(flag.item()) < self.world:
+                raise RuntimeError(f"range_search: rank {int(flag.item())} cannot allocate the exchange buffers "
+                                   f"({self.world} x {stride} keys)")
+            dist.all_gather_into_tensor(gathered.view(-1), mine, group=self.group)
+        return self._range_merge(gathered, rows[:, :nq + 1].contiguous(), int(totals.sum()))
 
     # ---- peer-memory exchange (csrc/exchange.cu) ---------------------------
     def _ensure_mailbox(self, n_entries: int, device) -> bool:
