@@ -99,6 +99,15 @@ static int require_device(int device) {
     return IVR_OK;
 }
 
+// require_device() with its capability probe done once per thread and device, for entry points called per search
+static int require_device_once(int device) {
+    static thread_local int checked_device = -1;
+    if (checked_device == device) { IVR_CUDA(cudaSetDevice(device)); return IVR_OK; }
+    IVR_TRY(require_device(device));
+    checked_device = device;
+    return IVR_OK;
+}
+
 // Scoped device buffer for the host-pointer dedup / normalise entry points.  Stream-ordered allocation from the
 // device's default memory pool, whose release threshold require_device() raises to "never": after the first call
 // the blocks come back from the pool without a driver allocation (a cudaMalloc / cudaFree pair per call used to cost
@@ -459,6 +468,16 @@ static int range_args(const ivr_index* idx, const void* q, int64_t nq, float rad
     return IVR_OK;
 }
 
+// Exchange keys hold a 32-bit row: the global ids id_offset + [0, ntotal) must fit.
+static int check_key_ids(const ivr_index* idx, int64_t id_offset, const char* who) {
+    if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
+        set_error("%s: global row ids must stay below 2^32 (offset %lld + %lld rows)", who,
+                  static_cast<long long>(id_offset), static_cast<long long>(idx->ntotal));
+        return IVR_EUNSUPPORTED;
+    }
+    return IVR_OK;
+}
+
 }  // namespace ivr
 
 extern "C" {
@@ -479,11 +498,7 @@ int ivr_index_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq,
         set_error("search_keys: bad argument");
         return IVR_EINVAL;
     }
-    if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
-        set_error("search_keys: global row ids must stay below 2^32 (offset %lld + %lld rows)",
-                  static_cast<long long>(id_offset), static_cast<long long>(idx->ntotal));
-        return IVR_EUNSUPPORTED;
-    }
+    IVR_TRY(check_key_ids(idx, id_offset, "search_keys"));
     return search_device_impl(idx, q_dev, nq, k, nullptr, reinterpret_cast<int64_t*>(keys_dev), id_offset, path,
                               static_cast<cudaStream_t>(stream));
 }
@@ -502,22 +517,23 @@ int ivr_index_search(ivr_index* idx, const float* q_host, int64_t nq, int k, flo
     const size_t qb = static_cast<size_t>(nq) * idx->dim * sizeof(float);
     const size_t db = static_cast<size_t>(nq) * k * sizeof(float);
     const size_t ib = static_cast<size_t>(nq) * k * sizeof(int64_t);
-    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
-    IVR_TRY(ensure_pin(idx, up(qb) + up(db) + up(ib)));
+    Carve carve;                                                    // the same layout in the pinned and the device buffer
+    const size_t o_q = carve(qb), o_d = carve(db), o_i = carve(ib);
+    IVR_TRY(ensure_pin(idx, carve.size));
     char* pin = static_cast<char*>(idx->pin);
-    IVR_TRY(ensure_io(idx, up(qb) + up(db) + up(ib)));
+    IVR_TRY(ensure_io(idx, carve.size));
     char* io = static_cast<char*>(idx->io);
-    float* dq = reinterpret_cast<float*>(io);
-    float* dd = reinterpret_cast<float*>(io + up(qb));
-    int64_t* di = reinterpret_cast<int64_t*>(io + up(qb) + up(db));
-    memcpy(pin, q_host, qb);
-    IVR_CUDA(cudaMemcpyAsync(dq, pin, qb, cudaMemcpyHostToDevice, st));
+    float* dq = reinterpret_cast<float*>(io + o_q);
+    float* dd = reinterpret_cast<float*>(io + o_d);
+    int64_t* di = reinterpret_cast<int64_t*>(io + o_i);
+    memcpy(pin + o_q, q_host, qb);
+    IVR_CUDA(cudaMemcpyAsync(dq, pin + o_q, qb, cudaMemcpyHostToDevice, st));
     IVR_TRY(search_device_impl(idx, dq, nq, k, dd, di, 0, path, st));
-    IVR_CUDA(cudaMemcpyAsync(pin + up(qb), dd, db, cudaMemcpyDeviceToHost, st));
-    IVR_CUDA(cudaMemcpyAsync(pin + up(qb) + up(db), di, ib, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_d, dd, db, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_i, di, ib, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaStreamSynchronize(st));
-    memcpy(D_host, pin + up(qb), db);
-    memcpy(I_host, pin + up(qb) + up(db), ib);
+    memcpy(D_host, pin + o_d, db);
+    memcpy(I_host, pin + o_i, ib);
     return IVR_OK;
 }
 
@@ -538,11 +554,7 @@ int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq
 int ivr_index_range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
                                        int64_t* lims_dev, uint64_t* keys_dev, int64_t id_offset, void* stream) {
     IVR_TRY(range_args(idx, q_dev, nq, radius, capacity, lims_dev, keys_dev, keys_dev));
-    if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
-        set_error("range_search_keys: global row ids must stay below 2^32 (offset %lld + %lld rows)",
-                  static_cast<long long>(id_offset), static_cast<long long>(idx->ntotal));
-        return IVR_EUNSUPPORTED;
-    }
+    IVR_TRY(check_key_ids(idx, id_offset, "range_search_keys"));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (nq == 0) {
         IVR_CUDA(cudaSetDevice(idx->device));
@@ -560,35 +572,39 @@ int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, floa
     if (nq == 0) { lims_host[0] = 0; return IVR_OK; }
     IVR_CUDA(cudaSetDevice(idx->device));
     cudaStream_t st = idx->stream;
-    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
     const size_t qb = static_cast<size_t>(nq) * idx->dim * sizeof(float);
     const size_t lb = static_cast<size_t>(nq + 1) * sizeof(int64_t);
     const size_t db = static_cast<size_t>(capacity) * sizeof(float), ib = static_cast<size_t>(capacity) * sizeof(int64_t);
-    IVR_TRY(ensure_pin(idx, up(qb) + up(lb)));
-    IVR_TRY(ensure_io(idx, up(qb) + up(lb) + up(db) + up(ib)));
+    Carve carve;                                                    // the pinned buffer holds the first two parts
+    const size_t o_q = carve(qb), o_l = carve(lb);
+    IVR_TRY(ensure_pin(idx, carve.size));
+    const size_t o_d = carve(db), o_i = carve(ib);
+    IVR_TRY(ensure_io(idx, carve.size));
     char* pin = static_cast<char*>(idx->pin);
     char* io = static_cast<char*>(idx->io);
-    float* dq = reinterpret_cast<float*>(io);
-    int64_t* dl = reinterpret_cast<int64_t*>(io + up(qb));
-    float* dd = reinterpret_cast<float*>(io + up(qb) + up(lb));
-    int64_t* di = reinterpret_cast<int64_t*>(io + up(qb) + up(lb) + up(db));
-    memcpy(pin, q_host, qb);
-    IVR_CUDA(cudaMemcpyAsync(dq, pin, qb, cudaMemcpyHostToDevice, st));
+    float* dq = reinterpret_cast<float*>(io + o_q);
+    int64_t* dl = reinterpret_cast<int64_t*>(io + o_l);
+    float* dd = reinterpret_cast<float*>(io + o_d);
+    int64_t* di = reinterpret_cast<int64_t*>(io + o_i);
+    memcpy(pin + o_q, q_host, qb);
+    IVR_CUDA(cudaMemcpyAsync(dq, pin + o_q, qb, cudaMemcpyHostToDevice, st));
     IVR_TRY(ivr_index_range_search_device(idx, dq, nq, radius, capacity, dl, dd, di, 0, st));
-    IVR_CUDA(cudaMemcpyAsync(pin + up(qb), dl, lb, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_l, dl, lb, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaStreamSynchronize(st));
-    memcpy(lims_host, pin + up(qb), lb);
+    memcpy(lims_host, pin + o_l, lb);
     const int64_t total = lims_host[nq];
     if (total == 0 || total > capacity) return IVR_OK;              // nothing to copy / the caller retries
     // the hits, through the pinned buffer sized to what was found
     const size_t hd = static_cast<size_t>(total) * sizeof(float), hi = static_cast<size_t>(total) * sizeof(int64_t);
-    IVR_TRY(ensure_pin(idx, up(hd) + up(hi)));
+    Carve hits;
+    const size_t o_hd = hits(hd), o_hi = hits(hi);
+    IVR_TRY(ensure_pin(idx, hits.size));
     pin = static_cast<char*>(idx->pin);
-    IVR_CUDA(cudaMemcpyAsync(pin, dd, hd, cudaMemcpyDeviceToHost, st));
-    IVR_CUDA(cudaMemcpyAsync(pin + up(hd), di, hi, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_hd, dd, hd, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_hi, di, hi, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaStreamSynchronize(st));
-    staged_memcpy(D_host, pin, hd);
-    staged_memcpy(I_host, pin + up(hd), hi);
+    staged_memcpy(D_host, pin + o_hd, hd);
+    staged_memcpy(I_host, pin + o_hi, hi);
     return IVR_OK;
 }
 
@@ -655,9 +671,7 @@ int ivr_topk_merge_keys_device(int device, const uint64_t* keys_parts, int n_par
         return IVR_EUNSUPPORTED;
     }
     if (nq == 0) return IVR_OK;
-    static thread_local int checked_device = -1;       // the capability probe is done once per thread and device
-    if (checked_device != device) { IVR_TRY(require_device(device)); checked_device = device; }
-    else IVR_CUDA(cudaSetDevice(device));
+    IVR_TRY(require_device_once(device));
     MergeIn in{};
     in.entries = keys_parts; in.counts = nullptr;
     in.list_stride = nq * k; in.q_stride = k;
@@ -677,9 +691,7 @@ int ivr_range_merge_keys_device(int device, const uint64_t* keys_parts, int64_t 
         set_error("range_merge_keys: n_parts * part_stride or n_parts * (nq + 1) overflows");
         return IVR_EINVAL;
     }
-    static thread_local int checked_device = -1;       // the capability probe is done once per thread and device
-    if (checked_device != device) { IVR_TRY(require_device(device)); checked_device = device; }
-    else IVR_CUDA(cudaSetDevice(device));
+    IVR_TRY(require_device_once(device));
     return range_merge_keys_device(keys_parts, part_stride, lims_parts, n_parts, nq, lims, D, I,
                                    static_cast<cudaStream_t>(stream));
 }

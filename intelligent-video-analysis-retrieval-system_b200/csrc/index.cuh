@@ -3,6 +3,12 @@
 
 #include "common.cuh"
 
+namespace ivr {
+// Event slots of the search timing (ivr_index_last_timing): interval i runs from ev[2i] to ev[2i + 1], so
+// score_ms = scoring launches, merge_ms = the final merge, prep_ms = query preparation.
+enum TimingMark { kScoreBegin = 0, kScoreEnd = 1, kMergeBegin = 2, kMergeEnd = 3, kPrepBegin = 4, kPrepEnd = 5 };
+}  // namespace ivr
+
 struct ivr_index {
     int      dim      = 0;        // logical dimension (as given by the caller)
     int      dpad     = 0;        // storage dimension: dim padded to a multiple of 64
@@ -42,7 +48,7 @@ struct ivr_index {
 
     // timing of the last device search
     bool        timing = false;
-    cudaEvent_t ev[6]  = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    cudaEvent_t ev[6]  = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // indexed by ivr::TimingMark
     bool        ev_valid[3] = {false, false, false};
     int         launches[3] = {0, 0, 0};
     int         last_path = 0;
@@ -55,6 +61,17 @@ int  ensure_ws(ivr_index* idx, size_t bytes);
 int  ensure_pin(ivr_index* idx, size_t bytes);
 int  ensure_io(ivr_index* idx, size_t bytes);
 int  ensure_capacity(ivr_index* idx, int64_t rows, cudaStream_t st, bool exact = false);
+
+// Records timing mark m of the current search on st when `timed`.
+inline void timing_mark(ivr_index* idx, bool timed, TimingMark m, cudaStream_t st) {
+    if (timed) cudaEventRecord(idx->ev[m], st);
+}
+
+// Consecutive 256-byte-aligned parts of one buffer: carve(bytes) returns the next part's offset, `size` the total.
+struct Carve {
+    size_t size = 0;
+    size_t operator()(size_t bytes) { const size_t o = size; size += (bytes + 255) / 256 * 256; return o; }
+};
 
 // search back-ends (search_stream.cu / search_mma.cu / topk_merge.cu)
 int search_stream(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,

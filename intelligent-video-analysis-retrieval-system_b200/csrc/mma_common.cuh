@@ -364,10 +364,45 @@ static int env_int(const char* name, int dflt) {
     return (e && *e) ? atoi(e) : dflt;
 }
 
-// shared by the batched and the small-batch host paths (defined in search_mma.cu)
+// ---- shared by the batched, the small-batch and the range host paths (defined in search_mma.cu) ----
 int launch_queries_to_f16(const float* q, __half* out, float* scale, uint32_t* tau_g, int64_t nq, int64_t nq_pad,
                           int dim, int dpad, cudaStream_t st);
-int launch_seed_tau(const uint64_t* keys, const int* counts, uint32_t* tau_g, int64_t nq, int k, cudaStream_t st);
+// The TMA descriptor of the (windowed) row matrix in box_rows-row boxes, cached on the handle until the rows move,
+// grow or the box changes.
+int row_tmap(ivr_index* idx, int box_rows, const CUtensorMap** tmx);
+// Queries to fp16 [nq_pad, dpad] with their scales and -inf thresholds, bracketed by the prep timing marks, then
+// their TMA descriptor in box_rows-row boxes.  `zero_bytes` at `zero` are cleared inside the bracket.
+int prepare_queries(ivr_index* idx, bool timed, const float* q_dev, int64_t nq, int64_t nq_pad, __half* q_h,
+                    float* q_scale, uint32_t* tau_g, int box_rows, CUtensorMap* tmq, cudaStream_t st,
+                    void* zero = nullptr, size_t zero_bytes = 0);
+
+// A batch searched in n seeded launches: after each scoring launch, fold_launch(seq, ph, lists) merges its candidate
+// lists -- straight into D / I when n == 1, otherwise into per-launch keys whose exact k-th best score per query
+// raises the shared thresholds (tau_g) of the next launch; finish_launches merges the per-launch keys into D / I.
+// The caller marks kScoreBegin before the first scoring launch; the scoring launches are bracketed together, so with
+// several launches the (tiny) merges between them count as score_ms.
+struct LaunchSeq {
+    ivr_index*   idx;
+    cudaStream_t st;
+    bool         timed;
+    int64_t      nq;
+    int          k, n;                       // n = number of launches
+    float*       D;
+    int64_t*     I;
+    int64_t      id_offset;
+    // workspace: fp16 queries [nq_pad, dpad], their scales and thresholds [nq_pad], per-launch keys [n][nq][k] and
+    // counts [n][nq], merge scratch for up to max_lists lists per query, then the caller's own part
+    __half*   q_h;
+    float*    q_scale;
+    uint32_t* tau_g;
+    uint64_t* keys, *tmp_e;
+    int*      counts, *tmp_c;
+    char*     own;
+};
+// Lays out the workspace of a sequence whose first nine fields are set, with own_bytes for the caller at seq->own.
+int begin_launches(LaunchSeq* seq, int64_t nq_pad, int max_lists, size_t own_bytes);
+int fold_launch(LaunchSeq& seq, int ph, const MergeIn& lists);
+int finish_launches(LaunchSeq& seq);
 
 // small-batch kernel (search_mma_small.cu)
 int  search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,

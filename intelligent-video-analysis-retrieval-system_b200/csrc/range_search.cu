@@ -100,8 +100,7 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
                                                           static_cast<uint64_t*>(nullptr), items, static_cast<int>(nq),
                                                           static_cast<const int64_t*>(nullptr),
                                                           static_cast<const int64_t*>(nullptr), st));
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    Carve carve;
     const size_t o_q   = carve(static_cast<size_t>(chunk) * idx->dpad * 2);
     const size_t o_sc  = carve(static_cast<size_t>(n_chunks) * chunk * 4);
     const size_t o_tg  = carve(static_cast<size_t>(chunk) * 4);
@@ -112,7 +111,7 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
     const size_t o_seg = carve(static_cast<size_t>(capacity) * 8);
     const size_t o_srt = carve(static_cast<size_t>(capacity) * 8);
     const size_t o_tmp = carve(std::max(scan_bytes, sort_bytes));
-    IVR_TRY(ensure_ws(idx, off));
+    IVR_TRY(ensure_ws(idx, carve.size));
     char* ws = static_cast<char*>(idx->ws);
     __half* q_h = reinterpret_cast<__half*>(ws + o_q);
     float* q_scale = reinterpret_cast<float*>(ws + o_sc);

@@ -653,9 +653,82 @@ int launch_queries_to_f16(const float* q, __half* out, float* scale, uint32_t* t
     IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }
-int launch_seed_tau(const uint64_t* keys, const int* counts, uint32_t* tau_g, int64_t nq, int k, cudaStream_t st) {
-    seed_tau_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, st>>>(keys, counts, tau_g, nq, k);
-    IVR_CUDA(cudaGetLastError());
+
+int row_tmap(ivr_index* idx, int box_rows, const CUtensorMap** tmx) {
+    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != box_rows) {
+        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, box_rows));
+        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = box_rows;
+    }
+    *tmx = reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    return IVR_OK;
+}
+
+int prepare_queries(ivr_index* idx, bool timed, const float* q_dev, int64_t nq, int64_t nq_pad, __half* q_h,
+                    float* q_scale, uint32_t* tau_g, int box_rows, CUtensorMap* tmq, cudaStream_t st,
+                    void* zero, size_t zero_bytes) {
+    timing_mark(idx, timed, kPrepBegin, st);
+    IVR_TRY(launch_queries_to_f16(q_dev, q_h, q_scale, tau_g, nq, nq_pad, idx->dim, idx->dpad, st));
+    if (zero_bytes) IVR_CUDA(cudaMemsetAsync(zero, 0, zero_bytes, st));
+    idx->launches[2]++;
+    timing_mark(idx, timed, kPrepEnd, st);
+    return make_tmap(tmq, q_h, nq_pad, idx->dpad, box_rows);
+}
+
+int begin_launches(LaunchSeq* seq, int64_t nq_pad, int max_lists, size_t own_bytes) {
+    const int64_t nq = seq->nq;
+    const int k = seq->k;
+    Carve carve;
+    const size_t o_q  = carve(static_cast<size_t>(nq_pad) * seq->idx->dpad * 2);
+    const size_t o_sc = carve(static_cast<size_t>(nq_pad) * 4);
+    const size_t o_tg = carve(static_cast<size_t>(nq_pad) * 4);
+    const size_t o_pk = carve(static_cast<size_t>(seq->n) * nq * k * 8);
+    const size_t o_pc = carve(static_cast<size_t>(seq->n) * nq * 4);
+    const size_t o_t  = carve(merge_tmp_entries(max_lists, nq, k) * 8);
+    const size_t o_tc = carve((static_cast<size_t>(max_lists) * nq + 64) * 4);
+    const size_t o_own = carve(own_bytes);
+    IVR_TRY(ensure_ws(seq->idx, carve.size));
+    char* ws = static_cast<char*>(seq->idx->ws);
+    seq->q_h = reinterpret_cast<__half*>(ws + o_q);
+    seq->q_scale = reinterpret_cast<float*>(ws + o_sc);
+    seq->tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
+    seq->keys = reinterpret_cast<uint64_t*>(ws + o_pk);
+    seq->counts = reinterpret_cast<int*>(ws + o_pc);
+    seq->tmp_e = reinterpret_cast<uint64_t*>(ws + o_t);
+    seq->tmp_c = reinterpret_cast<int*>(ws + o_tc);
+    seq->own = ws + o_own;
+    return IVR_OK;
+}
+
+int fold_launch(LaunchSeq& s, int ph, const MergeIn& lists) {
+    if (s.n == 1) {
+        timing_mark(s.idx, s.timed, kScoreEnd, s.st); timing_mark(s.idx, s.timed, kMergeBegin, s.st);
+        return merge_lists_final(lists, s.nq, s.k, s.D, s.I, s.id_offset, s.tmp_e, s.tmp_c, s.st, &s.idx->launches[1],
+                                 s.q_scale);
+    }
+    uint64_t* keys = s.keys + static_cast<size_t>(ph) * s.nq * s.k;
+    int* counts = s.counts + static_cast<size_t>(ph) * s.nq;
+    IVR_TRY(merge_lists_keys(lists, s.nq, s.k, keys, counts, s.tmp_e, s.tmp_c, s.st, &s.idx->launches[1]));
+    if (ph + 1 < s.n) {
+        // the k-th best of this launch: tau_g already holds the earlier launches' (atomicMax: the seed can only rise)
+        seed_tau_kernel<<<static_cast<unsigned>((s.nq + 255) / 256), 256, 0, s.st>>>(keys, counts, s.tau_g, s.nq, s.k);
+        IVR_CUDA(cudaGetLastError());
+        s.idx->launches[1]++;
+    }
+    return IVR_OK;
+}
+
+int finish_launches(LaunchSeq& s) {
+    if (s.n > 1) {
+        timing_mark(s.idx, s.timed, kScoreEnd, s.st); timing_mark(s.idx, s.timed, kMergeBegin, s.st);
+        MergeIn in{};
+        in.entries = s.keys; in.counts = s.counts;
+        in.list_stride = s.nq * s.k; in.q_stride = s.k; in.cnt_list_stride = s.nq; in.cnt_q_stride = 1;
+        in.n_lists = s.n; in.fixed_count = 0; in.raw = 0;
+        IVR_TRY(merge_lists_final(in, s.nq, s.k, s.D, s.I, s.id_offset, s.tmp_e, s.tmp_c, s.st, &s.idx->launches[1],
+                                  s.q_scale));
+    }
+    timing_mark(s.idx, s.timed, kMergeEnd, s.st);
+    if (s.timed) s.idx->ev_valid[0] = s.idx->ev_valid[1] = s.idx->ev_valid[2] = true;
     return IVR_OK;
 }
 
@@ -804,52 +877,51 @@ static int launch_cluster(Kern kern, const CUtensorMap& tq, const CUtensorMap& t
     return IVR_OK;
 }
 
+// The instantiations run_plan picks from, in the order they are instantiated (the order of the kernels in the
+// module, which can change their register allocation): search_mma_xres_kernel<E, TN> by
+// [(256 - TN) / 32][E == 0] for the tile heights of xres_tile_rows(), search_mma_kernel<CG, E> by [2 - CG][E == 0].
+using XresKernel = void (*)(const CUtensorMap, const CUtensorMap, const XresParams);
+using QresKernel = void (*)(const CUtensorMap, const CUtensorMap, const MmaParams);
+static const XresKernel kXresKernels[5][2] = {
+    {search_mma_xres_kernel<8, 256>, search_mma_xres_kernel<0, 256>},
+    {search_mma_xres_kernel<8, 224>, search_mma_xres_kernel<0, 224>},
+    {search_mma_xres_kernel<8, 192>, search_mma_xres_kernel<0, 192>},
+    {search_mma_xres_kernel<8, 160>, search_mma_xres_kernel<0, 160>},
+    {search_mma_xres_kernel<8, 128>, search_mma_xres_kernel<0, 128>}};
+static const QresKernel kQresKernels[2][2] = {{search_mma_kernel<2, 8>, search_mma_kernel<2, 0>},
+                                              {search_mma_kernel<1, 8>, search_mma_kernel<1, 0>}};
+
 // Runs one planned launch with its scratch at `lists` / `aux`; fills `in` for the merge kernel.
 static int run_plan(Plan& pl, const CUtensorMap& tmq, const CUtensorMap& tmx, uint32_t* tau_g, char* lists, char* aux,
-                    int k, cudaStream_t st, MergeIn* in) {
-    *in = MergeIn{};
+                    cudaStream_t st, MergeIn* in) {
+    const int e0 = pl.E != 8;
+    int64_t nq_pad;
+    int C;
+    int* counts;
     if (pl.xres) {
         XresParams& p = pl.x;
         p.tau_g = tau_g;
         p.lists = reinterpret_cast<uint64_t*>(lists);
-        p.counts = reinterpret_cast<int*>(aux);
+        p.counts = counts = reinterpret_cast<int*>(aux);
         IVR_CUDA(cudaMemsetAsync(p.counts, 0, static_cast<size_t>(pl.n_lists) * p.nq_pad * 4, st));
-        int rc;
-        if (p.tn == 256) rc = pl.E == 8 ? launch_cluster(search_mma_xres_kernel<8, 256>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                        : launch_cluster(search_mma_xres_kernel<0, 256>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        else if (p.tn == 192) rc = pl.E == 8 ? launch_cluster(search_mma_xres_kernel<8, 192>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                             : launch_cluster(search_mma_xres_kernel<0, 192>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        else if (p.tn == 224) rc = pl.E == 8 ? launch_cluster(search_mma_xres_kernel<8, 224>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                             : launch_cluster(search_mma_xres_kernel<0, 224>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        else if (p.tn == 160) rc = pl.E == 8 ? launch_cluster(search_mma_xres_kernel<8, 160>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                             : launch_cluster(search_mma_xres_kernel<0, 160>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        else             rc = pl.E == 8 ? launch_cluster(search_mma_xres_kernel<8, 128>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                        : launch_cluster(search_mma_xres_kernel<0, 128>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        IVR_TRY(rc);
-        in->entries = p.lists; in->counts = p.counts;
-        in->list_stride = static_cast<int64_t>(p.nq_pad) * p.C; in->q_stride = p.C;
-        in->cnt_list_stride = p.nq_pad; in->cnt_q_stride = 1;
-        in->n_lists = pl.n_lists; in->fixed_count = 0; in->raw = 1; in->interleave = 1;
+        IVR_TRY(launch_cluster(kXresKernels[(256 - p.tn) / 32][e0], tmq, tmx, p, pl.grid, 2, pl.smem, st));
+        nq_pad = p.nq_pad; C = p.C;
     } else {
         MmaParams& p = pl.q;
         p.tau_g = tau_g;
         p.lists = reinterpret_cast<uint64_t*>(lists);
-        size_t off = 0;
-        auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return aux + o; };
-        p.state = reinterpret_cast<int2*>(carve(static_cast<size_t>(pl.grid) * p.segs_max * 2 * kTileQ * sizeof(int2)));
-        p.counts = reinterpret_cast<int*>(carve(static_cast<size_t>(pl.n_lists) * p.nq_pad * 4));
+        Carve carve;
+        p.state = reinterpret_cast<int2*>(aux + carve(static_cast<size_t>(pl.grid) * p.segs_max * 2 * kTileQ * sizeof(int2)));
+        p.counts = counts = reinterpret_cast<int*>(aux + carve(static_cast<size_t>(pl.n_lists) * p.nq_pad * 4));
         IVR_CUDA(cudaMemsetAsync(p.counts, 0, static_cast<size_t>(pl.n_lists) * p.nq_pad * 4, st));
-        int rc;
-        if (pl.cg == 2) rc = pl.E == 8 ? launch_cluster(search_mma_kernel<2, 8>, tmq, tmx, p, pl.grid, 2, pl.smem, st)
-                                       : launch_cluster(search_mma_kernel<2, 0>, tmq, tmx, p, pl.grid, 2, pl.smem, st);
-        else            rc = pl.E == 8 ? launch_cluster(search_mma_kernel<1, 8>, tmq, tmx, p, pl.grid, 1, pl.smem, st)
-                                       : launch_cluster(search_mma_kernel<1, 0>, tmq, tmx, p, pl.grid, 1, pl.smem, st);
-        IVR_TRY(rc);
-        in->entries = p.lists; in->counts = p.counts;
-        in->list_stride = static_cast<int64_t>(p.nq_pad) * p.C; in->q_stride = p.C;
-        in->cnt_list_stride = p.nq_pad; in->cnt_q_stride = 1;
-        in->n_lists = pl.n_lists; in->fixed_count = 0; in->raw = 1; in->interleave = 1;
+        IVR_TRY(launch_cluster(kQresKernels[2 - pl.cg][e0], tmq, tmx, p, pl.grid, pl.cg, pl.smem, st));
+        nq_pad = p.nq_pad; C = p.C;
     }
+    *in = MergeIn{};
+    in->entries = reinterpret_cast<const uint64_t*>(lists); in->counts = counts;
+    in->list_stride = nq_pad * C; in->q_stride = C;
+    in->cnt_list_stride = nq_pad; in->cnt_q_stride = 1;
+    in->n_lists = pl.n_lists; in->fixed_count = 0; in->raw = 1; in->interleave = 1;
     return IVR_OK;
 }
 
@@ -908,78 +980,25 @@ static int search_mma_batch(ivr_index* idx, const float* q_dev, int64_t nq, int 
         aux_bytes = std::max(aux_bytes, plan[ph].aux_bytes);
         max_lists = std::max(max_lists, plan[ph].n_lists);
     }
-    // workspace carve-up
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t o_q  = carve(static_cast<size_t>(nq_pad) * idx->dpad * 2);
-    const size_t o_sc = carve(static_cast<size_t>(nq_pad) * 4);
-    const size_t o_tg = carve(static_cast<size_t>(nq_pad) * 4);
-    const size_t o_l  = carve(list_bytes);
-    const size_t o_a  = carve(aux_bytes);
-    const size_t o_pk = carve(static_cast<size_t>(n_phases) * nq * k * 8);   // per-launch merged keys [phase][nq][k]
-    const size_t o_pc = carve(static_cast<size_t>(n_phases) * nq * 4);
-    const size_t tmp_keys = merge_tmp_entries(max_lists, nq, k);
-    const size_t o_t  = carve(tmp_keys * 8);
-    const size_t o_tc = carve((static_cast<size_t>(max_lists) * nq + 64) * 4);
-    IVR_TRY(ensure_ws(idx, off));
-    char* ws = static_cast<char*>(idx->ws);
-    __half* q_h = reinterpret_cast<__half*>(ws + o_q);
-    float* q_scale = reinterpret_cast<float*>(ws + o_sc);
-    uint32_t* tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
-    uint64_t* ph_keys = reinterpret_cast<uint64_t*>(ws + o_pk);
-    int* ph_counts = reinterpret_cast<int*>(ws + o_pc);
-    uint64_t* tmp_e = reinterpret_cast<uint64_t*>(ws + o_t);
-    int* tmp_c = reinterpret_cast<int*>(ws + o_tc);
-    const bool timed = idx->timing && first_batch;
+    Carve own;
+    const size_t o_l = own(list_bytes), o_a = own(aux_bytes);
+    LaunchSeq seq{idx, st, idx->timing && first_batch, nq, k, n_phases, D_dev, I_dev, id_offset};
+    IVR_TRY(begin_launches(&seq, nq_pad, max_lists, own.size));
 
-    if (timed) cudaEventRecord(idx->ev[4], st);
-    IVR_TRY(launch_queries_to_f16(q_dev, q_h, q_scale, tau_g, nq, nq_pad, idx->dim, idx->dpad, st));
-    idx->launches[2]++;
-    if (timed) cudaEventRecord(idx->ev[5], st);
-
-    // TMA descriptors (the row descriptor is cached until the matrix moves or grows)
-    const int box_rows = tile_rows / (xres ? 2 : cg);
     CUtensorMap tmq;
-    IVR_TRY(make_tmap(&tmq, q_h, nq_pad, idx->dpad, kTileQ));
-    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != box_rows) {
-        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, box_rows));
-        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = box_rows;
-    }
-    const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    const CUtensorMap* tmx;
+    const int box_rows = tile_rows / (xres ? 2 : cg);
+    IVR_TRY(prepare_queries(idx, seq.timed, q_dev, nq, nq_pad, seq.q_h, seq.q_scale, seq.tau_g, kTileQ, &tmq, st));
+    IVR_TRY(row_tmap(idx, box_rows, &tmx));
 
-    // scoring launches are bracketed together by ev[0]/ev[1]; the (tiny) per-phase merges run between
-    // them and are therefore included in "score_ms" when there are several launches
-    if (timed) cudaEventRecord(idx->ev[0], st);
+    timing_mark(idx, seq.timed, kScoreBegin, st);
     for (int ph = 0; ph < n_phases; ++ph) {
         MergeIn in;
-        IVR_TRY(run_plan(plan[ph], tmq, tmx, tau_g, ws + o_l, ws + o_a, k, st, &in));
+        IVR_TRY(run_plan(plan[ph], tmq, *tmx, seq.tau_g, seq.own + o_l, seq.own + o_a, st, &in));
         idx->launches[0]++;
-        if (n_phases == 1) {
-            if (timed) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
-            IVR_TRY(merge_lists_final(in, nq, k, D_dev, I_dev, id_offset, tmp_e, tmp_c, st, &idx->launches[1], q_scale));
-        } else {
-            IVR_TRY(merge_lists_keys(in, nq, k, ph_keys + static_cast<size_t>(ph) * nq * k,
-                                     ph_counts + static_cast<size_t>(ph) * nq, tmp_e, tmp_c, st, &idx->launches[1]));
-            if (ph + 1 < n_phases) {                               // atomicMax: the seed can only rise
-                IVR_TRY(launch_seed_tau(ph_keys + static_cast<size_t>(ph) * nq * k, ph_counts + static_cast<size_t>(ph) * nq,
-                                        tau_g, nq, k, st));
-                idx->launches[1]++;
-            }
-        }
+        IVR_TRY(fold_launch(seq, ph, in));
     }
-    if (n_phases > 1) {
-        if (timed) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
-        MergeIn in{};
-        in.entries = ph_keys; in.counts = ph_counts;
-        in.list_stride = nq * k; in.q_stride = k; in.cnt_list_stride = nq; in.cnt_q_stride = 1;
-        in.n_lists = n_phases; in.fixed_count = 0; in.raw = 0;
-        IVR_TRY(merge_lists_final(in, nq, k, D_dev, I_dev, id_offset, tmp_e, tmp_c, st, &idx->launches[1], q_scale));
-    }
-    if (timed) {
-        cudaEventRecord(idx->ev[3], st);
-        idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
-    }
-    return IVR_OK;
+    return finish_launches(seq);
 }
 
 int search_mma(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,

@@ -463,15 +463,6 @@ static bool small_shape(const ivr_index* idx, int64_t nq, int k, SmallShape* s) 
     return true;
 }
 
-// The TMA descriptor of the (windowed) row matrix in 128-row boxes, cached on the handle.
-static int small_row_tmap(ivr_index* idx) {
-    if (idx->tmap_rows_base != idx->rows || idx->tmap_rows_n != idx->ntotal || idx->tmap_rows_box != kSmallTileRows) {
-        IVR_TRY(make_tmap(reinterpret_cast<CUtensorMap*>(idx->tmap_rows), idx->rows, idx->ntotal, idx->dpad, kSmallTileRows));
-        idx->tmap_rows_base = idx->rows; idx->tmap_rows_n = idx->ntotal; idx->tmap_rows_box = kSmallTileRows;
-    }
-    return IVR_OK;
-}
-
 bool mma_small_supported(const ivr_index* idx, int64_t nq, int k) {
     SmallShape s;
     return small_shape(idx, nq, k, &s);
@@ -482,8 +473,7 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
                                  int64_t* I_dev, int64_t id_offset, cudaStream_t st) {
     const int64_t nt = (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
     const int64_t stride = nt * kSmallTileRows;                      // padded rows per query
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    Carve carve;
     const size_t o_q  = carve(static_cast<size_t>(sh.npad) * idx->dpad * 2);
     const size_t o_sc = carve(static_cast<size_t>(sh.npad) * 4);
     const size_t o_tg = carve(static_cast<size_t>(sh.npad) * 4);
@@ -492,7 +482,7 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
     const size_t zero_bytes = (static_cast<size_t>(sh.npad) * (nt + n_groups) + 2 * nq) * 4;   // tile + group maxima, pool counters, tickets
     const size_t o_z  = carve(zero_bytes);
     const size_t o_p  = carve(static_cast<size_t>(nq) * kSelectPoolCap * 8);
-    IVR_TRY(ensure_ws(idx, off));
+    IVR_TRY(ensure_ws(idx, carve.size));
     char* ws = static_cast<char*>(idx->ws);
     __half* q_h = reinterpret_cast<__half*>(ws + o_q);
     float* q_scale = reinterpret_cast<float*>(ws + o_sc);
@@ -502,16 +492,10 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
     int* pool_cnt = reinterpret_cast<int*>(group_max + static_cast<size_t>(sh.npad) * n_groups);
     const bool timed = idx->timing;
 
-    if (timed) cudaEventRecord(idx->ev[4], st);
-    IVR_TRY(launch_queries_to_f16(q_dev, q_h, q_scale, tau_g, nq, sh.npad, idx->dim, idx->dpad, st));
-    IVR_CUDA(cudaMemsetAsync(ws + o_z, 0, zero_bytes, st));
-    idx->launches[2]++;
-    if (timed) cudaEventRecord(idx->ev[5], st);
-
     CUtensorMap tmq;
-    IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
-    IVR_TRY(small_row_tmap(idx));
-    const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    const CUtensorMap* tmx;
+    IVR_TRY(prepare_queries(idx, timed, q_dev, nq, sh.npad, q_h, q_scale, tau_g, sh.npad, &tmq, st, ws + o_z, zero_bytes));
+    IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
     IVR_CUDA(cudaFuncSetAttribute(search_mma_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(sh.smem)));
     SmallParams p{};
@@ -523,21 +507,19 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
     p.dump = reinterpret_cast<float*>(ws + o_s); p.dump_stride = stride; p.tile_max = tile_max; p.n_tiles = nt;
     p.group_max = group_max; p.n_groups = n_groups;
     const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(nt, 1)));
-    if (timed) cudaEventRecord(idx->ev[0], st);
-    search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
+    timing_mark(idx, timed, kScoreBegin, st);
+    search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
     IVR_CUDA(cudaGetLastError());
     idx->launches[0]++;
-    if (timed) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
+    timing_mark(idx, timed, kScoreEnd, st); timing_mark(idx, timed, kMergeBegin, st);
     MergeIn in{};
     in.dense = p.dump; in.dense_q_stride = stride; in.dense_rows = idx->ntotal; in.dense_len = kSmallTileRows;
     in.cnt_list_stride = 1; in.cnt_q_stride = nt;                   // strides of the maxima array
     in.n_lists = static_cast<int>(nt);
     IVR_TRY(merge_select_final(in, tile_max, nq, k, D_dev, I_dev, id_offset, reinterpret_cast<uint64_t*>(ws + o_p),
                                pool_cnt, pool_cnt + nq, idx->sm_count, st, &idx->launches[1], q_scale, group_max, n_groups));
-    if (timed) {
-        cudaEventRecord(idx->ev[3], st);
-        idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
-    }
+    timing_mark(idx, timed, kMergeEnd, st);
+    if (timed) idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
     idx->last_kernel = "search_mma_small_kernel";
     return IVR_OK;
 }
@@ -574,52 +556,31 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
 
     const int max_grid = static_cast<int>(std::min<int64_t>(sms, std::max<int64_t>(nt, 1)));
     const int max_lists = std::max(4 * max_grid, 3);
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t o_q  = carve(static_cast<size_t>(sh.npad) * idx->dpad * 2);
-    const size_t o_sc = carve(static_cast<size_t>(sh.npad) * 4);
-    const size_t o_tg = carve(static_cast<size_t>(sh.npad) * 4);
-    const size_t o_l  = carve(static_cast<size_t>(max_lists) * sh.npad * sh.C * 8);
-    const size_t o_c  = carve(static_cast<size_t>(max_lists) * sh.npad * 4);
-    const size_t o_pk = carve(static_cast<size_t>(3) * nq * k * 8);      // per-launch merged keys [phase][nq][k]
-    const size_t o_pc = carve(static_cast<size_t>(3) * nq * 4);
-    const size_t o_t  = carve(merge_tmp_entries(max_lists, nq, k) * 8);
-    const size_t o_tc = carve((static_cast<size_t>(max_lists) * nq + 64) * 4);
-    IVR_TRY(ensure_ws(idx, off));
-    char* ws = static_cast<char*>(idx->ws);
-    __half* q_h = reinterpret_cast<__half*>(ws + o_q);
-    float* q_scale = reinterpret_cast<float*>(ws + o_sc);
-    uint32_t* tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
-    uint64_t* ph_keys = reinterpret_cast<uint64_t*>(ws + o_pk);
-    int* ph_counts = reinterpret_cast<int*>(ws + o_pc);
-    uint64_t* tmp_e = reinterpret_cast<uint64_t*>(ws + o_t);
-    int* tmp_c = reinterpret_cast<int*>(ws + o_tc);
-    const bool timed = idx->timing;
-
-    if (timed) cudaEventRecord(idx->ev[4], st);
-    IVR_TRY(launch_queries_to_f16(q_dev, q_h, q_scale, tau_g, nq, sh.npad, idx->dim, idx->dpad, st));
-    idx->launches[2]++;
-    if (timed) cudaEventRecord(idx->ev[5], st);
+    Carve own;
+    const size_t o_l = own(static_cast<size_t>(max_lists) * sh.npad * sh.C * 8);
+    const size_t o_c = own(static_cast<size_t>(max_lists) * sh.npad * 4);
+    LaunchSeq seq{idx, st, idx->timing, nq, k, n_phases, D_dev, I_dev, id_offset};
+    IVR_TRY(begin_launches(&seq, sh.npad, max_lists, own.size));
 
     CUtensorMap tmq;
-    IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
-    IVR_TRY(small_row_tmap(idx));
-    const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    const CUtensorMap* tmx;
+    IVR_TRY(prepare_queries(idx, seq.timed, q_dev, nq, sh.npad, seq.q_h, seq.q_scale, seq.tau_g, sh.npad, &tmq, st));
+    IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
     IVR_CUDA(cudaFuncSetAttribute(search_mma_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(sh.smem)));
 
-    if (timed) cudaEventRecord(idx->ev[0], st);
+    timing_mark(idx, seq.timed, kScoreBegin, st);
     for (int ph = 0; ph < n_phases; ++ph) {
         SmallParams p{};
         p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad; p.k = k; p.C = sh.C;
         p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
         p.tile0 = bounds[ph]; p.nt = bounds[ph + 1] - bounds[ph];
         p.row_policy = kL2EvictFirst;                                // every row is read exactly once
-        p.lists = reinterpret_cast<uint64_t*>(ws + o_l);
-        p.counts = reinterpret_cast<int*>(ws + o_c);
-        p.tau_g = tau_g;
+        p.lists = reinterpret_cast<uint64_t*>(seq.own + o_l);
+        p.counts = reinterpret_cast<int*>(seq.own + o_c);
+        p.tau_g = seq.tau_g;
         const int grid = static_cast<int>(std::min<int64_t>(sms, std::max<int64_t>(p.nt, 1)));
-        search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
+        search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
         IVR_CUDA(cudaGetLastError());
         idx->launches[0]++;
         MergeIn in{};
@@ -627,33 +588,9 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
         in.list_stride = static_cast<int64_t>(sh.npad) * sh.C; in.q_stride = sh.C;
         in.cnt_list_stride = sh.npad; in.cnt_q_stride = 1;
         in.n_lists = 4 * grid; in.fixed_count = 0; in.raw = 1;
-        if (n_phases == 1) {
-            if (timed) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
-            IVR_TRY(merge_lists_final(in, nq, k, D_dev, I_dev, id_offset, tmp_e, tmp_c, st, &idx->launches[1], q_scale));
-        } else {
-            IVR_TRY(merge_lists_keys(in, nq, k, ph_keys + static_cast<size_t>(ph) * nq * k,
-                                     ph_counts + static_cast<size_t>(ph) * nq, tmp_e, tmp_c, st, &idx->launches[1]));
-            if (ph + 1 < n_phases) {
-                // the k-th best so far: after launch 0 it is launch 0's; after launch 1 tau_g already holds
-                // launch 0's, so seeding with launch 1's own k-th best can only raise it
-                IVR_TRY(launch_seed_tau(ph_keys + static_cast<size_t>(ph) * nq * k, ph_counts + static_cast<size_t>(ph) * nq,
-                                        tau_g, nq, k, st));
-                idx->launches[1]++;
-            }
-        }
+        IVR_TRY(fold_launch(seq, ph, in));
     }
-    if (n_phases > 1) {
-        if (timed) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
-        MergeIn in{};
-        in.entries = ph_keys; in.counts = ph_counts;
-        in.list_stride = nq * k; in.q_stride = k; in.cnt_list_stride = nq; in.cnt_q_stride = 1;
-        in.n_lists = n_phases; in.fixed_count = 0; in.raw = 0;
-        IVR_TRY(merge_lists_final(in, nq, k, D_dev, I_dev, id_offset, tmp_e, tmp_c, st, &idx->launches[1], q_scale));
-    }
-    if (timed) {
-        cudaEventRecord(idx->ev[3], st);
-        idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
-    }
+    IVR_TRY(finish_launches(seq));
     idx->last_kernel = "search_mma_small_kernel";
     return IVR_OK;
 }
@@ -671,9 +608,9 @@ int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sca
         return IVR_EUNSUPPORTED;
     }
     CUtensorMap tmq;
+    const CUtensorMap* tmx;
     IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
-    IVR_TRY(small_row_tmap(idx));
-    const CUtensorMap& tmx = *reinterpret_cast<const CUtensorMap*>(idx->tmap_rows);
+    IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
     IVR_CUDA(cudaFuncSetAttribute(search_mma_small_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(sh.smem)));
     SmallRangeParams p{};
@@ -684,7 +621,7 @@ int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sca
     p.radius = radius; p.q_scale = q_scale; p.q_base = static_cast<uint32_t>(q_base);
     p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
     const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(p.nt, 1)));
-    search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
+    search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
     IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }

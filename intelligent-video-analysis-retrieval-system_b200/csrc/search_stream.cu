@@ -205,12 +205,11 @@ int search_stream(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* 
     const size_t tmp_keys = merge_tmp_entries(static_cast<int>(n_lists), kStreamMaxNq, k);
     const size_t cnt_ints = static_cast<size_t>(n_lists) * kStreamMaxNq * 2 + 1024;
     const bool select = k <= kSelectMaxK;             // one-launch merge by the list-maxima bound; exact radix levels above
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    Carve carve;
     const size_t o_l = carve(list_keys * 8), o_t = carve(tmp_keys * 8),
                  o_c = carve(cnt_ints * 4), o_m = carve(static_cast<size_t>(n_lists) * kStreamMaxNq * 4),
                  o_p = carve(static_cast<size_t>(kStreamMaxNq) * kSelectPoolCap * 8);
-    IVR_TRY(ensure_ws(idx, off));
+    IVR_TRY(ensure_ws(idx, carve.size));
     char* ws = static_cast<char*>(idx->ws);
     uint64_t* lists = reinterpret_cast<uint64_t*>(ws + o_l);
     uint64_t* tmp = reinterpret_cast<uint64_t*>(ws + o_t);
@@ -223,7 +222,8 @@ int search_stream(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* 
     for (int64_t q0 = 0; q0 < nq; q0 += kStreamMaxNq) {
         const int b_real = static_cast<int>(nq - q0 < kStreamMaxNq ? nq - q0 : kStreamMaxNq);
         const int b = (b_real == 3) ? 4 : b_real;             // kernel batch (3 is padded to 4)
-        if (idx->timing && q0 == 0) { cudaEventRecord(idx->ev[4], st); cudaEventRecord(idx->ev[5], st); cudaEventRecord(idx->ev[0], st); }
+        const bool timed = idx->timing && q0 == 0;         // the first batch; the kernel reads fp32 queries: no prep
+        timing_mark(idx, timed, kPrepBegin, st); timing_mark(idx, timed, kPrepEnd, st); timing_mark(idx, timed, kScoreBegin, st);
         int rc;
         switch (kcap) {
             case 128: rc = launch_stream_nq<8>(idx, b, b_real, q_dev + q0 * idx->dim, k, C, lists, counts, maxima, grid, st); break;   // k <= 128: register sort
@@ -231,7 +231,7 @@ int search_stream(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* 
         }
         IVR_TRY(rc);
         idx->launches[0]++;
-        if (idx->timing && q0 == 0) { cudaEventRecord(idx->ev[1], st); cudaEventRecord(idx->ev[2], st); }
+        timing_mark(idx, timed, kScoreEnd, st); timing_mark(idx, timed, kMergeBegin, st);
         MergeIn in{};
         in.entries = lists; in.counts = counts;
         in.list_stride = static_cast<int64_t>(b) * C; in.q_stride = C;
@@ -243,7 +243,7 @@ int search_stream(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* 
         else
             IVR_TRY(merge_lists_final(in, b_real, k, D_dev ? D_dev + q0 * k : nullptr, I_dev + q0 * k, id_offset, tmp,
                                       tmp_counts, st, &idx->launches[1]));
-        if (idx->timing && q0 == 0) cudaEventRecord(idx->ev[3], st);
+        timing_mark(idx, timed, kMergeEnd, st);
     }
     if (idx->timing) idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = true;
     return IVR_OK;
