@@ -88,7 +88,8 @@ int ensure_capacity(ivr_index* idx, int64_t rows, cudaStream_t st, bool exact) {
     return IVR_OK;
 }
 
-// fp32 [n, dim] -> fp16 [n, dpad] (round-to-nearest-even, saturating at +-65504, zero padded).
+// fp32 [n, dim] -> fp16 [n, dpad] (round-to-nearest-even, saturating at +-65504, zero padded).  NaN stays NaN:
+// such a row scores NaN against every query, and the searches never return a NaN score.
 // The reference only ever adds L2-normalised rows (unified_index.py:1776, core.py:1189-1196), for
 // which fp16 (11 significant bits) is 8x more accurate than bf16 at the same tensor-core rate.
 __global__ void rows_to_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst,
@@ -100,8 +101,8 @@ __global__ void rows_to_f16_kernel(const float* __restrict__ src, __half* __rest
         const int c = static_cast<int>(i % (dpad / 2)) * 2;
         float a = (c < dim) ? src[r * dim + c] : 0.f;
         float b = (c + 1 < dim) ? src[r * dim + c + 1] : 0.f;
-        a = fminf(fmaxf(a, -65504.f), 65504.f);
-        b = fminf(fmaxf(b, -65504.f), 65504.f);
+        if (!isnan(a)) a = fminf(fmaxf(a, -65504.f), 65504.f);
+        if (!isnan(b)) b = fminf(fmaxf(b, -65504.f), 65504.f);
         reinterpret_cast<__half2*>(dst)[i] = __floats2half2_rn(a, b);
     }
 }

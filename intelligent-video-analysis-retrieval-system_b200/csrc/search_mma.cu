@@ -612,7 +612,9 @@ search_mma_xres_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_
 
 // fp32 [nq, dim] -> fp16 [nq_pad, dpad] (zero padded), one warp per query.  Each query is scaled by
 // a power of two so that its largest component lies in [0.5, 1): exact, keeps fp16 in range for
-// any query norm, and is undone on the final scores (scale[q]).
+// any query norm, and is undone on the final scores (scale[q]).  The exponent is clamped to [-127, 127] so that
+// both 2^e and 2^-e are finite fp32: below 2^-128 the largest component lands under 0.5, from 2^128 * 0.5 up in
+// [1, 2); a zero or non-finite maximum keeps e = 0.
 __global__ void queries_to_f16_kernel(const float* __restrict__ q, __half* __restrict__ out,
                                       float* __restrict__ scale, uint32_t* __restrict__ tau_g,
                                       int64_t nq, int64_t nq_pad, int dim, int dpad) {
@@ -624,7 +626,10 @@ __global__ void queries_to_f16_kernel(const float* __restrict__ q, __half* __res
         for (int c = lane; c < dim; c += 32) mx = fmaxf(mx, fabsf(q[r * dim + c]));
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     int e = 0;
-    if (mx > 0.f && mx < 3.0e38f) frexpf(mx, &e);                 // mx = m * 2^e, m in [0.5, 1)
+    if (mx > 0.f && isfinite(mx)) {
+        frexpf(mx, &e);                                            // mx = m * 2^e, m in [0.5, 1)
+        e = min(max(e, -127), 127);
+    }
     const float down = ldexpf(1.0f, -e);
     for (int c = lane; c < dpad; c += 32)
         out[r * dpad + c] = __float2half_rn((r < nq && c < dim) ? q[r * dim + c] * down : 0.f);

@@ -239,7 +239,9 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
                         const uint32_t bits = valid ? v[i] : 0xff800000u;   // rows past the end: -inf
                         float* dst = p.dump + static_cast<int64_t>(c0 + i) * p.dump_stride + row;
                         *dst = __uint_as_float(bits);                    // 32 consecutive rows: one 128-byte store per query
-                        const uint32_t mx = __reduce_max_sync(0xffffffffu, f2ord(__uint_as_float(bits)));
+                        // the maxima bound the scores the merge keys, which skips NaN: a NaN counts as -inf here
+                        const uint32_t mb = (bits & 0x7fffffffu) > 0x7f800000u ? 0xff800000u : bits;
+                        const uint32_t mx = __reduce_max_sync(0xffffffffu, f2ord(__uint_as_float(mb)));
                         if (lane == 0) {
                             atomicMax(p.tile_max + static_cast<int64_t>(c0 + i) * p.n_tiles + tile, mx);
                             atomicMax(p.group_max + static_cast<int64_t>(c0 + i) * p.n_groups + grp, mx);
@@ -325,9 +327,22 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
 }
 
+// The largest fp32 t with fp32(t * scale) <= radius, so that "score > t" is exactly "the reported score, fp32(score *
+// scale), > radius".  scale is a power of two, so this is radius / scale whenever that division is exact; at the ends
+// of the float range the rescaled scores round (to subnormals or to inf) and the threshold moves to the rounding
+// boundary of radius instead: mid, between radius and the next float up, rounds to whichever is even.
+__device__ __forceinline__ float range_threshold(float radius, float scale) {
+    if (isinf(radius) && radius > 0.f) return radius;
+    const float up = nextafterf(radius, __int_as_float(0x7f800000));
+    const double mid = 0.5 * (static_cast<double>(radius) + (isinf(up) ? 0x1p128 : static_cast<double>(up)));
+    const double b = mid / static_cast<double>(scale);
+    float t = __double2float_rd(b);
+    if ((__float_as_uint(radius) & 1u) && static_cast<double>(t) == b) t = nextafterf(t, __int_as_float(0xff800000));
+    return t;
+}
+
 // RANGE mode: the same producer and MMA warps; the epilogue compares every score with a threshold that never moves
-// (radius / q_scale[q]: q_scale is a power of two, so the division is exact and "score > radius" survives it, except
-// at the ends of the float range) and appends the survivors to ONE hit pool shared by all CTAs and launches.  One
+// (range_threshold(radius, q_scale[q])) and appends the survivors to ONE hit pool shared by all CTAs and launches.  One
 // 64-bit cursor reservation per warp and 32-query chunk, no lists, no compaction, no counts.  Writes at or past
 // `capacity` are dropped, but the cursor still advances, so the true total is always known.
 struct SmallRangeParams {
@@ -355,7 +370,7 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
 
     small_setup(sm, &tmap_q, &tmap_x, p.stages, p.nbuf, warp, lane);
     for (int i = threadIdx.x; i < kSmallMaxQ; i += kSmallThreads)      // padded queries admit nothing
-        tau_s[i] = (i < p.nq) ? p.radius / p.q_scale[i] : __int_as_float(0x7f800000);
+        tau_s[i] = (i < p.nq) ? range_threshold(p.radius, p.q_scale[i]) : __int_as_float(0x7f800000);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();

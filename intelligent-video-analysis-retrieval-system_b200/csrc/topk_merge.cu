@@ -40,6 +40,11 @@ struct MergeOut {
     int64_t   nq;
 };
 
+// key of a materialised score; 0 (no key) for NaN, the score of a row holding a NaN, which is never returned
+__device__ __forceinline__ uint64_t dense_key(float score, int64_t row) {
+    return isnan(score) ? 0ull : make_key(score, static_cast<uint32_t>(row));
+}
+
 template <typename F>
 __device__ __forceinline__ void for_each_key(const MergeIn& in, int64_t q, int l0, int l1, F&& f) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
@@ -48,7 +53,8 @@ __device__ __forceinline__ void for_each_key(const MergeIn& in, int64_t q, int l
         for (int l = l0 + warp; l < l1; l += nwarps)
             for (int i = lane; i < in.dense_len; i += 32) {
                 const int64_t row = static_cast<int64_t>(l) * in.dense_len + i;
-                if (row < in.dense_rows) f(make_key(base[row], static_cast<uint32_t>(row)));
+                const uint64_t key = (row < in.dense_rows) ? dense_key(base[row], row) : 0ull;
+                if (key != 0ull) f(key);
             }
         return;
     }
@@ -472,7 +478,7 @@ merge_select_kernel(MergeIn in, MergeOut out, SelectArgs sa, int k, int kpad) {
                     if (in.dense) {
                         const int64_t row = static_cast<int64_t>(l) * in.dense_len + i;
                         if (i < cnt && row < in.dense_rows)
-                            key[u] = make_key(in.dense[q * in.dense_q_stride + row], static_cast<uint32_t>(row));
+                            key[u] = dense_key(in.dense[q * in.dense_q_stride + row], row);
                     } else if (i < cnt) {
                         key[u] = base[static_cast<int64_t>(i) * es];
                         if (in.raw) key[u] = make_key(__uint_as_float(static_cast<uint32_t>(key[u])), static_cast<uint32_t>(key[u] >> 32));
