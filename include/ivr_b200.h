@@ -131,6 +131,30 @@ IVR_API int ivr_index_range_search_keys_device(ivr_index* idx, const float* q_de
                                                int64_t capacity, int64_t* lims_dev, uint64_t* keys_dev,
                                                int64_t id_offset, void* stream);
 
+/* Exact range self-join: every pair of distinct stored rows whose inner product is strictly greater than `radius`.
+ * No reference call does this (the reference compares frames only within one scene or one folder); it finds the
+ * same footage across videos: a shared intro, advert or news segment, or a re-upload.  The rows joined are those of
+ * the search window (ivr_index_set_window), or all rows; call their count n.
+ *   lims   int64   [n + 1]    row i's hits (i = position in the window) are D[lims[i] : lims[i+1]], I[...]
+ *   D      float32 [capacity] scores, descending within a row (ties -> lower id)
+ *   I      int64   [capacity] stored row ids (window first + position)
+ * Row i's hits are the rows j != i with score(i, j) > radius, score = the fp32 tensor-core inner product of the two
+ * stored fp16 rows (no query scaling).  Each pair is scored once, so the result is symmetric with equal score bits
+ * both ways.  A row holding a NaN is never a hit and has no hits.  Apart from the diagonal, the result equals
+ * ivr_index_range_search over the window's reconstructed rows wherever the two give the same fp32 score.  The capacity
+ * convention is that of ivr_index_range_search: when lims[n] > capacity only lims[n] (the exact total) is meaningful
+ * and D / I are untouched.  Checks, before any device call and in this order: a NaN radius, a negative capacity, a
+ * NULL index or lims, or NULL D / I with capacity > 0 are IVR_EINVAL; capacity above 2^31-1, padded dim above 4096,
+ * an index of 2^32 rows or more and a window of 2^31-1 rows or more are IVR_EUNSUPPORTED.  A window reaching beyond
+ * the rows is IVR_EINVAL, and so many rows that the join needs more than 2^31-1 work units (about 50 M at 512 dims)
+ * IVR_EUNSUPPORTED, when the call runs.  The device variant never blocks the host; its scratch grows the handle's
+ * workspace by about 28 bytes per capacity entry and 36 bytes per row.  The host variant stages through the
+ * handle's pinned buffer. */
+IVR_API int ivr_index_range_self_join(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_host,
+                                      float* D_host, int64_t* I_host);
+IVR_API int ivr_index_range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev,
+                                             float* D_dev, int64_t* I_dev, void* stream);
+
 /* Search window: until cleared (count < 0) every search on this handle scores only the stored rows
  * [first, first + count) -- ids are still "stored row + id_offset", k > count pads as usual, a window reaching beyond
  * ntotal fails the search with IVR_EINVAL.  No data moves: this is how a row shard that also holds a replica of its

@@ -468,6 +468,40 @@ static int range_args(const ivr_index* idx, const void* q, int64_t nq, float rad
     return IVR_OK;
 }
 
+// Checks of ivr_index_range_self_join*(), in an order that needs no device.  The join covers the rows of the search
+// window; their count is the number of CUB segments, an int.
+static int join_args(const ivr_index* idx, float radius, int64_t capacity, const void* lims, const void* D,
+                     const void* I) {
+    if (radius != radius) { set_error("range_self_join: radius is NaN"); return IVR_EINVAL; }
+    if (capacity < 0) {
+        set_error("range_self_join: capacity must be >= 0 (got %lld)", static_cast<long long>(capacity));
+        return IVR_EINVAL;
+    }
+    if (!idx || !lims || (capacity > 0 && (!D || !I))) {
+        set_error("range_self_join: bad argument (NULL index or buffer)");
+        return IVR_EINVAL;
+    }
+    if (capacity > INT_MAX) {
+        set_error("range_self_join: at most 2^31-1 hits per call (capacity %lld)", static_cast<long long>(capacity));
+        return IVR_EUNSUPPORTED;
+    }
+    if (small_range_chunk(idx) < 16) {
+        set_error("range_self_join: dim %d is wider than the small-batch kernel holds (padded dim <= 4096)", idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    if (idx->ntotal >= (1ll << 32)) {
+        set_error("range_self_join: the hit key holds a 32-bit row; the index has %lld rows",
+                  static_cast<long long>(idx->ntotal));
+        return IVR_EUNSUPPORTED;
+    }
+    if ((idx->win_count >= 0 ? idx->win_count : idx->ntotal) >= INT_MAX) {
+        set_error("range_self_join: at most 2^31-2 rows per join (window of %lld rows)",
+                  static_cast<long long>(idx->win_count));
+        return IVR_EUNSUPPORTED;
+    }
+    return IVR_OK;
+}
+
 // Exchange keys hold a 32-bit row: the global ids id_offset + [0, ntotal) must fit.
 static int check_key_ids(const ivr_index* idx, int64_t id_offset, const char* who) {
     if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
@@ -595,6 +629,53 @@ int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, floa
     const int64_t total = lims_host[nq];
     if (total == 0 || total > capacity) return IVR_OK;              // nothing to copy / the caller retries
     // the hits, through the pinned buffer sized to what was found
+    const size_t hd = static_cast<size_t>(total) * sizeof(float), hi = static_cast<size_t>(total) * sizeof(int64_t);
+    Carve hits;
+    const size_t o_hd = hits(hd), o_hi = hits(hi);
+    IVR_TRY(ensure_pin(idx, hits.size));
+    pin = static_cast<char*>(idx->pin);
+    IVR_CUDA(cudaMemcpyAsync(pin + o_hd, dd, hd, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_hi, di, hi, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaStreamSynchronize(st));
+    staged_memcpy(D_host, pin + o_hd, hd);
+    staged_memcpy(I_host, pin + o_hi, hi);
+    return IVR_OK;
+}
+
+int ivr_index_range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev, float* D_dev,
+                                     int64_t* I_dev, void* stream) {
+    IVR_TRY(join_args(idx, radius, capacity, lims_dev, D_dev, I_dev));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);       // NULL = the legacy default stream, as in CUDA
+    return with_search_window(idx, 0, st, "range_self_join", [&](int64_t id_offset) {
+        return range_self_join_device(idx, radius, capacity, lims_dev, D_dev, I_dev, id_offset, st);
+    });
+}
+
+int ivr_index_range_self_join(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_host, float* D_host,
+                              int64_t* I_host) {
+    IVR_TRY(join_args(idx, radius, capacity, lims_host, D_host, I_host));
+    IVR_CUDA(cudaSetDevice(idx->device));
+    cudaStream_t st = idx->stream;
+    // a window reaching past the rows fails in the device call, before anything is copied back
+    const int64_t n = std::min(idx->win_count >= 0 ? idx->win_count : idx->ntotal, idx->ntotal);
+    const size_t lb = static_cast<size_t>(n + 1) * sizeof(int64_t);
+    const size_t db = static_cast<size_t>(capacity) * sizeof(float), ib = static_cast<size_t>(capacity) * sizeof(int64_t);
+    Carve carve;                                                    // the pinned buffer holds the first part
+    const size_t o_l = carve(lb);
+    IVR_TRY(ensure_pin(idx, carve.size));
+    const size_t o_d = carve(db), o_i = carve(ib);
+    IVR_TRY(ensure_io(idx, carve.size));
+    char* pin = static_cast<char*>(idx->pin);
+    char* io = static_cast<char*>(idx->io);
+    int64_t* dl = reinterpret_cast<int64_t*>(io + o_l);
+    float* dd = reinterpret_cast<float*>(io + o_d);
+    int64_t* di = reinterpret_cast<int64_t*>(io + o_i);
+    IVR_TRY(ivr_index_range_self_join_device(idx, radius, capacity, dl, dd, di, st));
+    IVR_CUDA(cudaMemcpyAsync(pin + o_l, dl, lb, cudaMemcpyDeviceToHost, st));
+    IVR_CUDA(cudaStreamSynchronize(st));
+    memcpy(lims_host, pin + o_l, lb);
+    const int64_t total = lims_host[n];
+    if (total == 0 || total > capacity) return IVR_OK;              // nothing to copy / the caller retries
     const size_t hd = static_cast<size_t>(total) * sizeof(float), hi = static_cast<size_t>(total) * sizeof(int64_t);
     Carve hits;
     const size_t o_hd = hits(hd), o_hi = hits(hi);

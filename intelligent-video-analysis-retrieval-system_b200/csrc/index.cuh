@@ -87,6 +87,9 @@ int  range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float r
 // the same search, hits left as exchange keys make_key(score, row + id_offset) in the order of D / I
 int  range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
                               int64_t* lims, uint64_t* keys, int64_t id_offset, cudaStream_t st);
+// lims [ntotal + 1], D, I = every pair of distinct current rows with score > radius, by first row (range_search.cu)
+int  range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
+                            int64_t id_offset, cudaStream_t st);
 // merge of per-part sorted range runs into lims / D / I (ivr_range_merge_keys_device); no scratch, two launches
 int  range_merge_keys_device(const uint64_t* keys_parts, int64_t part_stride, const int64_t* lims_parts, int n_parts,
                              int64_t nq, int64_t* lims, float* D, int64_t* I, cudaStream_t st);

@@ -412,5 +412,9 @@ int  search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, flo
 int  search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
                             float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
                             cudaStream_t st);
+// its self-join epilogue: one launch that appends both (i, j) and (j, i) of every pair i < j of the stored rows with
+// score > radius to the hit pool of range_search.cu
+int  search_mma_small_join(ivr_index* idx, float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx,
+                           int64_t capacity, cudaStream_t st);
 
 }  // namespace ivr

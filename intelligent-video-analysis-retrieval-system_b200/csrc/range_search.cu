@@ -7,7 +7,8 @@
 //      (packed key, query) pairs; the 64-bit cursor counts every hit, also those past the pool's capacity;
 //   3. if the pool held them all: histogram by query, exclusive scan into lims, scatter into the query segments,
 //      segmented sort descending (the key order: score descending, then lower row), unpack to D / I.
-// Step 3 reads the cursor on the device, so nothing here waits for the GPU.  Algorithmic bytes:
+// Step 3 reads the cursor on the device, so nothing here waits for the GPU.  The self-join (range_self_join_device)
+// fills the same pool from the join kernel, with the stored rows as queries, and shares step 3.  Algorithmic bytes:
 // ntotal * dpad * 2 per query chunk, plus 12 bytes per hit in the pool and 12 in the output.
 #include "mma_common.cuh"
 
@@ -80,19 +81,15 @@ __global__ void range_pack_keys_kernel(const uint64_t* __restrict__ sorted,
     }
 }
 
-// The body shared by both range entry points: score, group and sort every hit into lims / the sorted pool, then
-// finish(sorted, cursor, q_scale, grid, threads) queues the last step, which writes the caller's output.
-template <class Finish>
-static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
-                               int64_t* lims, cudaStream_t st, Finish&& finish) {
-    if (idx->ntotal == 0) {
-        IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t), st));
-        return IVR_OK;
-    }
-    const int chunk = small_range_chunk(idx);
-    const int64_t n_chunks = (nq + chunk - 1) / chunk;
+// The hit pool and its grouping, shared by range search and the self-join.  `carve` holds the caller's own workspace
+// parts; the pool's follow.  score(ws, cursor, keys, qidx) queues the launches that fill the pool of `capacity` (key,
+// segment) entries; the segments [0, nq) are then grouped on the device: histogram, scan into lims, scatter, segmented
+// sort descending (score descending, then lower row); finish(ws, sorted, cursor, grid, threads) queues the last step,
+// which writes the caller's output.  lims[nq] ends as the exact total.
+template <class Score, class Finish>
+static int range_pool_sorted(ivr_index* idx, Carve carve, int64_t nq, int64_t capacity, int64_t* lims, cudaStream_t st,
+                             Score&& score, Finish&& finish) {
     const int items = static_cast<int>(capacity);        // the caller checked capacity <= INT_MAX
-
     size_t scan_bytes = 0, sort_bytes = 0;
     IVR_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<const int64_t*>(nullptr),
                                            static_cast<int64_t*>(nullptr), static_cast<int>(nq + 1), st));
@@ -100,10 +97,6 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
                                                           static_cast<uint64_t*>(nullptr), items, static_cast<int>(nq),
                                                           static_cast<const int64_t*>(nullptr),
                                                           static_cast<const int64_t*>(nullptr), st));
-    Carve carve;
-    const size_t o_q   = carve(static_cast<size_t>(chunk) * idx->dpad * 2);
-    const size_t o_sc  = carve(static_cast<size_t>(n_chunks) * chunk * 4);
-    const size_t o_tg  = carve(static_cast<size_t>(chunk) * 4);
     const size_t zero_bytes = (1 + 2 * static_cast<size_t>(nq) + 1) * 8;   // cursor, counts [nq + 1], fill [nq]
     const size_t o_z   = carve(zero_bytes);
     const size_t o_k   = carve(static_cast<size_t>(capacity) * 8);
@@ -113,9 +106,6 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
     const size_t o_tmp = carve(std::max(scan_bytes, sort_bytes));
     IVR_TRY(ensure_ws(idx, carve.size));
     char* ws = static_cast<char*>(idx->ws);
-    __half* q_h = reinterpret_cast<__half*>(ws + o_q);
-    float* q_scale = reinterpret_cast<float*>(ws + o_sc);
-    uint32_t* tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
     unsigned long long* cursor = reinterpret_cast<unsigned long long*>(ws + o_z);
     unsigned long long* counts = cursor + 1;
     unsigned long long* fill = counts + nq + 1;
@@ -126,12 +116,7 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
     void* tmp = ws + o_tmp;
 
     IVR_CUDA(cudaMemsetAsync(cursor, 0, zero_bytes, st));
-    for (int64_t c = 0; c < n_chunks; ++c) {
-        const int64_t q0 = c * chunk, m = std::min<int64_t>(chunk, nq - q0);
-        IVR_TRY(launch_queries_to_f16(q_dev + q0 * idx->dim, q_h, q_scale + q0, tau_g, m, (m + 15) / 16 * 16, idx->dim,
-                                      idx->dpad, st));
-        IVR_TRY(search_mma_small_range(idx, q_h, q_scale + q0, m, q0, radius, cursor, keys, qidx, capacity, st));
-    }
+    IVR_TRY(score(ws, cursor, keys, qidx));
     const int grid = idx->sm_count * 4, threads = 256;
     range_histogram_kernel<<<grid, threads, 0, st>>>(qidx, cursor, capacity, counts);
     IVR_CUDA(cudaGetLastError());
@@ -142,11 +127,44 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
     if (items > 0)
         IVR_CUDA(cub::DeviceSegmentedSort::SortKeysDescending(tmp, sort_bytes, seg, sorted, items, static_cast<int>(nq),
                                                               lims, lims + 1, st));
-    IVR_TRY(finish(static_cast<const uint64_t*>(sorted), static_cast<const unsigned long long*>(cursor),
-                   static_cast<const float*>(q_scale), grid, threads));
+    IVR_TRY(finish(static_cast<const char*>(ws), static_cast<const uint64_t*>(sorted),
+                   static_cast<const unsigned long long*>(cursor), grid, threads));
     // lims[nq] = the true total: equal to the scan's when the pool held every hit, the size to retry with otherwise
     IVR_CUDA(cudaMemcpyAsync(lims + nq, cursor, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
     return IVR_OK;
+}
+
+// The body shared by both range entry points: score every query chunk into the pool, group and sort it into lims /
+// the sorted pool, then finish(sorted, cursor, q_scale, grid, threads) queues the last step, which writes the
+// caller's output.
+template <class Finish>
+static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                               int64_t* lims, cudaStream_t st, Finish&& finish) {
+    if (idx->ntotal == 0) {
+        IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    const int chunk = small_range_chunk(idx);
+    const int64_t n_chunks = (nq + chunk - 1) / chunk;
+    Carve carve;
+    const size_t o_q   = carve(static_cast<size_t>(chunk) * idx->dpad * 2);
+    const size_t o_sc  = carve(static_cast<size_t>(n_chunks) * chunk * 4);
+    const size_t o_tg  = carve(static_cast<size_t>(chunk) * 4);
+    return range_pool_sorted(idx, carve, nq, capacity, lims, st,
+                             [&](char* ws, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx) {
+        __half* q_h = reinterpret_cast<__half*>(ws + o_q);
+        float* q_scale = reinterpret_cast<float*>(ws + o_sc);
+        uint32_t* tau_g = reinterpret_cast<uint32_t*>(ws + o_tg);
+        for (int64_t c = 0; c < n_chunks; ++c) {
+            const int64_t q0 = c * chunk, m = std::min<int64_t>(chunk, nq - q0);
+            IVR_TRY(launch_queries_to_f16(q_dev + q0 * idx->dim, q_h, q_scale + q0, tau_g, m, (m + 15) / 16 * 16,
+                                          idx->dim, idx->dpad, st));
+            IVR_TRY(search_mma_small_range(idx, q_h, q_scale + q0, m, q0, radius, cursor, keys, qidx, capacity, st));
+        }
+        return IVR_OK;
+    }, [&](const char* ws, const uint64_t* sorted, const unsigned long long* cursor, int grid, int threads) {
+        return finish(sorted, cursor, reinterpret_cast<const float*>(ws + o_sc), grid, threads);
+    });
 }
 
 int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
@@ -167,6 +185,36 @@ int range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, flo
                                    int grid, int threads) {
         range_pack_keys_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset,
                                                          keys);
+        IVR_CUDA(cudaGetLastError());
+        return IVR_OK;
+    });
+}
+
+__global__ void range_fill_kernel(float* __restrict__ x, int64_t n, float v) {
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+        x[i] = v;
+}
+
+// lims, D, I = range_self_join(radius): the join kernel (search_mma_small.cu) puts both (i, j) and (j, i) of every
+// pair into the pool, segmented by the first row; the grouping is range search's, and the unpack's scales are ones.
+int range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
+                           int64_t id_offset, cudaStream_t st) {
+    const int64_t n = idx->ntotal;
+    if (n == 0) {
+        IVR_CUDA(cudaMemsetAsync(lims, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    Carve carve;
+    const size_t o_one = carve(static_cast<size_t>(n) * 4);
+    return range_pool_sorted(idx, carve, n, capacity, lims, st,
+                             [&](char*, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx) {
+        return search_mma_small_join(idx, radius, cursor, keys, qidx, capacity, st);
+    }, [&](const char* ws, const uint64_t* sorted, const unsigned long long* cursor, int grid, int threads) {
+        float* ones = reinterpret_cast<float*>(const_cast<char*>(ws) + o_one);
+        range_fill_kernel<<<grid, threads, 0, st>>>(ones, n, 1.0f);
+        IVR_CUDA(cudaGetLastError());
+        range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, n, ones, id_offset, D, I);
         IVR_CUDA(cudaGetLastError());
         return IVR_OK;
     });

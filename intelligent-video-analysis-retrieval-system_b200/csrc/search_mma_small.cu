@@ -27,11 +27,15 @@
 // query would otherwise cost more than the streaming itself).
 // The per-(CTA, warp) survivors are folded by topk_merge.cu.
 // A third epilogue, with a fixed threshold, runs in its own __global__ (search_mma_small_range_kernel) for the exact
-// range search of range_search.cu; it shares the producer and MMA code below.
+// range search of range_search.cu; it shares the producer and MMA code below.  A fourth, search_mma_small_join_kernel,
+// serves the self-join of range_search.cu: stored rows on both operands, the upper triangle of the score matrix.
 //
 // Replaces D, I = index.search(x, k) for small batches (unified_index.py:503, core.py:891).
 // Algorithmic bytes: ntotal * dpad * 2 per search.
 #include "mma_common.cuh"
+
+#include <climits>
+#include <numeric>
 
 namespace ivr {
 
@@ -452,6 +456,145 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
 }
 
+// JOIN mode (range_self_join of range_search.cu): both operands are stored rows.  A unit of work is (column block b,
+// segment s): B = the npad rows [b * npad, (b + 1) * npad) resident in shared memory, A = the row tiles
+// [s * seg_tiles, (s + 1) * seg_tiles) that hold a row below the block's last row.  Units are numbered segment-major,
+// so the CTAs resident together stream the same row tiles and L2 serves all but the first read of each.  seg_tiles *
+// 128 is a multiple of npad: segment s starts at block s * seg_blocks and holds nb - s * seg_blocks units.
+struct SmallJoinParams {
+    int64_t  n;                        // rows of the (windowed) index
+    int      npad, kblocks, stages, nbuf, buf_cols;
+    int      seg_tiles;                // row tiles per segment
+    int64_t  nb, seg_blocks, n_seg;    // column blocks; blocks a segment start moves by; segments
+    uint64_t row_policy;
+    float    radius;
+    unsigned long long* cursor;        // pool entries reserved so far
+    uint64_t* keys;                    // [capacity] make_key(score, column row)
+    uint32_t* qidx;                    // [capacity] the other row of the pair
+    unsigned long long capacity;
+};
+
+// Warp 0, one lane: the npad-row block of B at row b_row once, then row tiles [t0, t1) of A through the ring.
+__device__ __forceinline__ void small_produce_join(const SmallSmem& sm, const CUtensorMap* tmap_b, int b_row,
+                                                   const CUtensorMap* tmap_x, int kblocks, int stages, int64_t t0,
+                                                   int64_t t1, uint64_t policy) {
+    mbar_expect_tx(sm.q_full(), sm.q_bytes);
+    for (int kb = 0; kb < kblocks; ++kb)
+        tma_load_2d<1>(sm.smem_q + kb * sm.q_block, tmap_b, sm.q_full(), kb * kKBlock, b_row, policy);
+    int stage = 0; uint32_t phase = 0;
+    for (int64_t t = t0; t < t1; ++t) {
+        const int row0 = static_cast<int>(t * kSmallTileRows);
+        for (int kb = 0; kb < kblocks; ++kb) {
+            mbar_wait(sm.empty_bar(stage), phase ^ 1);
+            mbar_expect_tx(sm.full_bar(stage), kSmallStageBytes);
+            tma_load_2d<1>(sm.smem_a + stage * kSmallStageBytes, tmap_x, sm.full_bar(stage), kb * kKBlock, row0, policy);
+            if (++stage == stages) { stage = 0; phase ^= 1; }
+        }
+    }
+}
+
+// One CTA per unit (see SmallJoinParams).  The epilogue keeps (i, j) with i < j < n and score > radius and appends
+// two pool entries per pair, (make_key(s, j), i) and (make_key(s, i), j): one 64-bit cursor reservation per warp and
+// 32-column chunk.  Entries at or past `capacity` are dropped but counted.
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_join_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_x,
+                             const SmallJoinParams p) {
+    extern __shared__ __align__(1024) uint8_t smem_raw[];
+    const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+    // unit -> (segment s, block b): segments before s hold P(s) = s * nb - seg_blocks * s * (s - 1) / 2 units
+    const int64_t u = blockIdx.x;
+    int64_t lo = 0, hi = p.n_seg - 1;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi + 1) >> 1;
+        if (mid * p.nb - p.seg_blocks * mid * (mid - 1) / 2 <= u) lo = mid; else hi = mid - 1;
+    }
+    const int64_t s = lo;
+    const int64_t b = s * p.seg_blocks + (u - (s * p.nb - p.seg_blocks * s * (s - 1) / 2));
+    const int64_t jb = b * p.npad;                                     // first column row
+    const int64_t j_end = jb + p.npad < p.n ? jb + p.npad : p.n;
+    const int64_t t_end = (j_end + kSmallTileRows - 1) / kSmallTileRows;   // the tiles up to the block's last row
+    const int64_t t0 = s * p.seg_tiles, t1 = t0 + p.seg_tiles < t_end ? t0 + p.seg_tiles : t_end;
+
+    small_setup(sm, &tmap_b, &tmap_x, p.stages, p.nbuf, warp, lane);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    uint32_t tmem_base;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
+
+    if (warp == 0 && lane == 0) {
+        small_produce_join(sm, &tmap_b, static_cast<int>(jb), &tmap_x, p.kblocks, p.stages, t0, t1, p.row_policy);
+    } else if (warp == 1 && lane == 0) {
+        small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, t0, t1);
+    } else if (warp >= 2) {
+        // ============================ epilogue: upper triangle, fixed threshold ========
+        const int quarter = warp & 3;                              // the TMEM lanes this warp may read
+        int buf = 0; uint32_t bphase = 0;
+        for (int64_t t = t0; t < t1; ++t) {
+            const int64_t i = t * kSmallTileRows + quarter * 32 + lane;
+            mbar_wait(sm.tfull_bar(buf), bphase);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
+                                   static_cast<uint32_t>(buf * p.buf_cols);
+            for (int c0 = 0; c0 < p.npad; c0 += 32) {
+                uint32_t v[32];
+                if (p.npad - c0 >= 32) {
+                    tmem_ld_32x32(taddr + c0, v);
+                } else {                                            // npad is a multiple of 16: a 16-column tail
+#pragma unroll
+                    for (int k = 16; k < 32; ++k) v[k] = 0xff800000u;
+                    tmem_ld_32x16(taddr + c0, v);
+                }
+                tmem_wait_ld(v);
+                if (c0 + 32 >= p.npad) {                            // accumulator fully read: hand it back
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_local(sm.tempty_bar(buf));
+                }
+                unsigned m = 0;
+#pragma unroll
+                for (int k = 0; k < 32; ++k) m |= (__uint_as_float(v[k]) > p.radius ? 1u : 0u) << k;
+                // column k is row j = jc + k: keep i < j < n.  This also drops the zero-filled rows past n, whose
+                // score 0 can exceed a negative radius, and every A row i >= n (then no j > i is below n).
+                const int64_t jc = jb + c0;
+                const int64_t above = i - jc, below = p.n - jc;     // keep k > above and k < below
+                m &= above < 0 ? 0xffffffffu : (above >= 31 ? 0u : 0xffffffffu << (above + 1));
+                m &= below >= 32 ? 0xffffffffu : (below <= 0 ? 0u : (1u << below) - 1u);
+                const int cnt = __popc(m);
+                int incl = cnt;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int x = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += x;
+                }
+                const int total = __shfl_sync(0xffffffffu, incl, 31);
+                if (total == 0) continue;                           // warp-uniform
+                unsigned long long slot = 0;
+                if (lane == 0) slot = atomicAdd(p.cursor, 2ull * static_cast<unsigned long long>(total));
+                slot = __shfl_sync(0xffffffffu, slot, 0) + 2ull * static_cast<unsigned long long>(incl - cnt);
+                const uint32_t row_i = static_cast<uint32_t>(i);
+#pragma unroll
+                for (int k = 0; k < 32; ++k) {
+                    if (!((m >> k) & 1u)) continue;
+                    const float sc = __uint_as_float(v[k]);
+                    const uint32_t row_j = static_cast<uint32_t>(jc + k);
+                    if (slot < p.capacity)     { p.keys[slot] = make_key(sc, row_j);     p.qidx[slot] = row_i; }
+                    if (slot + 1 < p.capacity) { p.keys[slot + 1] = make_key(sc, row_i); p.qidx[slot + 1] = row_j; }
+                    slot += 2;
+                }
+            }
+            if (++buf == p.nbuf) { buf = 0; bphase ^= 1; }
+        }
+    }
+
+    // ------------------------------------------------------------------ teardown ----
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
+}
+
 // ------------------------------------------------------------------ host side ----
 struct SmallShape { int npad, stages, nbuf, buf_cols, C; size_t smem; };
 
@@ -637,6 +780,48 @@ int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sca
     p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
     const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(p.nt, 1)));
     search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
+    IVR_CUDA(cudaGetLastError());
+    return IVR_OK;
+}
+
+// One CTA per unit rather than a persistent grid: a CTA then never reloads B behind MMAs still reading it, and the
+// units, ~40 row tiles of 1.8 us of tensor work each at 512 dims, are long enough that the set-up of a CTA (barriers,
+// TMEM, the 128 KB block of B) costs a few percent.
+int search_mma_small_join(ivr_index* idx, float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx,
+                          int64_t capacity, cudaStream_t st) {
+    const int64_t n = idx->ntotal;
+    const int npad = small_range_chunk(idx);
+    SmallShape sh;
+    if (!pipe_shape(idx, npad, &sh)) {
+        set_error("range_self_join: dim %d does not fit the small-batch kernel", idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    int seg_tiles = npad / std::gcd(npad, kSmallTileRows);          // the least tile count that ends on a block edge
+    seg_tiles *= (40 + seg_tiles - 1) / seg_tiles;                  // ~40 row tiles per unit
+    SmallJoinParams p{};
+    p.n = n; p.npad = sh.npad;
+    p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
+    p.seg_tiles = seg_tiles;
+    p.nb = (n + npad - 1) / npad;
+    p.seg_blocks = static_cast<int64_t>(seg_tiles) * kSmallTileRows / npad;
+    p.n_seg = ((n + kSmallTileRows - 1) / kSmallTileRows + seg_tiles - 1) / seg_tiles;
+    const int64_t units = p.n_seg * p.nb - p.seg_blocks * p.n_seg * (p.n_seg - 1) / 2;
+    if (units > INT_MAX) {
+        set_error("range_self_join: %lld rows need %lld work units, more than one launch holds (2^31-1)",
+                  static_cast<long long>(n), static_cast<long long>(units));
+        return IVR_EUNSUPPORTED;
+    }
+    p.row_policy = kL2EvictNormal;                                   // other CTAs re-read the same row tiles
+    p.radius = radius;
+    p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
+    const CUtensorMap* cached;
+    IVR_TRY(row_tmap(idx, kSmallTileRows, &cached));
+    const CUtensorMap tmx = *cached;                                 // the cache holds one box height at a time
+    IVR_TRY(row_tmap(idx, npad, &cached));
+    const CUtensorMap tmb = *cached;
+    IVR_CUDA(cudaFuncSetAttribute(search_mma_small_join_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(sh.smem)));
+    search_mma_small_join_kernel<<<static_cast<unsigned>(units), kSmallThreads, sh.smem, st>>>(tmb, tmx, p);
     IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }

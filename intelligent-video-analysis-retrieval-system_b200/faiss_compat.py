@@ -52,6 +52,7 @@ class IndexFlatIP:
         nat.check(nat.lib.ivr_index_create(self.d, self.device, C.byref(h)))
         self._h = h
         self.search_path = nat.PATH_AUTO
+        self._window_count = -1
 
     # -- lifecycle -------------------------------------------------------
     def close(self):
@@ -84,6 +85,7 @@ class IndexFlatIP:
         """Searches score only the stored rows [first, first + count) until cleared (``count < 0``); ids stay
         "stored row + id_offset".  No data moves (``ivr_index_set_window``)."""
         nat.check(nat.lib.ivr_index_set_window(self._handle(), int(first), int(count)))
+        self._window_count = int(count)
 
     def reserve(self, n_rows: int):
         nat.check(nat.lib.ivr_index_reserve(self._handle(), int(n_rows)))
@@ -245,6 +247,50 @@ class IndexFlatIP:
                 return lims, total, out
             cap = total
 
+    def range_self_join(self, radius: float):
+        """lims, D, I = every pair of distinct stored rows whose inner product is strictly greater than ``radius``,
+        over the rows of the search window (``set_window``) or all rows; n = their count.  Row i's hits (i = position
+        in the window) are ``D[lims[i]:lims[i+1]]`` (float32, descending, ties -> lower id) and ``I[...]`` (int64
+        stored row ids).  Each pair is scored once, so j is in row i's list iff i is in row j's, with the same score
+        bits.  A row holding a NaN has no hits and is no hit."""
+        radius = _radius(radius, "range_self_join")
+        n = self._join_rows()
+        lims = np.zeros(n + 1, np.int64)
+        cap = _join_capacity(n)
+        while True:                                     # at most twice: the first call reports the exact total
+            D = np.empty(cap, np.float32)
+            I = np.empty(cap, np.int64)
+            nat.check(nat.lib.ivr_index_range_self_join(self._handle(), radius, cap, lims.ctypes.data,
+                                                        D.ctypes.data, I.ctypes.data))
+            total = int(lims[n])
+            if total <= cap:
+                return lims, D[:total].copy(), I[:total].copy()
+            cap = total
+
+    def range_self_join_tensor(self, radius: float):
+        """Device-resident ``range_self_join`` on torch's current stream; returns CUDA tensors (lims, D, I).  Sizing
+        the outputs reads ``lims[n]`` back to the host once (twice when more hits than the first capacity guess turn
+        up), so this call waits for the join to finish."""
+        import torch
+        radius = _radius(radius, "range_self_join")
+        n = self._join_rows()
+        dev = torch.device("cuda", self.device)
+        lims = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        cap = _join_capacity(n)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        while True:
+            D = torch.empty(cap, dtype=torch.float32, device=dev)
+            I = torch.empty(cap, dtype=torch.int64, device=dev)
+            nat.check(nat.lib.ivr_index_range_self_join_device(self._handle(), radius, cap, lims.data_ptr(),
+                                                               D.data_ptr(), I.data_ptr(), st))
+            total = int(lims[n].item())
+            if total <= cap:
+                return lims, D[:total], I[:total]
+            cap = total
+
+    def _join_rows(self) -> int:
+        return self._window_count if self._window_count >= 0 else self.ntotal
+
     # -- instrumentation ---------------------------------------------------
     def set_timing(self, enable: bool = True):
         nat.check(nat.lib.ivr_index_set_timing(self._handle(), int(bool(enable))))
@@ -404,16 +450,23 @@ def read_index(path, flags: int = 0, device: int | None = None) -> IndexFlatIP:
     return index
 
 
-def _radius(radius) -> float:
+def _radius(radius, who: str = "range_search") -> float:
     r = float(radius)
     if r != r:
-        raise ValueError("range_search: radius is NaN")
+        raise ValueError(f"{who}: radius is NaN")
     return r
 
 
 def _range_capacity(nq: int, ntotal: int) -> int:
     """First guess of a range search's hit count: 1024 per query (at least 1 M), never more than nq * ntotal."""
     return min(nq * ntotal, max(nq * 1024, 1 << 20), (1 << 31) - 1)
+
+
+def _join_capacity(n: int) -> int:
+    """First guess of a self-join's pool size: 64 entries per row (at least 1 M), never more than the n(n-1) ordered
+    pairs.  A near-duplicate radius finds a handful of copies per row, so one call usually suffices; a radius that
+    finds more costs one retry with the exact total, not a pool sized for range search's 1024 hits per row."""
+    return min(n * (n - 1), max(64 * n, 1 << 20), (1 << 31) - 1)
 
 
 def _is_cuda_tensor(x) -> bool:
