@@ -245,11 +245,18 @@ banded_cosine_rw_kernel(const float* __restrict__ e, int64_t n, int64_t out_begi
                 float val = acc[0];
                 val += __shfl_xor_sync(0xffffffffu, val, 8);
                 val += __shfl_xor_sync(0xffffffffu, val, 16);
-                // 1 / ||row||: reciprocal square root + one Newton step (within 2 ulp of 1 / sqrt(ss); no slow-path
-                // branches); sklearn divides by the norm and maps a zero norm to 1
-                float inv = rsqrtf(ss);
-                inv = inv * fmaf(-0.5f * ss, inv * inv, 1.5f);
-                if (ss == 0.f) inv = 1.f;
+                // 1 / ||row||: reciprocal square root + one Newton step while ss is a normal fp32 below 2^126 (there
+                // inv * inv neither overflows nor goes subnormal).  Outside that range -- zero, subnormal, overflowed
+                // to inf, NaN -- take sklearn's 1 / sqrt(ss) with a zero norm mapped to 1: an overflowed norm gives
+                // cosine 0, not NaN.  ss is the same on every lane after the xor butterfly: the branch is warp-uniform.
+                // (The dots above use the raw row: a row whose norm itself exceeds FLT_MAX still overflows them.)
+                float inv;
+                if (ss >= 0x1p-126f && ss < 0x1p126f) {
+                    inv = rsqrtf(ss);
+                    inv = inv * fmaf(-0.5f * ss, inv * inv, 1.5f);
+                } else {
+                    inv = (ss == 0.f) ? 1.f : 1.0f / sqrtf(ss);
+                }
                 val *= inv;
 #pragma unroll
                 for (int j = 0; j < DV; ++j) {                              // frame t (normalised) replaces frame t - 8
