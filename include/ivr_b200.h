@@ -155,6 +155,43 @@ IVR_API int ivr_index_range_self_join(ivr_index* idx, float radius, int64_t capa
 IVR_API int ivr_index_range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev,
                                              float* D_dev, int64_t* I_dev, void* stream);
 
+/* ---- filtered search: a device row selection -----------------------------------------------------------------
+ * Replaces SearchParameters(sel=IDSelector...) on faiss.IndexFlatIP.search / range_search (the reference can only
+ * post-filter the global top-k: unified_index.py:185-238).  A selection is built once from a packed host bitmap --
+ * bit i & 31 of words[i >> 5] selects stored row i, for i < n_rows; rows at or past n_rows are not selected -- and
+ * reused by every filtered search on an index of the same device.  On creation the words are uploaded and the
+ * ascending list of 128-row tiles that hold a selected row is built on the device (4 bytes per tile), so a filtered
+ * search streams only those tiles.  n_rows may be 0 (selects nothing); n_rows < 0, a NULL out, or NULL words with
+ * n_rows > 0 are IVR_EINVAL, n_rows above 2^32 IVR_EUNSUPPORTED, all before any device call.  ivr_selection_count
+ * returns the number of selected rows (-1 for NULL); ivr_selection_destroy(NULL) is a no-op. */
+typedef struct ivr_selection ivr_selection;
+IVR_API int     ivr_selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr_selection** out);
+IVR_API int     ivr_selection_destroy(ivr_selection* sel);
+IVR_API int64_t ivr_selection_count(const ivr_selection* sel);
+
+/* ivr_index_search / ivr_index_range_search restricted to the selected rows, with the same outputs and semantics:
+ * top-k returns the k best selected rows (padded with -1 / -FLT_MAX when fewer are selected), range search every
+ * selected row scoring strictly above the radius; ties go to the lower id, a row holding a NaN is never a hit.
+ * Selected ids at or past ntotal are ignored.  Both run on the small-batch tcgen05 kernel's filtered variants
+ * (search_mma_small_sel_kernel / search_mma_small_sel_range_kernel) for every nq: queries go in chunks of at most 128
+ * (fewer where k or the dimension leave less room), and each chunk streams the selected row tiles once.  A selection
+ * with no row below ntotal writes the padding (or lims = 0) and launches no scoring kernel.  Errors, before any device
+ * call: the argument checks of the unfiltered call, a NULL selection, a search window set on the handle
+ * (ivr_index_set_window) and a selection of another device are IVR_EINVAL; an index of 2^32 rows or more, and a dim
+ * / k whose 16-query tile does not fit the kernel, are IVR_EUNSUPPORTED.  ivr_index_last_timing reports the filtered
+ * call; with several query chunks score_ms runs from the first chunk's scoring to the last one's, prep_ms is the first
+ * chunk's and merge_ms the last chunk's. */
+IVR_API int ivr_index_search_selected(ivr_index* idx, const ivr_selection* sel, const float* q_host, int64_t nq, int k,
+                                      float* D_host, int64_t* I_host);
+IVR_API int ivr_index_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
+                                             int k, float* D_dev, int64_t* I_dev, int64_t id_offset, void* stream);
+IVR_API int ivr_index_range_search_selected(ivr_index* idx, const ivr_selection* sel, const float* q_host, int64_t nq,
+                                            float radius, int64_t capacity, int64_t* lims_host, float* D_host,
+                                            int64_t* I_host);
+IVR_API int ivr_index_range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev,
+                                                   int64_t nq, float radius, int64_t capacity, int64_t* lims_dev,
+                                                   float* D_dev, int64_t* I_dev, int64_t id_offset, void* stream);
+
 /* Search window: until cleared (count < 0) every search on this handle scores only the stored rows
  * [first, first + count) -- ids are still "stored row + id_offset", k > count pads as usual, a window reaching beyond
  * ntotal fails the search with IVR_EINVAL.  No data moves: this is how a row shard that also holds a replica of its

@@ -11,7 +11,8 @@ module at the repository root (``import ivr_b200``).
 """
 from . import _native, faiss_compat, frame_filter, sharded           # noqa: F401
 from .facade import RAGBuilder, RAGRetriever                          # noqa: F401
-from .faiss_compat import IndexFlatIP, normalize_L2                   # noqa: F401
+from .faiss_compat import (IDSelectorBatch, IDSelectorBitmap, IDSelectorNot, IDSelectorRange,  # noqa: F401
+                           IndexFlatIP, SearchParameters, normalize_L2)
 from .frame_filter import FrameFilter                                 # noqa: F401
 from .relationships import build_similarity_relationships            # noqa: F401
 from .retriever import FAISSRetriever, KeyframeMetadata, SearchResult  # noqa: F401

@@ -57,6 +57,18 @@ PROTOTYPES = {
     "ivr_index_range_self_join": (C.c_int, [C.c_void_p, C.c_float, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ivr_index_range_self_join_device": (C.c_int, [C.c_void_p, C.c_float, C.c_int64, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_void_p]),
+    "ivr_selection_create": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
+    "ivr_selection_destroy": (C.c_int, [C.c_void_p]),
+    "ivr_selection_count": (C.c_int64, [C.c_void_p]),
+    "ivr_index_search_selected": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
+                                            C.c_void_p]),
+    "ivr_index_search_selected_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
+                                                   C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "ivr_index_range_search_selected": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
+                                                  C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ivr_index_range_search_selected_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
+                                                         C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                                         C.c_void_p]),
     "ivr_index_set_window": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64]),
     "ivr_index_set_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "ivr_index_last_timing": (C.c_int, [C.c_void_p, _c_f32p, _c_intp]),

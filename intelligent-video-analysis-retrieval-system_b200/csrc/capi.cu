@@ -335,6 +335,25 @@ int ivr_index_set_window(ivr_index* idx, int64_t first, int64_t count) {
 }
 
 int64_t ivr_index_ntotal(const ivr_index* idx) { return idx ? idx->ntotal : -1; }
+int ivr_selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr_selection** out) {
+    if (!out) { set_error("selection_create: out is NULL"); return IVR_EINVAL; }
+    *out = nullptr;
+    if (n_rows < 0) {
+        set_error("selection_create: n_rows must be >= 0 (got %lld)", static_cast<long long>(n_rows));
+        return IVR_EINVAL;
+    }
+    if (n_rows > 0 && !words_host) { set_error("selection_create: words is NULL"); return IVR_EINVAL; }
+    if (n_rows > (1ll << 32)) {
+        set_error("selection_create: row ids must stay below 2^32 (got %lld rows)", static_cast<long long>(n_rows));
+        return IVR_EUNSUPPORTED;
+    }
+    IVR_TRY(require_device(device));
+    return selection_create(device, words_host, n_rows, out);
+}
+
+int ivr_selection_destroy(ivr_selection* sel) { return selection_destroy(sel); }
+int64_t ivr_selection_count(const ivr_selection* sel) { return sel ? sel->count : -1; }
+
 int ivr_index_dim(const ivr_index* idx) { return idx ? idx->dim : -1; }
 int ivr_index_device(const ivr_index* idx) { return idx ? idx->device : -1; }
 
@@ -502,6 +521,56 @@ static int join_args(const ivr_index* idx, float radius, int64_t capacity, const
     return IVR_OK;
 }
 
+// Checks shared by the filtered entry points (ivr_index_*_selected*), in an order that needs no device.
+static int selected_args(const ivr_index* idx, const ivr_selection* sel, const char* who) {
+    if (!idx || !sel) { set_error("%s: bad argument (NULL index or selection)", who); return IVR_EINVAL; }
+    if (idx->win_count >= 0) {
+        set_error("%s: the index has a search window; filtered search covers all stored rows (clear the window with "
+                  "ivr_index_set_window(idx, 0, -1), or select only the window's rows)", who);
+        return IVR_EINVAL;
+    }
+    if (sel->device != idx->device) {
+        set_error("%s: the selection lives on device %d, the index on device %d", who, sel->device, idx->device);
+        return IVR_EINVAL;
+    }
+    if (idx->ntotal >= (1ll << 32)) {
+        set_error("%s: filtered search reports 32-bit rows; the index has %lld rows", who,
+                  static_cast<long long>(idx->ntotal));
+        return IVR_EUNSUPPORTED;
+    }
+    return IVR_OK;
+}
+
+// ivr_index_search_selected_device after the pointer checks: the top-k of the selected rows, on the filtered
+// small-batch kernel; no selected row below ntotal (or no row) writes the padding and scores nothing.
+static int search_selected_impl(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq, int k,
+                                float* D_dev, int64_t* I_dev, int64_t id_offset, cudaStream_t st) {
+    if (k <= 0) { set_error("search_selected: k must be positive (got %d)", k); return IVR_EINVAL; }
+    if (k > IVR_MAX_K) { set_error("search_selected: k=%d exceeds IVR_MAX_K=%d", k, IVR_MAX_K); return IVR_EUNSUPPORTED; }
+    IVR_TRY(selected_args(idx, sel, "search_selected"));
+    if (small_sel_chunk(idx, k) == 0) {
+        set_error("search_selected: dim %d with k=%d does not fit one 16-query tile of the small-batch kernel",
+                  idx->dim, k);
+        return IVR_EUNSUPPORTED;
+    }
+    if (nq == 0) return IVR_OK;
+    return with_search_window(idx, id_offset, st, "search_selected", [&](int64_t id_offset) {
+        idx->launches[0] = idx->launches[1] = idx->launches[2] = 0;
+        idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = false;
+        const int64_t n_tiles = selection_tiles(sel, idx->ntotal);
+        if (n_tiles == 0) {
+            const int64_t n = nq * k;
+            fill_empty_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(D_dev, I_dev, n);
+            IVR_CUDA(cudaGetLastError());
+            idx->last_path = 0;
+            return IVR_OK;
+        }
+        idx->last_path = IVR_PATH_MMA;
+        return search_mma_small_selected(idx, sel->tiles, sel->words, n_tiles, q_dev, nq, k, D_dev, I_dev, id_offset,
+                                         st);
+    });
+}
+
 // Exchange keys hold a 32-bit row: the global ids id_offset + [0, ntotal) must fit.
 static int check_key_ids(const ivr_index* idx, int64_t id_offset, const char* who) {
     if (id_offset < 0 || id_offset + idx->ntotal > 0x100000000ll) {
@@ -537,8 +606,15 @@ int ivr_index_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq,
                               static_cast<cudaStream_t>(stream));
 }
 
-int ivr_index_search(ivr_index* idx, const float* q_host, int64_t nq, int k, float* D_host,
-                     int64_t* I_host, int path) {
+}  // extern "C"
+
+namespace ivr {
+
+// The host-pointer top-k searches: queries in and D / I out through the handle's pinned and device staging buffers,
+// device_call(q_dev, D_dev, I_dev, stream) in between.
+template <class DeviceCall>
+static int host_search(ivr_index* idx, const float* q_host, int64_t nq, int k, float* D_host, int64_t* I_host,
+                       DeviceCall&& device_call) {
     if (!idx || nq < 0 || (nq > 0 && (!q_host || !D_host || !I_host))) {
         set_error("search: bad argument");
         return IVR_EINVAL;
@@ -562,13 +638,41 @@ int ivr_index_search(ivr_index* idx, const float* q_host, int64_t nq, int k, flo
     int64_t* di = reinterpret_cast<int64_t*>(io + o_i);
     memcpy(pin + o_q, q_host, qb);
     IVR_CUDA(cudaMemcpyAsync(dq, pin + o_q, qb, cudaMemcpyHostToDevice, st));
-    IVR_TRY(search_device_impl(idx, dq, nq, k, dd, di, 0, path, st));
+    IVR_TRY(device_call(dq, dd, di, st));
     IVR_CUDA(cudaMemcpyAsync(pin + o_d, dd, db, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaMemcpyAsync(pin + o_i, di, ib, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaStreamSynchronize(st));
     memcpy(D_host, pin + o_d, db);
     memcpy(I_host, pin + o_i, ib);
     return IVR_OK;
+}
+
+}  // namespace ivr
+
+extern "C" {
+
+int ivr_index_search(ivr_index* idx, const float* q_host, int64_t nq, int k, float* D_host,
+                     int64_t* I_host, int path) {
+    return host_search(idx, q_host, nq, k, D_host, I_host, [&](const float* dq, float* dd, int64_t* di, cudaStream_t st) {
+        return search_device_impl(idx, dq, nq, k, dd, di, 0, path, st);
+    });
+}
+
+int ivr_index_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq, int k,
+                                     float* D_dev, int64_t* I_dev, int64_t id_offset, void* stream) {
+    if (!idx || nq < 0 || (nq > 0 && (!q_dev || !D_dev || !I_dev))) {
+        set_error("search_selected: bad argument");
+        return IVR_EINVAL;
+    }
+    return search_selected_impl(idx, sel, q_dev, nq, k, D_dev, I_dev, id_offset, static_cast<cudaStream_t>(stream));
+}
+
+int ivr_index_search_selected(ivr_index* idx, const ivr_selection* sel, const float* q_host, int64_t nq, int k,
+                              float* D_host, int64_t* I_host) {
+    IVR_TRY(selected_args(idx, sel, "search_selected"));
+    return host_search(idx, q_host, nq, k, D_host, I_host, [&](const float* dq, float* dd, int64_t* di, cudaStream_t st) {
+        return search_selected_impl(idx, sel, dq, nq, k, dd, di, 0, st);
+    });
 }
 
 int ivr_index_range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
@@ -600,9 +704,15 @@ int ivr_index_range_search_keys_device(ivr_index* idx, const float* q_dev, int64
     });
 }
 
-int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, float radius, int64_t capacity,
-                           int64_t* lims_host, float* D_host, int64_t* I_host) {
-    IVR_TRY(range_args(idx, q_host, nq, radius, capacity, lims_host, D_host, I_host));
+}  // extern "C"
+
+namespace ivr {
+
+// The host-pointer range searches, after their argument checks: queries in, lims and the hits out through the
+// handle's pinned and device staging buffers, device_call(q_dev, lims_dev, D_dev, I_dev, stream) in between.
+template <class DeviceCall>
+static int host_range(ivr_index* idx, const float* q_host, int64_t nq, int64_t capacity, int64_t* lims_host,
+                      float* D_host, int64_t* I_host, DeviceCall&& device_call) {
     if (nq == 0) { lims_host[0] = 0; return IVR_OK; }
     IVR_CUDA(cudaSetDevice(idx->device));
     cudaStream_t st = idx->stream;
@@ -622,7 +732,7 @@ int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, floa
     int64_t* di = reinterpret_cast<int64_t*>(io + o_i);
     memcpy(pin + o_q, q_host, qb);
     IVR_CUDA(cudaMemcpyAsync(dq, pin + o_q, qb, cudaMemcpyHostToDevice, st));
-    IVR_TRY(ivr_index_range_search_device(idx, dq, nq, radius, capacity, dl, dd, di, 0, st));
+    IVR_TRY(device_call(dq, dl, dd, di, st));
     IVR_CUDA(cudaMemcpyAsync(pin + o_l, dl, lb, cudaMemcpyDeviceToHost, st));
     IVR_CUDA(cudaStreamSynchronize(st));
     memcpy(lims_host, pin + o_l, lb);
@@ -640,6 +750,47 @@ int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, floa
     staged_memcpy(D_host, pin + o_hd, hd);
     staged_memcpy(I_host, pin + o_hi, hi);
     return IVR_OK;
+}
+
+}  // namespace ivr
+
+extern "C" {
+
+int ivr_index_range_search(ivr_index* idx, const float* q_host, int64_t nq, float radius, int64_t capacity,
+                           int64_t* lims_host, float* D_host, int64_t* I_host) {
+    IVR_TRY(range_args(idx, q_host, nq, radius, capacity, lims_host, D_host, I_host));
+    return host_range(idx, q_host, nq, capacity, lims_host, D_host, I_host,
+                      [&](const float* dq, int64_t* dl, float* dd, int64_t* di, cudaStream_t st) {
+        return ivr_index_range_search_device(idx, dq, nq, radius, capacity, dl, dd, di, 0, st);
+    });
+}
+
+int ivr_index_range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
+                                           float radius, int64_t capacity, int64_t* lims_dev, float* D_dev,
+                                           int64_t* I_dev, int64_t id_offset, void* stream) {
+    IVR_TRY(range_args(idx, q_dev, nq, radius, capacity, lims_dev, D_dev, I_dev));
+    IVR_TRY(selected_args(idx, sel, "range_search_selected"));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (nq == 0) {
+        IVR_CUDA(cudaSetDevice(idx->device));
+        IVR_CUDA(cudaMemsetAsync(lims_dev, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return with_search_window(idx, id_offset, st, "range_search_selected", [&](int64_t id_offset) {
+        return range_search_selected_device(idx, sel, q_dev, nq, radius, capacity, lims_dev, D_dev, I_dev, id_offset,
+                                            st);
+    });
+}
+
+int ivr_index_range_search_selected(ivr_index* idx, const ivr_selection* sel, const float* q_host, int64_t nq,
+                                    float radius, int64_t capacity, int64_t* lims_host, float* D_host,
+                                    int64_t* I_host) {
+    IVR_TRY(range_args(idx, q_host, nq, radius, capacity, lims_host, D_host, I_host));
+    IVR_TRY(selected_args(idx, sel, "range_search_selected"));
+    return host_range(idx, q_host, nq, capacity, lims_host, D_host, I_host,
+                      [&](const float* dq, int64_t* dl, float* dd, int64_t* di, cudaStream_t st) {
+        return ivr_index_range_search_selected_device(idx, sel, dq, nq, radius, capacity, dl, dd, di, 0, st);
+    });
 }
 
 int ivr_index_range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev, float* D_dev,

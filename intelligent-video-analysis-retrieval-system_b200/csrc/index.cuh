@@ -3,6 +3,8 @@
 
 #include "common.cuh"
 
+#include <vector>
+
 namespace ivr {
 // Event slots of the search timing (ivr_index_last_timing): interval i runs from ev[2i] to ev[2i + 1], so
 // score_ms = scoring launches, merge_ms = the final merge, prep_ms = query preparation.
@@ -55,6 +57,16 @@ struct ivr_index {
     const char* last_kernel = "";
 };
 
+// A device row selection (ivr_selection_create, selection.cu): bit i & 31 of word i >> 5 selects stored row i.
+struct ivr_selection {
+    int       device = 0;
+    int64_t   n_rows = 0;              // rows the bitmap covers; rows at or past n_rows are not selected
+    int64_t   count  = 0;              // selected rows
+    uint32_t* words  = nullptr;        // [4 * ceil(n_rows / 128)] device bitmap, zero from row n_rows on
+    uint32_t* tiles  = nullptr;        // device, ascending: the 128-row tiles that hold a selected row
+    std::vector<uint32_t> tiles_host;  // the same list, to cut it at an index's tile count
+};
+
 namespace ivr {
 
 int  ensure_ws(ivr_index* idx, size_t bytes);
@@ -90,6 +102,21 @@ int  range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, fl
 // lims [ntotal + 1], D, I = every pair of distinct current rows with score > radius, by first row (range_search.cu)
 int  range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
                             int64_t id_offset, cudaStream_t st);
+// row selections (selection.cu): build the device bitmap and tile list of a new handle; the number of tiles of the
+// list that lie below an index of ntotal rows
+int  selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr_selection** out);
+int  selection_destroy(ivr_selection* sel);
+int64_t selection_tiles(const ivr_selection* sel, int64_t ntotal);
+// filtered top-k on the small-batch kernel (search_mma_small.cu): the n_tiles row tiles tiles[0 .. n_tiles) of a
+// selection, queries in chunks of small_sel_chunk(); small_sel_chunk() == 0: the dimension or k does not fit
+int  small_sel_chunk(const ivr_index* idx, int k);
+int  search_mma_small_selected(ivr_index* idx, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles,
+                               const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev, int64_t id_offset,
+                               cudaStream_t st);
+// range_search_device over the selected rows only (range_search.cu)
+int  range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
+                                  float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
+                                  int64_t id_offset, cudaStream_t st);
 // merge of per-part sorted range runs into lims / D / I (ivr_range_merge_keys_device); no scratch, two launches
 int  range_merge_keys_device(const uint64_t* keys_parts, int64_t part_stride, const int64_t* lims_parts, int n_parts,
                              int64_t nq, int64_t* lims, float* D, int64_t* I, cudaStream_t st);

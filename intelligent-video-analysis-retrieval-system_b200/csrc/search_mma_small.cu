@@ -29,6 +29,10 @@
 // A third epilogue, with a fixed threshold, runs in its own __global__ (search_mma_small_range_kernel) for the exact
 // range search of range_search.cu; it shares the producer and MMA code below.  A fourth, search_mma_small_join_kernel,
 // serves the self-join of range_search.cu: stored rows on both operands, the upper triangle of the score matrix.
+// Filtered search (ivr_selection, selection.cu) runs the top-k and range epilogues in their own __global__ functions,
+// search_mma_small_sel_kernel and search_mma_small_sel_range_kernel: the producer streams the row tiles of the
+// selection's tile list, and each epilogue warp ANDs its 32 rows' bitmap word into the row-validity test.  The kernel
+// bodies are templates on the row-tile source (AllRows / SelRows), so the unfiltered kernels compile as before.
 //
 // Replaces D, I = index.search(x, k) for small batches (unified_index.py:503, core.py:891).
 // Algorithmic bytes: ntotal * dpad * 2 per search.
@@ -118,16 +122,37 @@ __device__ __forceinline__ void small_setup(const SmallSmem& sm, const CUtensorM
     if (warp == 1) tmem_alloc<1>(sm.tmem_slot(), 512);
 }
 
-// Warp 0, one lane: the query tile once, then row tiles [j0, j1) through the ring.
+// Which row tiles a launch streams and which of their rows it may report.  The unfiltered kernels stream the
+// consecutive tiles tile0 + j and report every row; the filtered ones (search_mma_small_sel*_kernel) stream tile
+// tiles[j] of a selection's tile list and report the rows whose bit is set in its bitmap: bit lane of word
+// tile * 4 + quarter is row tile * 128 + quarter * 32 + lane, the 32 rows one epilogue warp drains.
+struct AllRows {
+    int64_t tile0;
+    __device__ __forceinline__ int64_t tile(int64_t j) const { return tile0 + j; }
+    __device__ __forceinline__ bool selected(int64_t, int, int) const { return true; }
+    __device__ __forceinline__ bool dump(const SmallParams& p) const { return p.dump != nullptr; }
+};
+struct SelRows {
+    const uint32_t* tiles;             // ascending tile ids; position j of the launch is tiles[j]
+    const uint32_t* words;             // the row bitmap, zero-padded to whole tiles
+    __device__ __forceinline__ int64_t tile(int64_t j) const { return __ldg(tiles + j); }
+    __device__ __forceinline__ bool selected(int64_t t, int quarter, int lane) const {
+        return (__ldg(words + t * 4 + quarter) >> lane) & 1u;
+    }
+    __device__ __forceinline__ bool dump(const SmallParams&) const { return false; }
+};
+
+// Warp 0, one lane: the query tile once, then row tiles rows.tile(j), j in [j0, j1), through the ring.
+template <class Rows>
 __device__ __forceinline__ void small_produce(const SmallSmem& sm, const CUtensorMap* tmap_q, const CUtensorMap* tmap_x,
-                                              int kblocks, int stages, int64_t tile0, int64_t j0, int64_t j1,
+                                              int kblocks, int stages, const Rows& rows, int64_t j0, int64_t j1,
                                               uint64_t row_policy) {
     mbar_expect_tx(sm.q_full(), sm.q_bytes);
     for (int kb = 0; kb < kblocks; ++kb)
         tma_load_2d<1>(sm.smem_q + kb * sm.q_block, tmap_q, sm.q_full(), kb * kKBlock, 0, kL2EvictLast);
     int stage = 0; uint32_t phase = 0;
     for (int64_t j = j0; j < j1; ++j) {
-        const int row0 = static_cast<int>((tile0 + j) * kSmallTileRows);
+        const int row0 = static_cast<int>(rows.tile(j) * kSmallTileRows);
         for (int kb = 0; kb < kblocks; ++kb) {
             mbar_wait(sm.empty_bar(stage), phase ^ 1);
             mbar_expect_tx(sm.full_bar(stage), kSmallStageBytes);
@@ -165,9 +190,11 @@ __device__ __forceinline__ void small_mma(const SmallSmem& sm, uint32_t tmem_bas
     }
 }
 
-__global__ void __launch_bounds__(kSmallThreads, 1)
-search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
-                        const SmallParams p) {
+// The body of the top-k kernels: the candidate-list epilogue over row tiles rows.tile(j), j in [j0, j1) -- and, for the
+// unfiltered kernel, dump mode (SmallParams::dump).
+template <class Rows>
+__device__ __forceinline__ void small_topk(const CUtensorMap& tmap_q, const CUtensorMap& tmap_x, const SmallParams& p,
+                                           const Rows& rows) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -187,7 +214,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
 
     if (warp == 0 && lane == 0) {
-        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, p.tile0, j0, j1, p.row_policy);
+        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, rows, j0, j1, p.row_policy);
     } else if (warp == 1 && lane == 0) {
         small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, j0, j1);
     } else if (warp >= 2) {
@@ -215,7 +242,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
         };
 
         int buf = 0; uint32_t bphase = 0; int64_t n = 0;
-        if (p.dump) {
+        if (rows.dump(p)) {
             // ---------------- dump mode: scores + per-tile maxima, no lists ----------------
             for (int64_t j = j0; j < j1; ++j) {
                 const int64_t tile = p.tile0 + j;
@@ -269,8 +296,9 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
                     if (t > tau_s[q]) tau_s[q] = t;
                 }
             __syncwarp();
-            const uint32_t row = static_cast<uint32_t>((p.tile0 + j) * kSmallTileRows + quarter * 32 + lane);
-            const bool valid = static_cast<int64_t>(row) < p.n_rows;
+            const int64_t tile = rows.tile(j);
+            const uint32_t row = static_cast<uint32_t>(tile * kSmallTileRows + quarter * 32 + lane);
+            const bool valid = static_cast<int64_t>(row) < p.n_rows && rows.selected(tile, quarter, lane);
             mbar_wait(sm.tfull_bar(buf), bphase);
             tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
@@ -321,7 +349,7 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
             if (++buf == p.nbuf) { buf = 0; bphase ^= 1; }
         }
         __syncwarp();
-        if (!p.dump)
+        if (!rows.dump(p))
             for (int q = lane; q < p.npad; q += 32) p.counts[wslot * p.npad + q] = cnt_w[q];
     }
 
@@ -329,6 +357,20 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     tc_fence_before();
     __syncthreads();
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
+}
+
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
+                        const SmallParams p) {
+    small_topk(tmap_q, tmap_x, p, AllRows{p.tile0});
+}
+
+// Filtered top-k: the list epilogue over the row tiles of a selection (SelRows).  p.tile0 and p.nt count positions in
+// the selection's tile list, so the seeded launches split the list as the unfiltered ones split the rows.  No dump mode.
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_sel_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
+                            const SmallParams p, const uint32_t* __restrict__ tiles, const uint32_t* __restrict__ words) {
+    small_topk(tmap_q, tmap_x, p, SelRows{tiles + p.tile0, words});
 }
 
 // The largest fp32 t with fp32(t * scale) <= radius, so that "score > t" is exactly "the reported score, fp32(score *
@@ -363,9 +405,10 @@ struct SmallRangeParams {
     unsigned long long capacity;
 };
 
-__global__ void __launch_bounds__(kSmallThreads, 1)
-search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
-                              const SmallRangeParams p) {
+// The body of the range kernels: the fixed-threshold epilogue over row tiles rows.tile(j), j in [j0, j1).
+template <class Rows>
+__device__ __forceinline__ void small_range(const CUtensorMap& tmap_q, const CUtensorMap& tmap_x, const SmallRangeParams& p,
+                                            const Rows& rows) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -382,7 +425,7 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
 
     if (warp == 0 && lane == 0) {
-        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, 0, j0, j1, p.row_policy);
+        small_produce(sm, &tmap_q, &tmap_x, p.kblocks, p.stages, rows, j0, j1, p.row_policy);
     } else if (warp == 1 && lane == 0) {
         small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, j0, j1);
     } else if (warp >= 2) {
@@ -390,8 +433,9 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
         const int quarter = warp & 3;                              // the TMEM lanes this warp may read
         int buf = 0; uint32_t bphase = 0;
         for (int64_t j = j0; j < j1; ++j) {
-            const int64_t row64 = j * kSmallTileRows + quarter * 32 + lane;
-            const bool valid = row64 < p.n_rows;
+            const int64_t tile = rows.tile(j);
+            const int64_t row64 = tile * kSmallTileRows + quarter * 32 + lane;
+            const bool valid = row64 < p.n_rows && rows.selected(tile, quarter, lane);
             const uint32_t row = static_cast<uint32_t>(row64);
             mbar_wait(sm.tfull_bar(buf), bphase);
             tc_fence_after();
@@ -454,6 +498,21 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
     tc_fence_before();
     __syncthreads();
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
+}
+
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
+                              const SmallRangeParams p) {
+    small_range(tmap_q, tmap_x, p, AllRows{0});
+}
+
+// Filtered range search: the fixed-threshold epilogue over the row tiles of a selection (SelRows); p.nt counts
+// positions in the selection's tile list.
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_sel_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
+                                  const SmallRangeParams p, const uint32_t* __restrict__ tiles,
+                                  const uint32_t* __restrict__ words) {
+    small_range(tmap_q, tmap_x, p, SelRows{tiles, words});
 }
 
 // JOIN mode (range_self_join of range_search.cu): both operands are stored rows.  A unit of work is (column block b,
@@ -682,22 +741,14 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
     return IVR_OK;
 }
 
-int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,
-                     int64_t id_offset, cudaStream_t st) {
-    SmallShape sh;
-    if (!small_shape(idx, nq, k, &sh)) { set_error("search_mma_small: unsupported shape (nq=%lld, k=%d, dim=%d)",
-                                                   static_cast<long long>(nq), k, idx->dim); return IVR_EUNSUPPORTED; }
-    const int64_t nt = (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
+// The seeded candidate-list launches over nt row tiles (for the filtered kernel: positions in a selection's tile list),
+// merged into D / I.  launch(grid, tmq, tmx, p) queues one scoring launch of `kernel`.  time_first marks the query
+// preparation and the start of the scoring, time_last the end of the scoring and the final merge.
+template <class Launch>
+static int small_list_search(ivr_index* idx, const SmallShape& sh, const float* q_dev, int64_t nq, int k, float* D_dev,
+                             int64_t* I_dev, int64_t id_offset, cudaStream_t st, int64_t nt, const void* kernel,
+                             bool time_first, bool time_last, Launch&& launch) {
     const int sms = idx->sm_count;
-    // Small shards: one launch that materialises the scores (see SmallParams::dump).  The seeded candidate-list path
-    // pays ~0.2 ms of fixed cost (2-3 launches, their merges, cold lists); writing the scores costs nq * 4 bytes per
-    // row.  Measured (dump vs lists, ms): 1 M x 512: 16 q 0.26 vs 0.37, 32 q 0.30 vs 0.37, 64 q 0.44 vs 0.41;
-    // 851 k x 768: 16 q 0.30 vs 0.41, 64 q 0.37 vs 0.43; 3 M x 512: 16 q 0.64 vs 0.68, 32 q 0.72 vs 0.68; 4 M: equal;
-    // 6 M: lists win.  Rule: up to 3.5 M rows while the scores add at most 1/6 to the row bytes.
-    // IVR_SMALL_DUMP_MAX_KROWS (0 = never) overrides the row limit: tests use it to reach both modes.
-    const int64_t dump_rows = static_cast<int64_t>(env_int("IVR_SMALL_DUMP_MAX_KROWS", 3500)) * 1000;
-    if (k <= kSelectMaxK && idx->ntotal <= dump_rows && sh.npad * 4 * 6 <= idx->dpad * 2)
-        return search_mma_small_dump(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st);
     // launch boundaries (in row tiles): one tile per CTA, then as many rows as keep the expected admissions per
     // list around 64 (k * rows_now / rows_before spread over 4 * sms lists), then the rest
     int64_t bounds[4] = {0, 0, 0, 0};
@@ -717,17 +768,16 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
     Carve own;
     const size_t o_l = own(static_cast<size_t>(max_lists) * sh.npad * sh.C * 8);
     const size_t o_c = own(static_cast<size_t>(max_lists) * sh.npad * 4);
-    LaunchSeq seq{idx, st, idx->timing, nq, k, n_phases, D_dev, I_dev, id_offset};
+    LaunchSeq seq{idx, st, time_last, nq, k, n_phases, D_dev, I_dev, id_offset};
     IVR_TRY(begin_launches(&seq, sh.npad, max_lists, own.size));
 
     CUtensorMap tmq;
     const CUtensorMap* tmx;
-    IVR_TRY(prepare_queries(idx, seq.timed, q_dev, nq, sh.npad, seq.q_h, seq.q_scale, seq.tau_g, sh.npad, &tmq, st));
+    IVR_TRY(prepare_queries(idx, time_first, q_dev, nq, sh.npad, seq.q_h, seq.q_scale, seq.tau_g, sh.npad, &tmq, st));
     IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
-    IVR_CUDA(cudaFuncSetAttribute(search_mma_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(sh.smem)));
+    IVR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sh.smem)));
 
-    timing_mark(idx, seq.timed, kScoreBegin, st);
+    timing_mark(idx, time_first, kScoreBegin, st);
     for (int ph = 0; ph < n_phases; ++ph) {
         SmallParams p{};
         p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad; p.k = k; p.C = sh.C;
@@ -738,7 +788,7 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
         p.counts = reinterpret_cast<int*>(seq.own + o_c);
         p.tau_g = seq.tau_g;
         const int grid = static_cast<int>(std::min<int64_t>(sms, std::max<int64_t>(p.nt, 1)));
-        search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
+        launch(grid, tmq, *tmx, p);
         IVR_CUDA(cudaGetLastError());
         idx->launches[0]++;
         MergeIn in{};
@@ -748,8 +798,61 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
         in.n_lists = 4 * grid; in.fixed_count = 0; in.raw = 1;
         IVR_TRY(fold_launch(seq, ph, in));
     }
-    IVR_TRY(finish_launches(seq));
+    return finish_launches(seq);
+}
+
+int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,
+                     int64_t id_offset, cudaStream_t st) {
+    SmallShape sh;
+    if (!small_shape(idx, nq, k, &sh)) { set_error("search_mma_small: unsupported shape (nq=%lld, k=%d, dim=%d)",
+                                                   static_cast<long long>(nq), k, idx->dim); return IVR_EUNSUPPORTED; }
+    const int64_t nt = (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
+    // Small shards: one launch that materialises the scores (see SmallParams::dump).  The seeded candidate-list path
+    // pays ~0.2 ms of fixed cost (2-3 launches, their merges, cold lists); writing the scores costs nq * 4 bytes per
+    // row.  Measured (dump vs lists, ms): 1 M x 512: 16 q 0.26 vs 0.37, 32 q 0.30 vs 0.37, 64 q 0.44 vs 0.41;
+    // 851 k x 768: 16 q 0.30 vs 0.41, 64 q 0.37 vs 0.43; 3 M x 512: 16 q 0.64 vs 0.68, 32 q 0.72 vs 0.68; 4 M: equal;
+    // 6 M: lists win.  Rule: up to 3.5 M rows while the scores add at most 1/6 to the row bytes.
+    // IVR_SMALL_DUMP_MAX_KROWS (0 = never) overrides the row limit: tests use it to reach both modes.
+    const int64_t dump_rows = static_cast<int64_t>(env_int("IVR_SMALL_DUMP_MAX_KROWS", 3500)) * 1000;
+    if (k <= kSelectMaxK && idx->ntotal <= dump_rows && sh.npad * 4 * 6 <= idx->dpad * 2)
+        return search_mma_small_dump(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+    IVR_TRY(small_list_search(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st, nt,
+                              reinterpret_cast<const void*>(search_mma_small_kernel), idx->timing, idx->timing,
+                              [&](int grid, const CUtensorMap& tmq, const CUtensorMap& tmx, const SmallParams& p) {
+        search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
+    }));
     idx->last_kernel = "search_mma_small_kernel";
+    return IVR_OK;
+}
+
+int small_sel_chunk(const ivr_index* idx, int k) {
+    SmallShape sh;
+    for (int c = kSmallMaxQ; c >= 16; c -= 16)
+        if (small_shape(idx, c, k, &sh)) return c;
+    return 0;
+}
+
+int search_mma_small_selected(ivr_index* idx, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles,
+                              const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev, int64_t id_offset,
+                              cudaStream_t st) {
+    const int chunk = small_sel_chunk(idx, k);
+    if (chunk == 0) {
+        set_error("search_selected: dim %d with k=%d does not fit the small-batch kernel", idx->dim, k);
+        return IVR_EUNSUPPORTED;
+    }
+    const int64_t n_chunks = (nq + chunk - 1) / chunk;
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        const int64_t q0 = c * chunk, m = std::min<int64_t>(chunk, nq - q0);
+        SmallShape sh;
+        small_shape(idx, m, k, &sh);                                 // fits: m <= chunk
+        IVR_TRY(small_list_search(idx, sh, q_dev + q0 * idx->dim, m, k, D_dev + q0 * k, I_dev + q0 * k, id_offset, st,
+                                  n_tiles, reinterpret_cast<const void*>(search_mma_small_sel_kernel),
+                                  idx->timing && c == 0, idx->timing && c == n_chunks - 1,
+                                  [&](int grid, const CUtensorMap& tmq, const CUtensorMap& tmx, const SmallParams& p) {
+            search_mma_small_sel_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p, tiles, words);
+        }));
+    }
+    idx->last_kernel = "search_mma_small_sel_kernel";
     return IVR_OK;
 }
 
@@ -759,7 +862,7 @@ int small_range_chunk(const ivr_index* idx) {
 
 int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
                            float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
-                           cudaStream_t st) {
+                           cudaStream_t st, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles) {
     SmallShape sh;
     if (nq > small_range_chunk(idx) || !pipe_shape(idx, nq, &sh)) {
         set_error("range_search: %lld queries of dim %d do not fit one query tile", static_cast<long long>(nq), idx->dim);
@@ -769,17 +872,19 @@ int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sca
     const CUtensorMap* tmx;
     IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
     IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
-    IVR_CUDA(cudaFuncSetAttribute(search_mma_small_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(sh.smem)));
+    const void* kernel = tiles ? reinterpret_cast<const void*>(search_mma_small_sel_range_kernel)
+                               : reinterpret_cast<const void*>(search_mma_small_range_kernel);
+    IVR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sh.smem)));
     SmallRangeParams p{};
     p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad;
     p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
-    p.nt = (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
+    p.nt = tiles ? n_tiles : (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
     p.row_policy = kL2EvictFirst;                                    // each launch reads every row once
     p.radius = radius; p.q_scale = q_scale; p.q_base = static_cast<uint32_t>(q_base);
     p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
     const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(p.nt, 1)));
-    search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
+    if (tiles) search_mma_small_sel_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p, tiles, words);
+    else search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
     IVR_CUDA(cudaGetLastError());
     return IVR_OK;
 }

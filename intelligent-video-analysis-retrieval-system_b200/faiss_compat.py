@@ -20,7 +20,9 @@ from . import _native as nat
 
 __all__ = ["Index", "IndexFlatIP", "IndexFlatL2", "IndexIVFFlat", "normalize_L2",
            "StandardGpuResources", "index_cpu_to_gpu", "index_gpu_to_cpu", "write_index",
-           "read_index", "serialize_index", "deserialize_index", "IO_FLAG_MMAP", "METRIC_INNER_PRODUCT"]
+           "read_index", "serialize_index", "deserialize_index", "IO_FLAG_MMAP", "METRIC_INNER_PRODUCT",
+           "SearchParameters", "IDSelector", "IDSelectorRange", "IDSelectorBatch", "IDSelectorBitmap",
+           "IDSelectorNot"]
 
 IO_FLAG_MMAP = 1
 METRIC_INNER_PRODUCT = 0
@@ -33,6 +35,111 @@ def _as_f32_2d(x, d=None, what="x"):
     if d is not None and a.shape[1] != d:
         raise ValueError(f"{what} has dimension {a.shape[1]}, index has {d}")   # FAISS asserts d == self.d
     return a
+
+
+# -- filtered search: FAISS's SearchParameters(sel=IDSelector...) ------------------------------------------------
+class IDSelector:
+    """Base of the id selectors.  ``words(ntotal)`` is the selection over ids [0, ntotal) as packed uint32 words (bit
+    ``i & 31`` of word ``i >> 5`` = id i), the layout of ``ivr_selection_create``.  The device selection built from it
+    is cached per (device, ntotal) and freed by ``close`` (or when the selector is collected)."""
+
+    def words(self, ntotal: int) -> np.ndarray:
+        return _pack_words(self._mask(int(ntotal)))
+
+    def _mask(self, ntotal: int) -> np.ndarray:       # bool [ntotal]
+        raise NotImplementedError
+
+    def _selection(self, device: int, ntotal: int):
+        cache = self.__dict__.setdefault("_sel_cache", {})
+        key = (int(device), int(ntotal))
+        h = cache.get(key)
+        if h is None:
+            w = self.words(ntotal)
+            h = C.c_void_p()
+            nat.check(nat.lib.ivr_selection_create(int(device), w.ctypes.data, int(ntotal), C.byref(h)))
+            cache[key] = h
+        return h
+
+    def count(self, ntotal: int, device: int | None = None) -> int:
+        """Selected ids below ``ntotal`` (computed by the device selection when ``device`` is given)."""
+        if device is None:
+            return int(self._mask(int(ntotal)).sum())
+        return int(nat.lib.ivr_selection_count(self._selection(device, ntotal)))
+
+    def close(self):
+        cache = self.__dict__.pop("_sel_cache", {})
+        for h in cache.values():
+            nat.lib.ivr_selection_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _pack_words(mask: np.ndarray) -> np.ndarray:
+    """bool [n] -> uint32 [ceil(n / 32)], bit i & 31 of word i >> 5 = mask[i]."""
+    b = np.packbits(np.asarray(mask, bool), bitorder="little")
+    b = np.concatenate([b, np.zeros(-b.size % 4, np.uint8)])
+    return b.view("<u4").astype(np.uint32)
+
+
+class IDSelectorRange(IDSelector):
+    """``faiss.IDSelectorRange(imin, imax)``: ids in the half-open range [imin, imax)."""
+
+    def __init__(self, imin: int, imax: int):
+        self.imin, self.imax = int(imin), int(imax)
+
+    def _mask(self, ntotal):
+        m = np.zeros(ntotal, bool)
+        m[max(self.imin, 0):max(min(self.imax, ntotal), 0)] = True
+        return m
+
+
+class IDSelectorBatch(IDSelector):
+    """``faiss.IDSelectorBatch(ids)``: the ids listed (duplicates and ids outside [0, ntotal) are ignored)."""
+
+    def __init__(self, ids):
+        self.ids = np.asarray(ids, np.int64).reshape(-1)
+
+    def _mask(self, ntotal):
+        m = np.zeros(ntotal, bool)
+        ids = self.ids[(self.ids >= 0) & (self.ids < ntotal)]
+        m[ids] = True
+        return m
+
+
+class IDSelectorBitmap(IDSelector):
+    """``faiss.IDSelectorBitmap(bitmap)``: ``bitmap`` is a 1-D uint8 array in FAISS's bit order, id i is selected
+    iff ``(bitmap[i >> 3] >> (i & 7)) & 1``; ids past the bitmap are not selected."""
+
+    def __init__(self, bitmap):
+        b = np.asarray(bitmap)
+        if b.dtype != np.uint8 or b.ndim != 1:
+            raise TypeError("IDSelectorBitmap expects a 1-D uint8 array")
+        self.bitmap = b.copy()
+
+    def _mask(self, ntotal):
+        bits = np.unpackbits(self.bitmap, bitorder="little")[:ntotal].astype(bool)
+        return np.concatenate([bits, np.zeros(ntotal - bits.size, bool)])
+
+
+class IDSelectorNot(IDSelector):
+    """``faiss.IDSelectorNot(sel)``: the ids in [0, ntotal) that ``sel`` does not select."""
+
+    def __init__(self, sel: IDSelector):
+        self.sel = sel
+
+    def _mask(self, ntotal):
+        return ~self.sel._mask(ntotal)
+
+
+class SearchParameters:
+    """``faiss.SearchParameters(sel=...)``: ``sel`` restricts a search to the ids it selects (None = all ids)."""
+
+    def __init__(self, sel: IDSelector | None = None):
+        self.sel = sel
 
 
 class IndexFlatIP:
@@ -116,10 +223,11 @@ class IndexFlatIP:
         return out
 
     # -- search ----------------------------------------------------------
-    def search(self, x, k: int):
-        """D, I = index.search(x, k): float32 [nq,k] descending, int64 [nq,k], -1 padded."""
+    def search(self, x, k: int, *, params: SearchParameters | None = None):
+        """D, I = index.search(x, k): float32 [nq,k] descending, int64 [nq,k], -1 padded.  ``params.sel`` restricts
+        the search to the ids it selects: the k best selected rows (``ivr_index_search_selected``)."""
         if _is_cuda_tensor(x):
-            return self.search_tensor(x, k)
+            return self.search_tensor(x, k, params=params)
         q = _as_f32_2d(x, self.d, "search(x)")
         k = int(k)
         if k <= 0:
@@ -127,13 +235,19 @@ class IndexFlatIP:
         nq = q.shape[0]
         D = np.empty((nq, k), np.float32)
         I = np.empty((nq, k), np.int64)
-        if nq:
+        sel = self._selection(params)
+        if nq and sel is None:
             nat.check(nat.lib.ivr_index_search(self._handle(), q.ctypes.data, nq, k,
                                                D.ctypes.data, I.ctypes.data, self.search_path))
+        elif nq:
+            nat.check(nat.lib.ivr_index_search_selected(self._handle(), sel, q.ctypes.data, nq, k,
+                                                        D.ctypes.data, I.ctypes.data))
         return D, I
 
-    def search_tensor(self, q, k: int, id_offset: int = 0, path: int | None = None):
-        """Device-resident search on torch's current stream; returns CUDA tensors (D, I)."""
+    def search_tensor(self, q, k: int, id_offset: int = 0, path: int | None = None,
+                      params: SearchParameters | None = None):
+        """Device-resident search on torch's current stream; returns CUDA tensors (D, I).  ``params.sel``: as in
+        ``search`` (``path`` does not apply: filtered search has one kernel)."""
         import torch
         if q.dim() != 2 or q.shape[1] != self.d:
             raise ValueError(f"search(x): expected [nq,{self.d}], got {tuple(q.shape)}")
@@ -144,11 +258,16 @@ class IndexFlatIP:
             raise ValueError("k must be positive")
         D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
         I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
-        if nq:
+        sel = self._selection(params)
+        if nq and sel is None:
             st = torch.cuda.current_stream(q.device).cuda_stream
             nat.check(nat.lib.ivr_index_search_device(
                 self._handle(), q.data_ptr(), nq, k, D.data_ptr(), I.data_ptr(), int(id_offset),
                 self.search_path if path is None else path, st))
+        elif nq:
+            st = torch.cuda.current_stream(q.device).cuda_stream
+            nat.check(nat.lib.ivr_index_search_selected_device(
+                self._handle(), sel, q.data_ptr(), nq, k, D.data_ptr(), I.data_ptr(), int(id_offset), st))
         return D, I
 
     def search_keys_tensor(self, q, k: int, id_offset: int = 0, out=None, path: int | None = None):
@@ -174,39 +293,52 @@ class IndexFlatIP:
                 self.search_path if path is None else path, st))
         return out
 
-    def range_search(self, x, radius: float):
+    def range_search(self, x, radius: float, *, params: SearchParameters | None = None):
         """lims, D, I = index.range_search(x, radius): every stored row whose inner product with the query is
         strictly greater than ``radius``.  Query i's hits are ``D[lims[i]:lims[i+1]]`` (float32, descending, ties ->
-        lower id) and ``I[lims[i]:lims[i+1]]`` (int64).  A CUDA tensor ``x`` runs ``range_search_tensor``."""
+        lower id) and ``I[lims[i]:lims[i+1]]`` (int64).  A CUDA tensor ``x`` runs ``range_search_tensor``.
+        ``params.sel`` restricts the search to the ids it selects (``ivr_index_range_search_selected``)."""
         if _is_cuda_tensor(x):
-            return self.range_search_tensor(x, radius)
+            return self.range_search_tensor(x, radius, params=params)
         q = _as_f32_2d(x, self.d, "range_search(x)")
         radius = _radius(radius)
         nq = q.shape[0]
         lims = np.zeros(nq + 1, np.int64)
         cap = _range_capacity(nq, self.ntotal)
+        sel = self._selection(params)
         while True:                                     # at most twice: the first call reports the exact total
             D = np.empty(cap, np.float32)
             I = np.empty(cap, np.int64)
-            nat.check(nat.lib.ivr_index_range_search(self._handle(), q.ctypes.data, nq, radius, cap,
-                                                     lims.ctypes.data, D.ctypes.data, I.ctypes.data))
+            if sel is None:
+                nat.check(nat.lib.ivr_index_range_search(self._handle(), q.ctypes.data, nq, radius, cap,
+                                                         lims.ctypes.data, D.ctypes.data, I.ctypes.data))
+            else:
+                nat.check(nat.lib.ivr_index_range_search_selected(self._handle(), sel, q.ctypes.data, nq, radius, cap,
+                                                                  lims.ctypes.data, D.ctypes.data, I.ctypes.data))
             total = int(lims[nq])
             if total <= cap:
                 return lims, D[:total].copy(), I[:total].copy()
             cap = total
 
-    def range_search_tensor(self, q, radius: float, id_offset: int = 0):
+    def range_search_tensor(self, q, radius: float, id_offset: int = 0, params: SearchParameters | None = None):
         """Device-resident range search on torch's current stream; returns CUDA tensors (lims, D, I), ids =
         stored row + ``id_offset``.  Sizing the outputs reads ``lims[nq]`` back to the host once (twice when more
-        hits than the first guess of the capacity turn up), so this call waits for the search to finish."""
+        hits than the first guess of the capacity turn up), so this call waits for the search to finish.
+        ``params.sel``: as in ``range_search``."""
         import torch
+        sel = self._selection(params)
 
         def call(q, radius, cap, lims, st):
             D = torch.empty(cap, dtype=torch.float32, device=q.device)
             I = torch.empty(cap, dtype=torch.int64, device=q.device)
-            nat.check(nat.lib.ivr_index_range_search_device(self._handle(), q.data_ptr(), q.shape[0], radius, cap,
-                                                            lims.data_ptr(), D.data_ptr(), I.data_ptr(),
-                                                            int(id_offset), st))
+            if sel is None:
+                nat.check(nat.lib.ivr_index_range_search_device(self._handle(), q.data_ptr(), q.shape[0], radius, cap,
+                                                                lims.data_ptr(), D.data_ptr(), I.data_ptr(),
+                                                                int(id_offset), st))
+            else:
+                nat.check(nat.lib.ivr_index_range_search_selected_device(
+                    self._handle(), sel, q.data_ptr(), q.shape[0], radius, cap, lims.data_ptr(), D.data_ptr(),
+                    I.data_ptr(), int(id_offset), st))
             return D, I
         lims, total, (D, I) = self._range_device(q, radius, call)
         return lims, D[:total], I[:total]
@@ -287,6 +419,11 @@ class IndexFlatIP:
             if total <= cap:
                 return lims, D[:total], I[:total]
             cap = total
+
+    def _selection(self, params):
+        """The device selection of ``params.sel`` for this index's device and row count; None = unfiltered."""
+        sel = getattr(params, "sel", None) if params is not None else None
+        return None if sel is None else sel._selection(self.device, self.ntotal)
 
     def _join_rows(self) -> int:
         return self._window_count if self._window_count >= 0 else self.ntotal

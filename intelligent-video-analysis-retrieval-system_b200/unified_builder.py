@@ -65,10 +65,11 @@ class UnifiedBuilderIntegration:
 
     # ---- search (unified_builder.py:190-251) ------------------------------
     def search_unified_fast(self, query_vector: "np.ndarray", k: int = 50,
-                            similarity_threshold: float = 0.0) -> List[Dict[str, Any]]:
+                            similarity_threshold: float = 0.0, videos=None) -> List[Dict[str, Any]]:
+        """``videos``: restrict the top-k to those folder names (``UnifiedIndex.search_vectors``)."""
         if not self.unified_index:
             raise ValueError("Unified index not loaded. Call load_unified_index_fast() first.")
-        results = self.unified_index.search_vectors(query_vector, k=k, filter_func=lambda meta: True)
+        results = self.unified_index.search_vectors(query_vector, k=k, filter_func=lambda meta: True, videos=videos)
         enriched = []
         for result in results:
             if result["similarity_score"] >= similarity_threshold:
@@ -83,11 +84,12 @@ class UnifiedBuilderIntegration:
         return enriched
 
     def search_unified_fast_batch(self, query_vectors, k: int = 50,
-                                  similarity_threshold: float = 0.0) -> List[List[Dict[str, Any]]]:
+                                  similarity_threshold: float = 0.0, videos=None) -> List[List[Dict[str, Any]]]:
         """``search_unified_fast`` for a batch of queries in one kernel call (same per-query result)."""
         if not self.unified_index:
             raise ValueError("Unified index not loaded. Call load_unified_index_fast() first.")
-        batches = self.unified_index.search_vectors_batch(query_vectors, k=k, filter_func=lambda meta: True)
+        batches = self.unified_index.search_vectors_batch(query_vectors, k=k, filter_func=lambda meta: True,
+                                                          videos=videos)
         out = []
         for results in batches:
             enriched = []

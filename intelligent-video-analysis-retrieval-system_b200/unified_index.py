@@ -58,6 +58,7 @@ class UnifiedIndex:
         self.faiss_index = None
         self.vectors = None
         self.metadata_list: List[Dict] = []
+        self._folder_rows: Optional[Dict[str, np.ndarray]] = None
         self.lock = threading.RLock()
 
     # ------------------------------------------------------------------ build
@@ -86,6 +87,7 @@ class UnifiedIndex:
             self.vectors = emb if keep_vectors else None
             self.metadata_list = list(metadata_list)
             self.metadata_cache = {}
+            self._folder_rows = None
             self.memory_maps = {"thumbnails": {}, "temporal": {}}
             self.is_loaded = True
         return {"processed_files": emb.shape[0], "vector_dim": emb.shape[1],
@@ -174,6 +176,7 @@ class UnifiedIndex:
                 self.vectors = emb.read() if (load_vectors and emb is not None) else None
                 self.metadata_list = r["metadata"]
                 self.metadata_cache = {}
+                self._folder_rows = None
                 self.memory_maps = {"thumbnails": {}, "temporal": {}}
                 self.is_loaded = True
         finally:
@@ -183,13 +186,17 @@ class UnifiedIndex:
 
     # ----------------------------------------------------------------- search
     def search_vectors(self, query_vector: np.ndarray, k: int = 50,
-                       filter_func: Callable = None) -> List[Dict[str, Any]]:
-        """Drop-in for unified_index.py:480-538 (one query -> list of hit dicts)."""
+                       filter_func: Callable = None, videos=None) -> List[Dict[str, Any]]:
+        """Drop-in for unified_index.py:480-538 (one query -> list of hit dicts).
+
+        ``videos`` (folder names) takes the top-k on the GPU over the frames whose ``metadata["folder_name"]`` is one
+        of them -- the k best frames of those videos, where ``filter_func`` can only drop hits from the global top-k.
+        ``filter_func`` still applies afterwards; unknown names select nothing."""
         if not self.is_loaded:
             raise ValueError("Index not loaded. Call load_unified_index() first.")
         try:
             start = time.time()
-            distances, indices = self.faiss_index.search(np.asarray(query_vector).reshape(1, -1), k)
+            distances, indices = self._search(np.asarray(query_vector).reshape(1, -1), k, videos)
             results = []
             for i, (dist, idx) in enumerate(zip(distances[0], indices[0])):
                 if idx == -1:
@@ -211,8 +218,9 @@ class UnifiedIndex:
             raise
 
     def search_vectors_batch(self, query_vectors, k: int = 50,
-                             filter_func: Callable = None) -> List[List[Dict[str, Any]]]:
-        """Many queries in ONE kernel call; element i equals ``search_vectors(query_vectors[i], k, filter_func)``.
+                             filter_func: Callable = None, videos=None) -> List[List[Dict[str, Any]]]:
+        """Many queries in ONE kernel call; element i equals ``search_vectors(query_vectors[i], k, filter_func,
+        videos)``.
 
         The reference is strictly one query per call (unified_index.py:503; system.py:733-826 loops over
         queries); batching is where the tensor-core path pays off (SURVEY.md section 8f, rank 4)."""
@@ -220,7 +228,7 @@ class UnifiedIndex:
             raise ValueError("Index not loaded. Call load_unified_index() first.")
         q = np.asarray(query_vectors)
         q = q.reshape(1, -1) if q.ndim == 1 else q.reshape(q.shape[0], -1)
-        distances, indices = self.faiss_index.search(q, k)
+        distances, indices = self._search(q, k, videos)
         out = []
         for drow, irow in zip(distances, indices):
             results = []
@@ -236,6 +244,32 @@ class UnifiedIndex:
                                 "metadata": metadata, "index": int(idx)})
             out.append(results)
         return out
+
+    def _search(self, q, k, videos):
+        """``faiss_index.search(q, k)``, restricted to the rows of ``videos`` when given."""
+        if videos is None:
+            return self.faiss_index.search(q, k)
+        sel = faiss.IDSelectorBatch(self.video_rows(videos))
+        try:
+            return self.faiss_index.search(q, k, params=faiss.SearchParameters(sel=sel))
+        finally:
+            sel.close()
+
+    def video_rows(self, videos) -> np.ndarray:
+        """Ascending row ids of the frames whose ``metadata["folder_name"]`` is in ``videos`` (a name or an iterable
+        of names); unknown names contribute nothing.  The folder -> rows map is built once per loaded index."""
+        if isinstance(videos, str):
+            videos = [videos]
+        with self.lock:
+            if self._folder_rows is None:
+                groups: Dict[str, List[int]] = {}
+                for i, meta in enumerate(self.metadata_list):
+                    name = meta.get("folder_name") if isinstance(meta, dict) else None
+                    if name is not None:
+                        groups.setdefault(name, []).append(i)
+                self._folder_rows = {name: np.asarray(rows, np.int64) for name, rows in groups.items()}
+            parts = [self._folder_rows[v] for v in set(videos) if v in self._folder_rows]
+        return np.sort(np.concatenate(parts)) if parts else np.zeros(0, np.int64)
 
     # README facade (README.md:124-136): batched, raw inner products, metadata join
     def search(self, query, top_k: int = 10):
