@@ -191,6 +191,26 @@ IVR_API int ivr_index_range_search_selected(ivr_index* idx, const ivr_selection*
 IVR_API int ivr_index_range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev,
                                                    int64_t nq, float radius, int64_t capacity, int64_t* lims_dev,
                                                    float* D_dev, int64_t* I_dev, int64_t id_offset, void* stream);
+/* The filtered searches with the hits left as PACKED exchange keys, the per-rank step of a filtered
+ * ShardedFlatIP.search / range_search.  Keys, padding (key 0) and the lims / capacity convention are those of
+ * ivr_index_search_keys_device and ivr_index_range_search_keys_device; the semantics are those of the filtered calls
+ * above, with ONE difference: these two take the handle's search window (ivr_index_set_window).  The selection is
+ * over stored rows; of them only the selected rows inside the window are scored and reported, with ids "stored row +
+ * id_offset" (the rows are not renumbered from the window's first row).  A shard that stores its neighbours'
+ * boundary rows therefore builds one selection of its stored rows, once, and searches it under whatever window its
+ * elastic boundaries give: the window's tiles are cut out of the selection's tile list on the host, without a device
+ * sync, and every row of two overlapping shards is reported by the one whose window holds it.  A selection with no
+ * selected row inside the window writes key 0 everywhere (or lims = 0) and launches no scoring kernel.  Errors,
+ * before any device call: the checks of ivr_index_search_keys_device / ivr_index_range_search_keys_device (including
+ * id_offset + ntotal > 2^32: IVR_EUNSUPPORTED) and of the filtered calls above, except that a window is allowed; a
+ * window reaching beyond ntotal is IVR_EINVAL.  ivr_index_last_timing reports them as the filtered calls above. */
+IVR_API int ivr_index_search_selected_keys_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev,
+                                                  int64_t nq, int k, uint64_t* keys_dev, int64_t id_offset,
+                                                  void* stream);
+IVR_API int ivr_index_range_search_selected_keys_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev,
+                                                        int64_t nq, float radius, int64_t capacity,
+                                                        int64_t* lims_dev, uint64_t* keys_dev, int64_t id_offset,
+                                                        void* stream);
 
 /* Search window: until cleared (count < 0) every search on this handle scores only the stored rows
  * [first, first + count) -- ids are still "stored row + id_offset", k > count pads as usual, a window reaching beyond

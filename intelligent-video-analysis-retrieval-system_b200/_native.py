@@ -69,6 +69,11 @@ PROTOTYPES = {
     "ivr_index_range_search_selected_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
                                                          C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                                          C.c_void_p]),
+    "ivr_index_search_selected_keys_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
+                                                        C.c_void_p, C.c_int64, C.c_void_p]),
+    "ivr_index_range_search_selected_keys_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                                              C.c_float, C.c_int64, C.c_void_p, C.c_void_p,
+                                                              C.c_int64, C.c_void_p]),
     "ivr_index_set_window": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64]),
     "ivr_index_set_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "ivr_index_last_timing": (C.c_int, [C.c_void_p, _c_f32p, _c_intp]),

@@ -521,10 +521,11 @@ static int join_args(const ivr_index* idx, float radius, int64_t capacity, const
     return IVR_OK;
 }
 
-// Checks shared by the filtered entry points (ivr_index_*_selected*), in an order that needs no device.
-static int selected_args(const ivr_index* idx, const ivr_selection* sel, const char* who) {
+// Checks shared by the filtered entry points (ivr_index_*_selected*), in an order that needs no device; `windowed`:
+// the call honours the handle's search window (the *_selected_keys_device calls), else a window is refused.
+static int selected_args(const ivr_index* idx, const ivr_selection* sel, const char* who, bool windowed = false) {
     if (!idx || !sel) { set_error("%s: bad argument (NULL index or selection)", who); return IVR_EINVAL; }
-    if (idx->win_count >= 0) {
+    if (!windowed && idx->win_count >= 0) {
         set_error("%s: the index has a search window; filtered search covers all stored rows (clear the window with "
                   "ivr_index_set_window(idx, 0, -1), or select only the window's rows)", who);
         return IVR_EINVAL;
@@ -541,24 +542,47 @@ static int selected_args(const ivr_index* idx, const ivr_selection* sel, const c
     return IVR_OK;
 }
 
+// The preamble of the filtered calls that honour the search window (ivr_index_*_selected_keys_device): body(cut) runs
+// on the selected rows of the window, or of every stored row, after the rows added on other streams.  The selection is
+// over stored rows, so the rows are not shifted (RowWindow): the window's tiles are cut out of the selection's list on
+// the host and ids stay "stored row + id_offset".  A window reaching past the rows is IVR_EINVAL before any device call.
+template <class Body>
+static int with_selected_window(ivr_index* idx, const ivr_selection* sel, cudaStream_t st, const char* who,
+                                Body&& body) {
+    int64_t first = 0, end = idx->ntotal;
+    if (idx->win_count >= 0) {
+        if (idx->win_first + idx->win_count > idx->ntotal) {
+            set_error("%s: the window [%lld, +%lld) reaches beyond the %lld rows of the index", who,
+                      static_cast<long long>(idx->win_first), static_cast<long long>(idx->win_count),
+                      static_cast<long long>(idx->ntotal));
+            return IVR_EINVAL;
+        }
+        first = idx->win_first;
+        end = first + idx->win_count;
+    }
+    IVR_CUDA(cudaSetDevice(idx->device));
+    if (idx->rows_ready_set) IVR_CUDA(cudaStreamWaitEvent(st, idx->rows_ready, 0));   // rows added on another stream
+    return body(selection_cut(sel, first, end));
+}
+
 // ivr_index_search_selected_device after the pointer checks: the top-k of the selected rows, on the filtered
-// small-batch kernel; no selected row below ntotal (or no row) writes the padding and scores nothing.
+// small-batch kernel; no selected row below ntotal (or no row) writes the padding and scores nothing.  `windowed`: the
+// selected rows of the search window only (ivr_index_search_selected_keys_device).  D_dev == nullptr: packed keys.
 static int search_selected_impl(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq, int k,
-                                float* D_dev, int64_t* I_dev, int64_t id_offset, cudaStream_t st) {
-    if (k <= 0) { set_error("search_selected: k must be positive (got %d)", k); return IVR_EINVAL; }
-    if (k > IVR_MAX_K) { set_error("search_selected: k=%d exceeds IVR_MAX_K=%d", k, IVR_MAX_K); return IVR_EUNSUPPORTED; }
-    IVR_TRY(selected_args(idx, sel, "search_selected"));
+                                float* D_dev, int64_t* I_dev, int64_t id_offset, cudaStream_t st,
+                                const char* who = "search_selected", bool windowed = false) {
+    if (k <= 0) { set_error("%s: k must be positive (got %d)", who, k); return IVR_EINVAL; }
+    if (k > IVR_MAX_K) { set_error("%s: k=%d exceeds IVR_MAX_K=%d", who, k, IVR_MAX_K); return IVR_EUNSUPPORTED; }
+    IVR_TRY(selected_args(idx, sel, who, windowed));
     if (small_sel_chunk(idx, k) == 0) {
-        set_error("search_selected: dim %d with k=%d does not fit one 16-query tile of the small-batch kernel",
-                  idx->dim, k);
+        set_error("%s: dim %d with k=%d does not fit one 16-query tile of the small-batch kernel", who, idx->dim, k);
         return IVR_EUNSUPPORTED;
     }
     if (nq == 0) return IVR_OK;
-    return with_search_window(idx, id_offset, st, "search_selected", [&](int64_t id_offset) {
+    auto run = [&](const SelCut& cut, int64_t id_offset) {
         idx->launches[0] = idx->launches[1] = idx->launches[2] = 0;
         idx->ev_valid[0] = idx->ev_valid[1] = idx->ev_valid[2] = false;
-        const int64_t n_tiles = selection_tiles(sel, idx->ntotal);
-        if (n_tiles == 0) {
+        if (cut.n_tiles == 0) {
             const int64_t n = nq * k;
             fill_empty_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(D_dev, I_dev, n);
             IVR_CUDA(cudaGetLastError());
@@ -566,8 +590,12 @@ static int search_selected_impl(ivr_index* idx, const ivr_selection* sel, const 
             return IVR_OK;
         }
         idx->last_path = IVR_PATH_MMA;
-        return search_mma_small_selected(idx, sel->tiles, sel->words, n_tiles, q_dev, nq, k, D_dev, I_dev, id_offset,
-                                         st);
+        return search_mma_small_selected(idx, cut, q_dev, nq, k, D_dev, I_dev, id_offset, st);
+    };
+    if (windowed)
+        return with_selected_window(idx, sel, st, who, [&](const SelCut& cut) { return run(cut, id_offset); });
+    return with_search_window(idx, id_offset, st, who, [&](int64_t id_offset) {
+        return run(selection_all(sel, idx->ntotal), id_offset);
     });
 }
 
@@ -777,8 +805,37 @@ int ivr_index_range_search_selected_device(ivr_index* idx, const ivr_selection* 
         return IVR_OK;
     }
     return with_search_window(idx, id_offset, st, "range_search_selected", [&](int64_t id_offset) {
-        return range_search_selected_device(idx, sel, q_dev, nq, radius, capacity, lims_dev, D_dev, I_dev, id_offset,
-                                            st);
+        return range_search_selected_device(idx, selection_all(sel, idx->ntotal), q_dev, nq, radius, capacity,
+                                            lims_dev, D_dev, I_dev, id_offset, st);
+    });
+}
+
+int ivr_index_search_selected_keys_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
+                                          int k, uint64_t* keys_dev, int64_t id_offset, void* stream) {
+    if (!idx || nq < 0 || (nq > 0 && (!q_dev || !keys_dev))) {
+        set_error("search_selected_keys: bad argument");
+        return IVR_EINVAL;
+    }
+    IVR_TRY(check_key_ids(idx, id_offset, "search_selected_keys"));
+    return search_selected_impl(idx, sel, q_dev, nq, k, nullptr, reinterpret_cast<int64_t*>(keys_dev), id_offset,
+                                static_cast<cudaStream_t>(stream), "search_selected_keys", /*windowed=*/true);
+}
+
+int ivr_index_range_search_selected_keys_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev,
+                                                int64_t nq, float radius, int64_t capacity, int64_t* lims_dev,
+                                                uint64_t* keys_dev, int64_t id_offset, void* stream) {
+    IVR_TRY(range_args(idx, q_dev, nq, radius, capacity, lims_dev, keys_dev, keys_dev));
+    IVR_TRY(selected_args(idx, sel, "range_search_selected_keys", /*windowed=*/true));
+    IVR_TRY(check_key_ids(idx, id_offset, "range_search_selected_keys"));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (nq == 0) {
+        IVR_CUDA(cudaSetDevice(idx->device));
+        IVR_CUDA(cudaMemsetAsync(lims_dev, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return with_selected_window(idx, sel, st, "range_search_selected_keys", [&](const SelCut& cut) {
+        return range_search_selected_keys_device(idx, cut, q_dev, nq, radius, capacity, lims_dev, keys_dev, id_offset,
+                                                 st);
     });
 }
 

@@ -64,7 +64,8 @@ struct ivr_selection {
     int64_t   count  = 0;              // selected rows
     uint32_t* words  = nullptr;        // [4 * ceil(n_rows / 128)] device bitmap, zero from row n_rows on
     uint32_t* tiles  = nullptr;        // device, ascending: the 128-row tiles that hold a selected row
-    std::vector<uint32_t> tiles_host;  // the same list, to cut it at an index's tile count
+    std::vector<uint32_t> tiles_host;  // the same list, to cut it at an index's tile count or to a search window
+    std::vector<uint32_t> words_host;  // the bitmap, to trim a window's partial first and last tiles
 };
 
 namespace ivr {
@@ -107,16 +108,31 @@ int  range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int6
 int  selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr_selection** out);
 int  selection_destroy(ivr_selection* sel);
 int64_t selection_tiles(const ivr_selection* sel, int64_t ntotal);
-// filtered top-k on the small-batch kernel (search_mma_small.cu): the n_tiles row tiles tiles[0 .. n_tiles) of a
-// selection, queries in chunks of small_sel_chunk(); small_sel_chunk() == 0: the dimension or k does not fit
+// What one filtered search streams and reports: the row tiles tiles[0 .. n_tiles) (a run of a selection's tile list)
+// and, of their rows, the selected ones in [row_lo, row_hi).  Stored-row coordinates: a search window is not shifted
+// to row 0 (RowWindow) but cut out here, because the selection's tile ids are stored tiles.
+struct SelCut {
+    const uint32_t* tiles;
+    const uint32_t* words;
+    int64_t n_tiles;
+    int64_t row_lo, row_hi;
+};
+// every selected row below ntotal (the tiles of selection_tiles)
+SelCut selection_all(const ivr_selection* sel, int64_t ntotal);
+// the selected rows of the stored rows [first, end): the tiles that hold one, found on the host (no device sync)
+SelCut selection_cut(const ivr_selection* sel, int64_t first, int64_t end);
+// filtered top-k on the small-batch kernel (search_mma_small.cu) over `cut`, queries in chunks of small_sel_chunk();
+// small_sel_chunk() == 0: the dimension or k does not fit.  D_dev == nullptr: packed keys into I_dev, as in search_mma
 int  small_sel_chunk(const ivr_index* idx, int k);
-int  search_mma_small_selected(ivr_index* idx, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles,
-                               const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev, int64_t id_offset,
-                               cudaStream_t st);
-// range_search_device over the selected rows only (range_search.cu)
-int  range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
-                                  float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
-                                  int64_t id_offset, cudaStream_t st);
+int  search_mma_small_selected(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, int k, float* D_dev,
+                               int64_t* I_dev, int64_t id_offset, cudaStream_t st);
+// range_search_device / range_search_keys_device over the selected rows of `cut` only (range_search.cu)
+int  range_search_selected_device(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, float radius,
+                                  int64_t capacity, int64_t* lims, float* D, int64_t* I, int64_t id_offset,
+                                  cudaStream_t st);
+int  range_search_selected_keys_device(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, float radius,
+                                       int64_t capacity, int64_t* lims, uint64_t* keys, int64_t id_offset,
+                                       cudaStream_t st);
 // merge of per-part sorted range runs into lims / D / I (ivr_range_merge_keys_device); no scratch, two launches
 int  range_merge_keys_device(const uint64_t* keys_parts, int64_t part_stride, const int64_t* lims_parts, int n_parts,
                              int64_t nq, int64_t* lims, float* D, int64_t* I, cudaStream_t st);

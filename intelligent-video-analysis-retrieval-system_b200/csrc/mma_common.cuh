@@ -408,12 +408,11 @@ int finish_launches(LaunchSeq& seq);
 int  search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,
                       int64_t id_offset, cudaStream_t st);
 // its range epilogue: one launch of <= small_range_chunk() queries that appends every (row, query) with
-// score > radius to the hit pool of range_search.cu; with `tiles`, only over the n_tiles row tiles listed there and the
-// rows set in the bitmap `words` (search_mma_small_sel_range_kernel)
+// score > radius to the hit pool of range_search.cu; with `cut`, only over the row tiles and rows of that part of a
+// selection (search_mma_small_sel_range_kernel)
 int  search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
                             float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
-                            cudaStream_t st, const uint32_t* tiles = nullptr, const uint32_t* words = nullptr,
-                            int64_t n_tiles = 0);
+                            cudaStream_t st, const SelCut* cut = nullptr);
 // its self-join epilogue: one launch that appends both (i, j) and (j, i) of every pair i < j of the stored rows with
 // score > radius to the hit pool of range_search.cu
 int  search_mma_small_join(ivr_index* idx, float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx,

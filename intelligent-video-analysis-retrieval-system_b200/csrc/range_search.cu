@@ -8,7 +8,8 @@
 //   3. if the pool held them all: histogram by query, exclusive scan into lims, scatter into the query segments,
 //      segmented sort descending (the key order: score descending, then lower row), unpack to D / I.
 // Step 3 reads the cursor on the device, so nothing here waits for the GPU.  A filtered search (ivr_selection) runs
-// step 2 on search_mma_small_sel_range_kernel over the selection's row tiles only.  The self-join (range_self_join_device)
+// step 2 on search_mma_small_sel_range_kernel over the row tiles of a cut of the selection only (SelCut: all stored rows,
+// or a search window's).  The self-join (range_self_join_device)
 // fills the same pool from the join kernel, with the stored rows as queries, and shares step 3.  Algorithmic bytes:
 // ntotal * dpad * 2 per query chunk, plus 12 bytes per hit in the pool and 12 in the output.
 #include "mma_common.cuh"
@@ -138,12 +139,11 @@ static int range_pool_sorted(ivr_index* idx, Carve carve, int64_t nq, int64_t ca
 // The body shared by both range entry points: score every query chunk into the pool, group and sort it into lims /
 // the sorted pool, then finish(sorted, cursor, q_scale, grid, threads) queues the last step, which writes the
 // caller's output.
-// With a selection, only the rows it selects are scored, and a selection without a row below ntotal scores nothing.
+// With a cut of a selection, only the rows it selects are scored, and a cut without a tile scores nothing.
 template <class Finish>
 static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
-                               int64_t* lims, cudaStream_t st, Finish&& finish, const ivr_selection* sel = nullptr) {
-    const int64_t n_tiles = sel ? selection_tiles(sel, idx->ntotal) : 0;
-    if (idx->ntotal == 0 || (sel && n_tiles == 0)) {
+                               int64_t* lims, cudaStream_t st, Finish&& finish, const SelCut* cut = nullptr) {
+    if (idx->ntotal == 0 || (cut && cut->n_tiles == 0)) {
         IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nq + 1) * sizeof(int64_t), st));
         return IVR_OK;
     }
@@ -163,7 +163,7 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
             IVR_TRY(launch_queries_to_f16(q_dev + q0 * idx->dim, q_h, q_scale + q0, tau_g, m, (m + 15) / 16 * 16,
                                           idx->dim, idx->dpad, st));
             IVR_TRY(search_mma_small_range(idx, q_h, q_scale + q0, m, q0, radius, cursor, keys, qidx, capacity, st,
-                                           sel ? sel->tiles : nullptr, sel ? sel->words : nullptr, n_tiles));
+                                           cut));
         }
         return IVR_OK;
     }, [&](const char* ws, const uint64_t* sorted, const unsigned long long* cursor, int grid, int threads) {
@@ -171,8 +171,9 @@ static int range_search_sorted(ivr_index* idx, const float* q_dev, int64_t nq, f
     });
 }
 
-int range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const float* q_dev, int64_t nq,
-                                 float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I, int64_t id_offset,
+// range search with the hits unpacked to D / I (cut == nullptr: every row)
+static int range_search_unpacked(ivr_index* idx, const SelCut* cut, const float* q_dev, int64_t nq, float radius,
+                                 int64_t capacity, int64_t* lims, float* D, int64_t* I, int64_t id_offset,
                                  cudaStream_t st) {
     return range_search_sorted(idx, q_dev, nq, radius, capacity, lims, st,
                                [&](const uint64_t* sorted, const unsigned long long* cursor, const float* q_scale,
@@ -180,16 +181,12 @@ int range_search_selected_device(ivr_index* idx, const ivr_selection* sel, const
         range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nq, q_scale, id_offset, D, I);
         IVR_CUDA(cudaGetLastError());
         return IVR_OK;
-    }, sel);
+    }, cut);
 }
 
-int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
-                        int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st) {
-    return range_search_selected_device(idx, nullptr, q_dev, nq, radius, capacity, lims, D, I, id_offset, st);
-}
-
-int range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
-                             int64_t* lims, uint64_t* keys, int64_t id_offset, cudaStream_t st) {
+// range search with the hits left as exchange keys (cut == nullptr: every row)
+static int range_search_packed(ivr_index* idx, const SelCut* cut, const float* q_dev, int64_t nq, float radius,
+                               int64_t capacity, int64_t* lims, uint64_t* keys, int64_t id_offset, cudaStream_t st) {
     return range_search_sorted(idx, q_dev, nq, radius, capacity, lims, st,
                                [&](const uint64_t* sorted, const unsigned long long* cursor, const float* q_scale,
                                    int grid, int threads) {
@@ -197,7 +194,29 @@ int range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, flo
                                                          keys);
         IVR_CUDA(cudaGetLastError());
         return IVR_OK;
-    });
+    }, cut);
+}
+
+int range_search_selected_device(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, float radius,
+                                 int64_t capacity, int64_t* lims, float* D, int64_t* I, int64_t id_offset,
+                                 cudaStream_t st) {
+    return range_search_unpacked(idx, &cut, q_dev, nq, radius, capacity, lims, D, I, id_offset, st);
+}
+
+int range_search_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                        int64_t* lims, float* D, int64_t* I, int64_t id_offset, cudaStream_t st) {
+    return range_search_unpacked(idx, nullptr, q_dev, nq, radius, capacity, lims, D, I, id_offset, st);
+}
+
+int range_search_selected_keys_device(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, float radius,
+                                      int64_t capacity, int64_t* lims, uint64_t* keys, int64_t id_offset,
+                                      cudaStream_t st) {
+    return range_search_packed(idx, &cut, q_dev, nq, radius, capacity, lims, keys, id_offset, st);
+}
+
+int range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, float radius, int64_t capacity,
+                             int64_t* lims, uint64_t* keys, int64_t id_offset, cudaStream_t st) {
+    return range_search_packed(idx, nullptr, q_dev, nq, radius, capacity, lims, keys, id_offset, st);
 }
 
 __global__ void range_fill_kernel(float* __restrict__ x, int64_t n, float v) {

@@ -33,6 +33,8 @@
 // search_mma_small_sel_kernel and search_mma_small_sel_range_kernel: the producer streams the row tiles of the
 // selection's tile list, and each epilogue warp ANDs its 32 rows' bitmap word into the row-validity test.  The kernel
 // bodies are templates on the row-tile source (AllRows / SelRows), so the unfiltered kernels compile as before.
+// A filtered search under a search window streams the UNSHIFTED stored rows: the host cuts the window's tiles out of
+// the selection's list, p.n_rows ends the window and SelRows::row_lo starts it (windows need not be tile-aligned).
 //
 // Replaces D, I = index.search(x, k) for small batches (unified_index.py:503, core.py:891).
 // Algorithmic bytes: ntotal * dpad * 2 per search.
@@ -124,8 +126,9 @@ __device__ __forceinline__ void small_setup(const SmallSmem& sm, const CUtensorM
 
 // Which row tiles a launch streams and which of their rows it may report.  The unfiltered kernels stream the
 // consecutive tiles tile0 + j and report every row; the filtered ones (search_mma_small_sel*_kernel) stream tile
-// tiles[j] of a selection's tile list and report the rows whose bit is set in its bitmap: bit lane of word
-// tile * 4 + quarter is row tile * 128 + quarter * 32 + lane, the 32 rows one epilogue warp drains.
+// tiles[j] of a selection's tile list and report the rows at or above row_lo whose bit is set in its bitmap: bit lane of
+// word tile * 4 + quarter is row tile * 128 + quarter * 32 + lane, the 32 rows one epilogue warp drains.  row_lo is the
+// first row of a search window (0 without one); the window's end is SmallParams::n_rows.
 struct AllRows {
     int64_t tile0;
     __device__ __forceinline__ int64_t tile(int64_t j) const { return tile0 + j; }
@@ -135,9 +138,10 @@ struct AllRows {
 struct SelRows {
     const uint32_t* tiles;             // ascending tile ids; position j of the launch is tiles[j]
     const uint32_t* words;             // the row bitmap, zero-padded to whole tiles
+    int64_t         row_lo;            // rows below it are not reported
     __device__ __forceinline__ int64_t tile(int64_t j) const { return __ldg(tiles + j); }
     __device__ __forceinline__ bool selected(int64_t t, int quarter, int lane) const {
-        return (__ldg(words + t * 4 + quarter) >> lane) & 1u;
+        return t * kSmallTileRows + quarter * 32 + lane >= row_lo && ((__ldg(words + t * 4 + quarter) >> lane) & 1u);
     }
     __device__ __forceinline__ bool dump(const SmallParams&) const { return false; }
 };
@@ -366,11 +370,13 @@ search_mma_small_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
 }
 
 // Filtered top-k: the list epilogue over the row tiles of a selection (SelRows).  p.tile0 and p.nt count positions in
-// the selection's tile list, so the seeded launches split the list as the unfiltered ones split the rows.  No dump mode.
+// the selection's tile list, so the seeded launches split the list as the unfiltered ones split the rows.  Rows below
+// row_lo or at or past p.n_rows are never reported.  No dump mode.
 __global__ void __launch_bounds__(kSmallThreads, 1)
 search_mma_small_sel_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
-                            const SmallParams p, const uint32_t* __restrict__ tiles, const uint32_t* __restrict__ words) {
-    small_topk(tmap_q, tmap_x, p, SelRows{tiles + p.tile0, words});
+                            const SmallParams p, const uint32_t* __restrict__ tiles, const uint32_t* __restrict__ words,
+                            int64_t row_lo) {
+    small_topk(tmap_q, tmap_x, p, SelRows{tiles + p.tile0, words, row_lo});
 }
 
 // The largest fp32 t with fp32(t * scale) <= radius, so that "score > t" is exactly "the reported score, fp32(score *
@@ -507,12 +513,12 @@ search_mma_small_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const 
 }
 
 // Filtered range search: the fixed-threshold epilogue over the row tiles of a selection (SelRows); p.nt counts
-// positions in the selection's tile list.
+// positions in the selection's tile list; rows below row_lo or at or past p.n_rows are never reported.
 __global__ void __launch_bounds__(kSmallThreads, 1)
 search_mma_small_sel_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
                                   const SmallRangeParams p, const uint32_t* __restrict__ tiles,
-                                  const uint32_t* __restrict__ words) {
-    small_range(tmap_q, tmap_x, p, SelRows{tiles, words});
+                                  const uint32_t* __restrict__ words, int64_t row_lo) {
+    small_range(tmap_q, tmap_x, p, SelRows{tiles, words, row_lo});
 }
 
 // JOIN mode (range_self_join of range_search.cu): both operands are stored rows.  A unit of work is (column block b,
@@ -742,12 +748,13 @@ static int search_mma_small_dump(ivr_index* idx, const SmallShape& sh, const flo
 }
 
 // The seeded candidate-list launches over nt row tiles (for the filtered kernel: positions in a selection's tile list),
-// merged into D / I.  launch(grid, tmq, tmx, p) queues one scoring launch of `kernel`.  time_first marks the query
-// preparation and the start of the scoring, time_last the end of the scoring and the final merge.
+// merged into D / I (packed keys into I when D == nullptr); rows at or past n_rows are not reported.
+// launch(grid, tmq, tmx, p) queues one scoring launch of `kernel`.  time_first marks the query preparation and the start
+// of the scoring, time_last the end of the scoring and the final merge.
 template <class Launch>
 static int small_list_search(ivr_index* idx, const SmallShape& sh, const float* q_dev, int64_t nq, int k, float* D_dev,
-                             int64_t* I_dev, int64_t id_offset, cudaStream_t st, int64_t nt, const void* kernel,
-                             bool time_first, bool time_last, Launch&& launch) {
+                             int64_t* I_dev, int64_t id_offset, cudaStream_t st, int64_t nt, int64_t n_rows,
+                             const void* kernel, bool time_first, bool time_last, Launch&& launch) {
     const int sms = idx->sm_count;
     // launch boundaries (in row tiles): one tile per CTA, then as many rows as keep the expected admissions per
     // list around 64 (k * rows_now / rows_before spread over 4 * sms lists), then the rest
@@ -780,7 +787,7 @@ static int small_list_search(ivr_index* idx, const SmallShape& sh, const float* 
     timing_mark(idx, time_first, kScoreBegin, st);
     for (int ph = 0; ph < n_phases; ++ph) {
         SmallParams p{};
-        p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad; p.k = k; p.C = sh.C;
+        p.n_rows = n_rows; p.nq = static_cast<int>(nq); p.npad = sh.npad; p.k = k; p.C = sh.C;
         p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
         p.tile0 = bounds[ph]; p.nt = bounds[ph + 1] - bounds[ph];
         p.row_policy = kL2EvictFirst;                                // every row is read exactly once
@@ -816,7 +823,7 @@ int search_mma_small(ivr_index* idx, const float* q_dev, int64_t nq, int k, floa
     const int64_t dump_rows = static_cast<int64_t>(env_int("IVR_SMALL_DUMP_MAX_KROWS", 3500)) * 1000;
     if (k <= kSelectMaxK && idx->ntotal <= dump_rows && sh.npad * 4 * 6 <= idx->dpad * 2)
         return search_mma_small_dump(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st);
-    IVR_TRY(small_list_search(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st, nt,
+    IVR_TRY(small_list_search(idx, sh, q_dev, nq, k, D_dev, I_dev, id_offset, st, nt, idx->ntotal,
                               reinterpret_cast<const void*>(search_mma_small_kernel), idx->timing, idx->timing,
                               [&](int grid, const CUtensorMap& tmq, const CUtensorMap& tmx, const SmallParams& p) {
         search_mma_small_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p);
@@ -832,9 +839,8 @@ int small_sel_chunk(const ivr_index* idx, int k) {
     return 0;
 }
 
-int search_mma_small_selected(ivr_index* idx, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles,
-                              const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev, int64_t id_offset,
-                              cudaStream_t st) {
+int search_mma_small_selected(ivr_index* idx, const SelCut& cut, const float* q_dev, int64_t nq, int k, float* D_dev,
+                              int64_t* I_dev, int64_t id_offset, cudaStream_t st) {
     const int chunk = small_sel_chunk(idx, k);
     if (chunk == 0) {
         set_error("search_selected: dim %d with k=%d does not fit the small-batch kernel", idx->dim, k);
@@ -845,11 +851,13 @@ int search_mma_small_selected(ivr_index* idx, const uint32_t* tiles, const uint3
         const int64_t q0 = c * chunk, m = std::min<int64_t>(chunk, nq - q0);
         SmallShape sh;
         small_shape(idx, m, k, &sh);                                 // fits: m <= chunk
-        IVR_TRY(small_list_search(idx, sh, q_dev + q0 * idx->dim, m, k, D_dev + q0 * k, I_dev + q0 * k, id_offset, st,
-                                  n_tiles, reinterpret_cast<const void*>(search_mma_small_sel_kernel),
+        IVR_TRY(small_list_search(idx, sh, q_dev + q0 * idx->dim, m, k, D_dev ? D_dev + q0 * k : nullptr,
+                                  I_dev + q0 * k, id_offset, st, cut.n_tiles, cut.row_hi,
+                                  reinterpret_cast<const void*>(search_mma_small_sel_kernel),
                                   idx->timing && c == 0, idx->timing && c == n_chunks - 1,
                                   [&](int grid, const CUtensorMap& tmq, const CUtensorMap& tmx, const SmallParams& p) {
-            search_mma_small_sel_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p, tiles, words);
+            search_mma_small_sel_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, tmx, p, cut.tiles, cut.words,
+                                                                              cut.row_lo);
         }));
     }
     idx->last_kernel = "search_mma_small_sel_kernel";
@@ -862,7 +870,7 @@ int small_range_chunk(const ivr_index* idx) {
 
 int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_scale, int64_t nq, int64_t q_base,
                            float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx, int64_t capacity,
-                           cudaStream_t st, const uint32_t* tiles, const uint32_t* words, int64_t n_tiles) {
+                           cudaStream_t st, const SelCut* cut) {
     SmallShape sh;
     if (nq > small_range_chunk(idx) || !pipe_shape(idx, nq, &sh)) {
         set_error("range_search: %lld queries of dim %d do not fit one query tile", static_cast<long long>(nq), idx->dim);
@@ -872,18 +880,19 @@ int search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sca
     const CUtensorMap* tmx;
     IVR_TRY(make_tmap(&tmq, q_h, sh.npad, idx->dpad, sh.npad));
     IVR_TRY(row_tmap(idx, kSmallTileRows, &tmx));
-    const void* kernel = tiles ? reinterpret_cast<const void*>(search_mma_small_sel_range_kernel)
-                               : reinterpret_cast<const void*>(search_mma_small_range_kernel);
+    const void* kernel = cut ? reinterpret_cast<const void*>(search_mma_small_sel_range_kernel)
+                             : reinterpret_cast<const void*>(search_mma_small_range_kernel);
     IVR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sh.smem)));
     SmallRangeParams p{};
-    p.n_rows = idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad;
+    p.n_rows = cut ? cut->row_hi : idx->ntotal; p.nq = static_cast<int>(nq); p.npad = sh.npad;
     p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
-    p.nt = tiles ? n_tiles : (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
+    p.nt = cut ? cut->n_tiles : (idx->ntotal + kSmallTileRows - 1) / kSmallTileRows;
     p.row_policy = kL2EvictFirst;                                    // each launch reads every row once
     p.radius = radius; p.q_scale = q_scale; p.q_base = static_cast<uint32_t>(q_base);
     p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
     const int grid = static_cast<int>(std::min<int64_t>(idx->sm_count, std::max<int64_t>(p.nt, 1)));
-    if (tiles) search_mma_small_sel_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p, tiles, words);
+    if (cut) search_mma_small_sel_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p, cut->tiles, cut->words,
+                                                                                    cut->row_lo);
     else search_mma_small_range_kernel<<<grid, kSmallThreads, sh.smem, st>>>(tmq, *tmx, p);
     IVR_CUDA(cudaGetLastError());
     return IVR_OK;

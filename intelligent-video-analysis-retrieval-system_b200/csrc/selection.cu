@@ -5,6 +5,8 @@
 // of the small-batch kernel drains -- so the list is one OR per tile and a compaction.  Both are built once per
 // selection and read by every filtered search: the producer warp streams tiles[j], the epilogue warps AND their
 // word into the row-validity test (search_mma_small.cu).  100 M rows: 12.5 MB of bitmap, at most 3 MB of tile list.
+// The host keeps a copy of both, so that a search can cut a window's tiles out of the list without touching the device
+// (selection_cut): the sharded index searches a different window of the same selection whenever its boundaries move.
 #include "index.cuh"
 
 #include <cub/device/device_select.cuh>
@@ -52,10 +54,12 @@ int selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr
     sel->device = device;
     sel->n_rows = n_rows;
     const int64_t n_tiles = (n_rows + 127) / 128, n_words = (n_rows + 31) / 32;
+    sel->words_host.resize(static_cast<size_t>(n_words));
     for (int64_t w = 0; w < n_words; ++w) {
-        const uint32_t word = words_host[w];
         const int64_t left = n_rows - w * 32;
-        sel->count += __builtin_popcount(left >= 32 ? word : word & ((1u << left) - 1u));
+        const uint32_t word = left >= 32 ? words_host[w] : words_host[w] & ((1u << left) - 1u);
+        sel->words_host[w] = word;
+        sel->count += __builtin_popcount(word);
     }
     if (n_tiles == 0) { *out = sel; return IVR_OK; }
 
@@ -105,10 +109,37 @@ int selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr
     return IVR_OK;
 }
 
-int64_t selection_tiles(const ivr_selection* sel, int64_t ntotal) {
-    const int64_t nt = (ntotal + 127) / 128;
-    return std::lower_bound(sel->tiles_host.begin(), sel->tiles_host.end(), static_cast<uint64_t>(nt),
-                            [](uint32_t t, uint64_t v) { return t < v; }) - sel->tiles_host.begin();
+// position of the first tile id >= t in the selection's tile list
+static int64_t tile_pos(const ivr_selection* sel, int64_t t) {
+    return std::lower_bound(sel->tiles_host.begin(), sel->tiles_host.end(), static_cast<uint64_t>(t),
+                            [](uint32_t v, uint64_t x) { return v < x; }) - sel->tiles_host.begin();
+}
+
+int64_t selection_tiles(const ivr_selection* sel, int64_t ntotal) { return tile_pos(sel, (ntotal + 127) / 128); }
+
+SelCut selection_all(const ivr_selection* sel, int64_t ntotal) {
+    return SelCut{sel->tiles, sel->words, selection_tiles(sel, ntotal), 0, ntotal};
+}
+
+// whether the host bitmap selects a row of [a, b)
+static bool any_selected(const ivr_selection* sel, int64_t a, int64_t b) {
+    b = std::min(b, sel->n_rows);
+    for (int64_t r = a; r < b; ++r)
+        if ((sel->words_host[r >> 5] >> (r & 31)) & 1u) return true;
+    return false;
+}
+
+// The tiles from first / 128 to ceil(end / 128) by two binary searches; a partial first or last tile whose selected rows
+// all lie outside the window is dropped, so an empty cut means "no selected row in the window".
+SelCut selection_cut(const ivr_selection* sel, int64_t first, int64_t end) {
+    int64_t lo = tile_pos(sel, first / 128), hi = tile_pos(sel, (end + 127) / 128);
+    if (lo < hi && first % 128 != 0 && sel->tiles_host[lo] == first / 128 &&
+        !any_selected(sel, first, std::min(end, (first / 128 + 1) * 128)))
+        ++lo;
+    if (lo < hi && end % 128 != 0 && sel->tiles_host[hi - 1] == end / 128 &&
+        !any_selected(sel, std::max(first, end / 128 * 128), end))
+        --hi;
+    return SelCut{sel->tiles + lo, sel->words, hi - lo, first, end};
 }
 
 }  // namespace ivr

@@ -41,7 +41,10 @@ def _as_f32_2d(x, d=None, what="x"):
 class IDSelector:
     """Base of the id selectors.  ``words(ntotal)`` is the selection over ids [0, ntotal) as packed uint32 words (bit
     ``i & 31`` of word ``i >> 5`` = id i), the layout of ``ivr_selection_create``.  The device selection built from it
-    is cached per (device, ntotal) and freed by ``close`` (or when the selector is collected)."""
+    is cached per (device, ntotal) and freed by ``close`` (or when the selector is collected).
+
+    A row shard applies a selector of GLOBAL ids to the rows it stores: ``slice_words`` / ``shard`` give the selection
+    of ids [first, first + count) renumbered from 0, cached per (device, ntotal_global, first, count)."""
 
     def words(self, ntotal: int) -> np.ndarray:
         return _pack_words(self._mask(int(ntotal)))
@@ -59,6 +62,44 @@ class IDSelector:
             nat.check(nat.lib.ivr_selection_create(int(device), w.ctypes.data, int(ntotal), C.byref(h)))
             cache[key] = h
         return h
+
+    def slice_words(self, ntotal_global: int, first: int, count: int) -> np.ndarray:
+        """The ids [first, first + count) of this selection over ``ntotal_global`` ids as packed words over ``count``
+        local rows: bit 0 is id ``first``.  Ids at or past ``ntotal_global`` are not selected."""
+        first, count = int(first), int(count)
+        if first < 0 or count < 0:
+            raise ValueError(f"slice_words: first ({first}) and count ({count}) must be >= 0")
+        m = self._mask(int(ntotal_global))[first:first + count]
+        return _pack_words(np.concatenate([m, np.zeros(count - m.size, bool)]))
+
+    def _slice_selection(self, device: int, ntotal_global: int, first: int, count: int):
+        cache = self.__dict__.setdefault("_sel_cache", {})
+        key = (int(device), int(ntotal_global), int(first), int(count))
+        h = cache.get(key)
+        if h is None:
+            w = self.slice_words(ntotal_global, first, count)
+            h = C.c_void_p()
+            nat.check(nat.lib.ivr_selection_create(int(device), w.ctypes.data, int(count), C.byref(h)))
+            cache[key] = h
+        return h
+
+    def shard(self, ntotal_global: int, first: int) -> "IDSelector":
+        """This selector of ids [0, ntotal_global) as seen by a shard whose stored row 0 is global id ``first``: a
+        selector of stored rows, for the per-rank filtered searches of ``ShardedFlatIP``."""
+        return _ShardSelector(self, int(ntotal_global), int(first))
+
+    def fingerprint(self, ntotal_global: int) -> tuple:
+        """(selected ids below ntotal_global, a 64-bit hash of the packed words): ranks compare it to find out that they
+        were given different selectors.  Cached per ntotal_global."""
+        import hashlib
+        cache = self.__dict__.setdefault("_fp_cache", {})
+        fp = cache.get(int(ntotal_global))
+        if fp is None:
+            w = self.words(int(ntotal_global))
+            h = hashlib.blake2b(w.astype("<u4").tobytes(), digest_size=8).digest()
+            fp = (int(np.unpackbits(w.view(np.uint8)).sum()), int.from_bytes(h, "little", signed=True))
+            cache[int(ntotal_global)] = fp
+        return fp
 
     def count(self, ntotal: int, device: int | None = None) -> int:
         """Selected ids below ``ntotal`` (computed by the device selection when ``device`` is given)."""
@@ -83,6 +124,24 @@ def _pack_words(mask: np.ndarray) -> np.ndarray:
     b = np.packbits(np.asarray(mask, bool), bitorder="little")
     b = np.concatenate([b, np.zeros(-b.size % 4, np.uint8)])
     return b.view("<u4").astype(np.uint32)
+
+
+class _ShardSelector(IDSelector):
+    """``IDSelector.shard``: ids [first, first + ntotal) of ``sel`` over ``ntotal_global`` ids, renumbered from 0.  Its
+    device selections are ``sel``'s slice selections (cached and freed there), so a new view per search costs nothing."""
+
+    def __init__(self, sel: IDSelector, ntotal_global: int, first: int):
+        self.sel, self.ntotal_global, self.first = sel, ntotal_global, first
+
+    def _mask(self, ntotal):
+        m = self.sel._mask(self.ntotal_global)[self.first:self.first + ntotal]
+        return np.concatenate([m, np.zeros(ntotal - m.size, bool)])
+
+    def _selection(self, device, ntotal):
+        return self.sel._slice_selection(device, self.ntotal_global, self.first, ntotal)
+
+    def close(self):
+        pass
 
 
 class IDSelectorRange(IDSelector):
@@ -270,10 +329,14 @@ class IndexFlatIP:
                 self._handle(), sel, q.data_ptr(), nq, k, D.data_ptr(), I.data_ptr(), int(id_offset), st))
         return D, I
 
-    def search_keys_tensor(self, q, k: int, id_offset: int = 0, out=None, path: int | None = None):
+    def search_keys_tensor(self, q, k: int, id_offset: int = 0, out=None, path: int | None = None,
+                           params: SearchParameters | None = None):
         """Device-resident search that leaves the hits as packed 64-bit keys (int64 tensor [nq, k] holding
         ``order_preserving(score) << 32 | ~(row + id_offset)``, 0 = padding): the 8-byte-per-hit payload of the
-        cross-shard exchange (``ShardedFlatIP``).  ``out`` may be a preallocated contiguous int64 [nq, k] tensor."""
+        cross-shard exchange (``ShardedFlatIP``).  ``out`` may be a preallocated contiguous int64 [nq, k] tensor.
+        ``params.sel`` selects stored rows, as in ``search``; unlike ``search`` the filtered call honours the search
+        window (``set_window``): only the selected rows inside it are reported (``ivr_index_search_selected_keys_device``;
+        ``path`` does not apply)."""
         import torch
         if q.dim() != 2 or q.shape[1] != self.d:
             raise ValueError(f"search(x): expected [nq,{self.d}], got {tuple(q.shape)}")
@@ -286,11 +349,16 @@ class IndexFlatIP:
             out = torch.empty((nq, k), dtype=torch.int64, device=q.device)
         elif out.shape != (nq, k) or out.dtype != torch.int64 or not out.is_contiguous():
             raise ValueError("out must be a contiguous int64 [nq, k] tensor")
-        if nq:
+        sel = self._selection(params)
+        if nq and sel is None:
             st = torch.cuda.current_stream(q.device).cuda_stream
             nat.check(nat.lib.ivr_index_search_keys_device(
                 self._handle(), q.data_ptr(), nq, k, out.data_ptr(), int(id_offset),
                 self.search_path if path is None else path, st))
+        elif nq:
+            st = torch.cuda.current_stream(q.device).cuda_stream
+            nat.check(nat.lib.ivr_index_search_selected_keys_device(
+                self._handle(), sel, q.data_ptr(), nq, k, out.data_ptr(), int(id_offset), st))
         return out
 
     def range_search(self, x, radius: float, *, params: SearchParameters | None = None):
@@ -343,18 +411,26 @@ class IndexFlatIP:
         lims, total, (D, I) = self._range_device(q, radius, call)
         return lims, D[:total], I[:total]
 
-    def range_search_keys_tensor(self, q, radius: float, id_offset: int = 0):
+    def range_search_keys_tensor(self, q, radius: float, id_offset: int = 0, params: SearchParameters | None = None):
         """``range_search_tensor`` with the hits left as packed 64-bit keys: returns CUDA int64 tensors (lims, keys),
         query i's hits are ``keys[lims[i]:lims[i+1]]`` holding ``order_preserving(score) << 32 | ~(row + id_offset)``
         in descending unsigned order (score descending, then lower id).  The per-rank step of
-        ``ShardedFlatIP.range_search``; global ids must stay below 2^32."""
+        ``ShardedFlatIP.range_search``; global ids must stay below 2^32.  ``params.sel``: as in
+        ``search_keys_tensor``, the selected stored rows inside the search window
+        (``ivr_index_range_search_selected_keys_device``)."""
         import torch
+        sel = self._selection(params)
 
         def call(q, radius, cap, lims, st):
             keys = torch.empty(cap, dtype=torch.int64, device=q.device)
-            nat.check(nat.lib.ivr_index_range_search_keys_device(self._handle(), q.data_ptr(), q.shape[0], radius,
-                                                                 cap, lims.data_ptr(), keys.data_ptr(),
-                                                                 int(id_offset), st))
+            if sel is None:
+                nat.check(nat.lib.ivr_index_range_search_keys_device(self._handle(), q.data_ptr(), q.shape[0], radius,
+                                                                     cap, lims.data_ptr(), keys.data_ptr(),
+                                                                     int(id_offset), st))
+            else:
+                nat.check(nat.lib.ivr_index_range_search_selected_keys_device(
+                    self._handle(), sel, q.data_ptr(), q.shape[0], radius, cap, lims.data_ptr(), keys.data_ptr(),
+                    int(id_offset), st))
             return (keys,)
         lims, total, (keys,) = self._range_device(q, radius, call)
         return lims, keys[:total]

@@ -229,8 +229,16 @@ class ShardedFlatIP:
     partition / offset / gather logic with a stand-in backend that speaks the same packed-key
     protocol: ``search_keys_tensor(q, k, id_offset, out)`` and ``merge(keys [world, nq, k], k)``; for
     ``range_search`` also ``range_search_tensor`` / ``range_search_keys_tensor(q, radius, id_offset)`` and
-    ``range_merge(keys [world, stride], lims [world, nq + 1], total)``); by default they are the CUDA index and the
-    CUDA merge kernels and fail loudly without a GPU.
+    ``range_merge(keys [world, stride], lims [world, nq + 1], total)``; for filtered searches the same calls with
+    ``params=`` holding a selector of stored rows, which must honour ``set_window``); by default they are the CUDA
+    index and the CUDA merge kernels and fail loudly without a GPU.
+
+    FILTERED SEARCH (``params=SearchParameters(sel=...)``): ``sel`` selects GLOBAL ids.  Each rank searches the
+    selector's slice of the rows it stores (``IDSelector.shard``: one device selection per selector, built once and
+    kept across boundary moves) under its current window, so the rows two ranks both store are reported by exactly
+    one of them; the keys take the unfiltered exchange and merge unchanged.  A filtered search streams only the
+    selected row tiles, so its time says nothing about a rank's row count: it sets the window but is not a timed
+    search of the elastic controller (no ``balance_log`` entry, no step of the search counter).
     """
 
     def __init__(self, d: int, group=None, device: Optional[int] = None,
@@ -402,36 +410,74 @@ class ShardedFlatIP:
         return float(self.local.ntotal) / (sum(ms) / len(ms))
 
     # ---- search --------------------------------------------------------
-    def search(self, q, k: int):
+    def search(self, q, k: int, params=None):
         """q: [nq, d] tensor (CUDA for the product path), replicated on every rank.
-        Returns (D [nq,k] float32 descending, I [nq,k] int64 global ids) on every rank."""
-        return self.search_async(q, k).result(copy=True)
+        Returns (D [nq,k] float32 descending, I [nq,k] int64 global ids) on every rank.  ``params``: see
+        ``search_async``."""
+        return self.search_async(q, k, params=params).result(copy=True)
 
-    def search_async(self, q, k: int) -> PendingSearch:
+    def search_async(self, q, k: int, params=None) -> PendingSearch:
         """Queue one search and return at once.  The local scoring runs on the current stream; with the peer
         exchange the push / arrival wait / merge run on the index's side stream, so the NEXT ``search_async`` starts
-        scoring while this one's exchange is still waiting for slower ranks.  Searches complete in issue order."""
+        scoring while this one's exchange is still waiting for slower ranks.  Searches complete in issue order.
+
+        ``params=SearchParameters(sel=...)`` restricts the search to the global ids ``sel`` selects: the k best of
+        them, padded with -1 / -FLT_MAX (see the class docstring).  Like ``q``, ``params`` must be the same on every
+        rank.  A filtered search takes a mailbox slot in issue order like any other, so filtered and unfiltered
+        ``search_async`` calls may be mixed; it is not a timed search of the elastic controller."""
         import torch
         import torch.distributed as dist
         k = int(k)
+        lp = self._local_params(q, params, k=k)
+        kw = {} if lp is None else {"params": lp}
         if self.world == 1:
-            D, I = self.local.search_tensor(q, k, id_offset=self.id_offset)
+            D, I = self.local.search_tensor(q, k, id_offset=self.id_offset, **kw)
             return PendingSearch(D, I, None, None)
         nq = q.shape[0]
         if self.exchange == "peer" and nq > 0 and self._ensure_mailbox(nq * k, q.device):
-            return self._search_peer(q, nq, k)
+            return self._search_peer(q, nq, k, kw)
         if self._keys is None or self._keys.shape != (nq, k) or self._keys.device != q.device:
             self._keys = torch.empty((nq, k), dtype=torch.int64, device=q.device)
             self._gathered = torch.empty((self.world, nq, k), dtype=torch.int64, device=q.device)
-        i = self._elastic_begin(q) if self._bounds is not None else -1
-        self.local.search_keys_tensor(q, k, id_offset=self.id_offset, out=self._keys)
+        i = self._local_begin(q, lp)
+        self.local.search_keys_tensor(q, k, id_offset=self.id_offset, out=self._keys, **kw)
         if i >= 0:
             self._timer.stop(i)
         dist.all_gather_into_tensor(self._gathered.view(self.world * nq, k), self._keys, group=self.group)
         D, I = self._merge(self._gathered, k)
         return PendingSearch(D, I, None, None)
 
-    def range_search(self, q, radius: float):
+    def _local_params(self, q, params, k=None, radius=None):
+        """The local index's ``params`` for a search with ``params`` (None = unfiltered): the selector's slice of the
+        rows this rank stores.  The argument checks of a filtered search run here, before any collective or mailbox
+        push; they depend only on arguments that are the same on every rank, so every rank raises alike."""
+        sel = getattr(params, "sel", None) if params is not None else None
+        if sel is None:
+            return None
+        from ._native import IVR_MAX_K
+        from .faiss_compat import IDSelector, SearchParameters
+        if not isinstance(sel, IDSelector):
+            raise TypeError(f"params.sel must be an IDSelector, got {type(sel).__name__}")
+        if q.dim() != 2 or q.shape[1] != self.d:
+            raise ValueError(f"search(x): expected [nq,{self.d}], got {tuple(q.shape)}")
+        if k is not None and not 1 <= k <= IVR_MAX_K:
+            raise ValueError(f"k must be in 1..{IVR_MAX_K} (got {k})")
+        if radius is not None and float(radius) != float(radius):
+            raise ValueError("range_search: radius is NaN")
+        return SearchParameters(sel=sel.shard(self.ntotal_global, self.id_offset))
+
+    def _local_begin(self, q, lp) -> int:
+        """Before a search's local scoring: the window of the current boundaries.  An unfiltered search is also a
+        timed search of the elastic controller (returns its number, -1 without elastic boundaries); a filtered one
+        (``lp`` not None) streams only its selected tiles and is not timed (returns -1)."""
+        if self._bounds is None:
+            return -1
+        if lp is not None:
+            self._set_window()
+            return -1
+        return self._elastic_begin(q)
+
+    def range_search(self, q, radius: float, params=None):
         """Exact range search over the rows of every rank: every row whose inner product with a query is strictly
         greater than ``radius``.  q: [nq, d] tensor, the same on every rank (as for ``search``).  Returns tensors
         (lims int64 [nq + 1], D float32, I int64 global ids) on q's device, identical on every rank; query i's hits
@@ -447,13 +493,20 @@ class ShardedFlatIP:
         The exchange always uses these collectives over ``group``, never the peer mailboxes (their slots are sized
         for nq * k and pipelined).  So ``range_search`` may be called between ``search_async`` calls: its scoring
         queues on the current stream behind theirs, it blocks the host until its run lengths are known, it takes no
-        mailbox slot, and the pending searches still complete in issue order."""
+        mailbox slot, and the pending searches still complete in issue order.
+
+        ``params=SearchParameters(sel=...)``: only the global ids ``sel`` selects (see the class docstring).  The
+        status row then also carries the selector's fingerprint (its selected count and a hash of its words), so ranks
+        called with different selectors all raise the same ``ValueError``.  ``params`` must be given on every rank or
+        on none."""
         import torch
         import torch.distributed as dist
+        lp = self._local_params(q, params, radius=radius)
+        kw = {} if lp is None else {"params": lp}
         if self._bounds is not None:
             self._set_window()
         if self.world == 1:
-            return self.local.range_search_tensor(q, radius, id_offset=self.id_offset)
+            return self.local.range_search_tensor(q, radius, id_offset=self.id_offset, **kw)
         nq, dev = q.shape[0], q.device
         if nq == 0:                                      # replicated queries: every rank takes this branch
             return (torch.zeros(1, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.float32, device=dev),
@@ -462,13 +515,14 @@ class ShardedFlatIP:
         err, rbits = None, 0
         try:
             rbits = int(np.float32(radius).view(np.int32))
-            lims, keys = self.local.range_search_keys_tensor(q, radius, id_offset=self.id_offset)
+            lims, keys = self.local.range_search_keys_tensor(q, radius, id_offset=self.id_offset, **kw)
         except Exception as e:
             err = e
             lims, keys = torch.zeros(nq + 1, dtype=torch.int64, device=dev), None
         # a batch of another size would also change the row length: queries must be replicated, as for search
-        row = torch.cat([lims, torch.tensor([0 if err is None else 1, nq, rbits], dtype=torch.int64, device=dev)])
-        rows = torch.empty((self.world, nq + 4), dtype=torch.int64, device=dev)
+        fp = [] if lp is None else list(params.sel.fingerprint(self.ntotal_global))
+        row = torch.cat([lims, torch.tensor([0 if err is None else 1, nq, rbits] + fp, dtype=torch.int64, device=dev)])
+        rows = torch.empty((self.world, nq + 4 + len(fp)), dtype=torch.int64, device=dev)
         dist.all_gather_into_tensor(rows.view(-1), row, group=self.group)
         host = rows.cpu().numpy()
         failed = np.nonzero(host[:, nq + 1])[0]
@@ -480,6 +534,13 @@ class ShardedFlatIP:
                 return f"nq={int(host[r, nq + 2])} radius={float(np.int32(host[r, nq + 3]).view(np.float32))}"
             raise ValueError(f"range_search: rank {int(differ[0])} was called with {call(int(differ[0]))}, "
                              f"rank 0 with {call(0)}")
+        if fp:
+            differ = np.nonzero(np.any(host[:, nq + 4:] != host[0, nq + 4:], axis=1))[0]
+            if differ.size:
+                def call(r):
+                    return f"a selector of {int(host[r, nq + 4])} ids (hash {int(host[r, nq + 5]) & ((1 << 64) - 1):016x})"
+                raise ValueError(f"range_search: rank {int(differ[0])} was called with {call(int(differ[0]))}, "
+                                 f"rank 0 with {call(0)}")
         totals = host[:, nq]
         stride = int(totals.max())
         gathered = torch.empty((self.world, 0), dtype=torch.int64, device=dev)
@@ -546,7 +607,7 @@ class ShardedFlatIP:
             self._comm = torch.cuda.Stream(device=device)
         return True
 
-    def _search_peer(self, q, nq: int, k: int) -> PendingSearch:
+    def _search_peer(self, q, nq: int, k: int, kw) -> PendingSearch:
         import torch
         S = _PeerExchange.SLOTS
         if self._slots is None or self._slots[0]["keys"].shape != (nq, k) or self._slots[0]["keys"].device != q.device:
@@ -562,8 +623,8 @@ class ShardedFlatIP:
         cur = torch.cuda.current_stream(q.device)
         if b["pushed"] is not None:                     # the push of search (step - S) has read this keys buffer
             cur.wait_event(b["pushed"])
-        i = self._elastic_begin(q) if self._bounds is not None else -1
-        self.local.search_keys_tensor(q, k, id_offset=self.id_offset, out=b["keys"])
+        i = self._local_begin(q, kw.get("params"))
+        self.local.search_keys_tensor(q, k, id_offset=self.id_offset, out=b["keys"], **kw)
         if i >= 0:
             self._timer.stop(i)
         scored = torch.cuda.Event()
