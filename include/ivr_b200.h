@@ -155,6 +155,37 @@ IVR_API int ivr_index_range_self_join(ivr_index* idx, float radius, int64_t capa
 IVR_API int ivr_index_range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev,
                                              float* D_dev, int64_t* I_dev, void* stream);
 
+/* ---- the pieces of a self-join across row shards (ShardedFlatIP.range_self_join) ------------------------------
+ * The stored fp16 rows [first, first + n) (all stored rows, whatever the search window) copied to dst, dpad halves
+ * per row (dpad = ivr_index_dpad: dim padded to a multiple of 64), with cudaMemcpyAsync on `stream`.  A NULL index,
+ * NULL dst with n > 0, first < 0, n < 0 or a range past ntotal are IVR_EINVAL. */
+IVR_API int ivr_index_dpad(const ivr_index* idx);
+IVR_API int ivr_index_rows_f16_device(ivr_index* idx, int64_t first, int64_t n, void* dst, void* stream);
+/* ivr_index_range_self_join_device with the hits left as PACKED exchange keys (the format of
+ * ivr_index_search_keys_device): keys[lims[i] : lims[i+1]] = make_key(score, partner stored row + id_offset), in the
+ * order of D / I.  Same contract and checks as ivr_index_range_self_join_device; in addition id_offset < 0 or
+ * id_offset + ntotal > 2^32 is IVR_EUNSUPPORTED. */
+IVR_API int ivr_index_range_self_join_keys_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev,
+                                                  uint64_t* keys_dev, int64_t id_offset, void* stream);
+/* The rows of the search window (n_self of them; all stored rows without one) against n_other other rows: every
+ * pair (window row i, other row j) whose inner product is strictly greater than `radius`, each pair scored once.
+ *   other_rows      fp16 [n_other, dpad] on the index's device, global ids other_first_id + j
+ *   other_is_lower  nonzero when the other rows' global ids are below the window's; that set is the streamed operand,
+ *                   as the lower row i of a pair is in ivr_index_range_self_join, so a pair scores the same bits
+ *   lims  int64  [n_self + n_other + 1]  window row i's hits are keys[lims[i] : lims[i+1]], other row j's are
+ *                                        keys[lims[n_self + j] : lims[n_self + j + 1]]
+ *   keys  uint64 [capacity]  make_key(score, global id of the partner), descending within a row; a window row's
+ *                            global id is its stored row + id_offset
+ * The capacity convention is that of ivr_index_range_search.  Checks, before any device call and in this order: a
+ * NaN radius, a negative capacity or n_other, a NULL index, lims, keys with capacity > 0, or other_rows with
+ * n_other > 0 are IVR_EINVAL; capacity above 2^31-1, padded dim above 4096, n_self + n_other of 2^31-1 or more, and a
+ * global id reaching 2^32 (id_offset < 0, id_offset + ntotal > 2^32, other_first_id < 0 or other_first_id + n_other >
+ * 2^32) are IVR_EUNSUPPORTED.  More than 2^31-1 work units run as several launches.  Never blocks the host. */
+IVR_API int ivr_index_range_cross_join_keys_device(ivr_index* idx, const void* other_rows, int64_t n_other,
+                                                   int64_t other_first_id, int other_is_lower, float radius,
+                                                   int64_t capacity, int64_t* lims_dev, uint64_t* keys_dev,
+                                                   int64_t id_offset, void* stream);
+
 /* ---- filtered search: a device row selection -----------------------------------------------------------------
  * Replaces SearchParameters(sel=IDSelector...) on faiss.IndexFlatIP.search / range_search (the reference can only
  * post-filter the global top-k: unified_index.py:185-238).  A selection is built once from a packed host bitmap --

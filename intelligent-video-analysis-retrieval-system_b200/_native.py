@@ -57,6 +57,13 @@ PROTOTYPES = {
     "ivr_index_range_self_join": (C.c_int, [C.c_void_p, C.c_float, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ivr_index_range_self_join_device": (C.c_int, [C.c_void_p, C.c_float, C.c_int64, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_void_p]),
+    "ivr_index_dpad": (C.c_int, [C.c_void_p]),
+    "ivr_index_rows_f16_device": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
+    "ivr_index_range_self_join_keys_device": (C.c_int, [C.c_void_p, C.c_float, C.c_int64, C.c_void_p, C.c_void_p,
+                                                        C.c_int64, C.c_void_p]),
+    "ivr_index_range_cross_join_keys_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int,
+                                                         C.c_float, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                                         C.c_void_p]),
     "ivr_selection_create": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
     "ivr_selection_destroy": (C.c_int, [C.c_void_p]),
     "ivr_selection_count": (C.c_int64, [C.c_void_p]),

@@ -897,6 +897,76 @@ int ivr_index_range_self_join(ivr_index* idx, float radius, int64_t capacity, in
     return IVR_OK;
 }
 
+int ivr_index_dpad(const ivr_index* idx) { return idx ? idx->dpad : -1; }
+
+int ivr_index_rows_f16_device(ivr_index* idx, int64_t first, int64_t n, void* dst, void* stream) {
+    if (!idx || (n > 0 && !dst) || first < 0 || n < 0 || first + n > idx->ntotal) {
+        set_error("rows_f16: bad argument (NULL index or dst, or rows [%lld, +%lld) outside the %lld stored rows)",
+                  static_cast<long long>(first), static_cast<long long>(n),
+                  static_cast<long long>(idx ? idx->ntotal : 0));
+        return IVR_EINVAL;
+    }
+    if (n == 0) return IVR_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    IVR_CUDA(cudaSetDevice(idx->device));
+    if (idx->rows_ready_set) IVR_CUDA(cudaStreamWaitEvent(st, idx->rows_ready, 0));   // rows added on another stream
+    IVR_CUDA(cudaMemcpyAsync(dst, idx->rows + first * idx->dpad, static_cast<size_t>(n) * idx->dpad * sizeof(__half),
+                             cudaMemcpyDeviceToDevice, st));
+    return IVR_OK;
+}
+
+int ivr_index_range_self_join_keys_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims_dev,
+                                          uint64_t* keys_dev, int64_t id_offset, void* stream) {
+    IVR_TRY(join_args(idx, radius, capacity, lims_dev, keys_dev, keys_dev));
+    IVR_TRY(check_key_ids(idx, id_offset, "range_self_join_keys"));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return with_search_window(idx, id_offset, st, "range_self_join_keys", [&](int64_t id_offset) {
+        return range_self_join_keys_device(idx, radius, capacity, lims_dev, keys_dev, id_offset, st);
+    });
+}
+
+int ivr_index_range_cross_join_keys_device(ivr_index* idx, const void* other_rows, int64_t n_other,
+                                           int64_t other_first_id, int other_is_lower, float radius,
+                                           int64_t capacity, int64_t* lims_dev, uint64_t* keys_dev,
+                                           int64_t id_offset, void* stream) {
+    if (radius != radius) { set_error("range_cross_join: radius is NaN"); return IVR_EINVAL; }
+    if (capacity < 0 || n_other < 0) {
+        set_error("range_cross_join: capacity and n_other must be >= 0 (got %lld, %lld)",
+                  static_cast<long long>(capacity), static_cast<long long>(n_other));
+        return IVR_EINVAL;
+    }
+    if (!idx || !lims_dev || (capacity > 0 && !keys_dev) || (n_other > 0 && !other_rows)) {
+        set_error("range_cross_join: bad argument (NULL index or buffer)");
+        return IVR_EINVAL;
+    }
+    if (capacity > INT_MAX) {
+        set_error("range_cross_join: at most 2^31-1 hits per call (capacity %lld)", static_cast<long long>(capacity));
+        return IVR_EUNSUPPORTED;
+    }
+    if (small_range_chunk(idx) < 16) {
+        set_error("range_cross_join: dim %d is wider than the small-batch kernel holds (padded dim <= 4096)", idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    const int64_t n_self = idx->win_count >= 0 ? idx->win_count : idx->ntotal;
+    if (n_self + n_other >= INT_MAX) {
+        set_error("range_cross_join: at most 2^31-2 rows on both sides together (%lld + %lld)",
+                  static_cast<long long>(n_self), static_cast<long long>(n_other));
+        return IVR_EUNSUPPORTED;
+    }
+    IVR_TRY(check_key_ids(idx, id_offset, "range_cross_join"));
+    if (other_first_id < 0 || other_first_id + n_other > 0x100000000ll) {
+        set_error("range_cross_join: global row ids must stay below 2^32 (other rows %lld + %lld)",
+                  static_cast<long long>(other_first_id), static_cast<long long>(n_other));
+        return IVR_EUNSUPPORTED;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return with_search_window(idx, id_offset, st, "range_cross_join", [&](int64_t id_offset) {
+        return range_cross_join_keys_device(idx, static_cast<const __half*>(other_rows), n_other, other_is_lower != 0,
+                                            static_cast<uint32_t>(id_offset), static_cast<uint32_t>(other_first_id),
+                                            radius, capacity, lims_dev, keys_dev, st);
+    });
+}
+
 int ivr_index_set_timing(ivr_index* idx, int enable) {
     if (!idx) { set_error("NULL index"); return IVR_EINVAL; }
     idx->timing = enable != 0;

@@ -103,6 +103,15 @@ int  range_search_keys_device(ivr_index* idx, const float* q_dev, int64_t nq, fl
 // lims [ntotal + 1], D, I = every pair of distinct current rows with score > radius, by first row (range_search.cu)
 int  range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
                             int64_t id_offset, cudaStream_t st);
+// the same join, hits left as exchange keys make_key(score, row + id_offset) in the order of D / I
+int  range_self_join_keys_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, uint64_t* keys,
+                                 int64_t id_offset, cudaStream_t st);
+// every pair (current row i, other row j) with score > radius, as exchange keys of global ids: lims [n + n_other + 1]
+// holds the current rows' segments, then the other rows'; current row i is global id self_id0 + i, other row j
+// other_id0 + j (range_search.cu)
+int  range_cross_join_keys_device(ivr_index* idx, const __half* other, int64_t n_other, bool other_is_lower,
+                                  uint32_t self_id0, uint32_t other_id0, float radius, int64_t capacity, int64_t* lims,
+                                  uint64_t* keys, cudaStream_t st);
 // row selections (selection.cu): build the device bitmap and tile list of a new handle; the number of tiles of the
 // list that lie below an index of ntotal rows
 int  selection_create(int device, const uint32_t* words_host, int64_t n_rows, ivr_selection** out);

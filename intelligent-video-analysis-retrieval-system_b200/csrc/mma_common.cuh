@@ -417,5 +417,10 @@ int  search_mma_small_range(ivr_index* idx, const __half* q_h, const float* q_sc
 // score > radius to the hit pool of range_search.cu
 int  search_mma_small_join(ivr_index* idx, float radius, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx,
                            int64_t capacity, cudaStream_t st);
+// its cross-join epilogue: every pair (stored row i, other row j) with score > radius, two pool entries each, keys of
+// global ids (self_id0 + i, other_id0 + j), segments i and n + j; one launch per 2^31-1 work units
+int  search_mma_small_cross_join(ivr_index* idx, const __half* other, int64_t n_other, bool other_is_lower,
+                                 uint32_t self_id0, uint32_t other_id0, float radius, unsigned long long* cursor,
+                                 uint64_t* keys, uint32_t* qidx, int64_t capacity, cudaStream_t st);
 
 }  // namespace ivr

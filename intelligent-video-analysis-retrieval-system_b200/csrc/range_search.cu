@@ -225,6 +225,24 @@ __global__ void range_fill_kernel(float* __restrict__ x, int64_t n, float v) {
         x[i] = v;
 }
 
+// The joins' pool over nseg segments: score(cursor, keys, qidx) fills it, the grouping is range search's, and
+// finish(sorted, cursor, ones, grid, threads) writes the output with scales of one (join scores are not rescaled).
+template <class Score, class Finish>
+static int join_pool_sorted(ivr_index* idx, int64_t nseg, int64_t capacity, int64_t* lims, cudaStream_t st,
+                            Score&& score, Finish&& finish) {
+    Carve carve;
+    const size_t o_one = carve(static_cast<size_t>(nseg) * 4);
+    return range_pool_sorted(idx, carve, nseg, capacity, lims, st,
+                             [&](char*, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx) {
+        return score(cursor, keys, qidx);
+    }, [&](const char* ws, const uint64_t* sorted, const unsigned long long* cursor, int grid, int threads) {
+        float* ones = reinterpret_cast<float*>(const_cast<char*>(ws) + o_one);
+        range_fill_kernel<<<grid, threads, 0, st>>>(ones, nseg, 1.0f);
+        IVR_CUDA(cudaGetLastError());
+        return finish(sorted, cursor, static_cast<const float*>(ones), grid, threads);
+    });
+}
+
 // lims, D, I = range_self_join(radius): the join kernel (search_mma_small.cu) puts both (i, j) and (j, i) of every
 // pair into the pool, segmented by the first row; the grouping is range search's, and the unpack's scales are ones.
 int range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, float* D, int64_t* I,
@@ -234,16 +252,48 @@ int range_self_join_device(ivr_index* idx, float radius, int64_t capacity, int64
         IVR_CUDA(cudaMemsetAsync(lims, 0, sizeof(int64_t), st));
         return IVR_OK;
     }
-    Carve carve;
-    const size_t o_one = carve(static_cast<size_t>(n) * 4);
-    return range_pool_sorted(idx, carve, n, capacity, lims, st,
-                             [&](char*, unsigned long long* cursor, uint64_t* keys, uint32_t* qidx) {
+    return join_pool_sorted(idx, n, capacity, lims, st, [&](unsigned long long* cursor, uint64_t* keys, uint32_t* qidx) {
         return search_mma_small_join(idx, radius, cursor, keys, qidx, capacity, st);
-    }, [&](const char* ws, const uint64_t* sorted, const unsigned long long* cursor, int grid, int threads) {
-        float* ones = reinterpret_cast<float*>(const_cast<char*>(ws) + o_one);
-        range_fill_kernel<<<grid, threads, 0, st>>>(ones, n, 1.0f);
-        IVR_CUDA(cudaGetLastError());
+    }, [&](const uint64_t* sorted, const unsigned long long* cursor, const float* ones, int grid, int threads) {
         range_unpack_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, n, ones, id_offset, D, I);
+        IVR_CUDA(cudaGetLastError());
+        return IVR_OK;
+    });
+}
+
+// The self-join with its hits left as exchange keys (ShardedFlatIP.range_self_join: a rank's own window).
+int range_self_join_keys_device(ivr_index* idx, float radius, int64_t capacity, int64_t* lims, uint64_t* keys,
+                                int64_t id_offset, cudaStream_t st) {
+    const int64_t n = idx->ntotal;
+    if (n == 0) {
+        IVR_CUDA(cudaMemsetAsync(lims, 0, sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return join_pool_sorted(idx, n, capacity, lims, st, [&](unsigned long long* cursor, uint64_t* pool, uint32_t* qidx) {
+        return search_mma_small_join(idx, radius, cursor, pool, qidx, capacity, st);
+    }, [&](const uint64_t* sorted, const unsigned long long* cursor, const float* ones, int grid, int threads) {
+        range_pack_keys_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, n, ones, id_offset, keys);
+        IVR_CUDA(cudaGetLastError());
+        return IVR_OK;
+    });
+}
+
+// The current rows against `other`: the cross-join kernel writes keys of global ids already, so the pack adds no
+// offset.  Segments [0, n) are the current rows, [n, n + n_other) the other rows; an empty side scores nothing.
+int range_cross_join_keys_device(ivr_index* idx, const __half* other, int64_t n_other, bool other_is_lower,
+                                 uint32_t self_id0, uint32_t other_id0, float radius, int64_t capacity, int64_t* lims,
+                                 uint64_t* keys, cudaStream_t st) {
+    const int64_t n = idx->ntotal, nseg = n + n_other;
+    if (n == 0 || n_other == 0) {
+        IVR_CUDA(cudaMemsetAsync(lims, 0, static_cast<size_t>(nseg + 1) * sizeof(int64_t), st));
+        return IVR_OK;
+    }
+    return join_pool_sorted(idx, nseg, capacity, lims, st,
+                            [&](unsigned long long* cursor, uint64_t* pool, uint32_t* qidx) {
+        return search_mma_small_cross_join(idx, other, n_other, other_is_lower, self_id0, other_id0, radius, cursor,
+                                           pool, qidx, capacity, st);
+    }, [&](const uint64_t* sorted, const unsigned long long* cursor, const float* ones, int grid, int threads) {
+        range_pack_keys_kernel<<<grid, threads, 0, st>>>(sorted, cursor, capacity, lims, nseg, ones, 0, keys);
         IVR_CUDA(cudaGetLastError());
         return IVR_OK;
     });

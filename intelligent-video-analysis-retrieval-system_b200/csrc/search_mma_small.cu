@@ -28,7 +28,9 @@
 // The per-(CTA, warp) survivors are folded by topk_merge.cu.
 // A third epilogue, with a fixed threshold, runs in its own __global__ (search_mma_small_range_kernel) for the exact
 // range search of range_search.cu; it shares the producer and MMA code below.  A fourth, search_mma_small_join_kernel,
-// serves the self-join of range_search.cu: stored rows on both operands, the upper triangle of the score matrix.
+// serves the self-join of range_search.cu: stored rows on both operands, the upper triangle of the score matrix.  A
+// fifth, search_mma_small_cross_join_kernel, scores the whole rectangle of two different row sets (one rank's window
+// against another rank's rows in ShardedFlatIP.range_self_join).
 // Filtered search (ivr_selection, selection.cu) runs the top-k and range epilogues in their own __global__ functions,
 // search_mma_small_sel_kernel and search_mma_small_sel_range_kernel: the producer streams the row tiles of the
 // selection's tile list, and each epilogue warp ANDs its 32 rows' bitmap word into the row-validity test.  The kernel
@@ -660,6 +662,121 @@ search_mma_small_join_kernel(const __grid_constant__ CUtensorMap tmap_b, const _
     if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
 }
 
+// CROSS-JOIN mode (range_cross_join_keys_device of range_search.cu): two different row sets, A (the one with the lower
+// global ids, streamed in 128-row tiles) and B (npad-row blocks resident in shared memory).  Every pair (i in A, j in
+// B) is scored, so a unit is (column block b, segment s) of the full rectangle; units are numbered segment-major,
+// u = s * nb + b, and a launch covers units [u0, u0 + gridDim.x).  Row ids in the pool are global: A row i is
+// a_id0 + i and lands in segment a_seg0 + i, B row j likewise.
+struct SmallCrossParams {
+    int64_t  n_a, n_b;                 // rows of A and of B
+    int      npad, kblocks, stages, nbuf, buf_cols;
+    int      seg_tiles;                // row tiles of A per segment
+    int64_t  nb;                       // column blocks of B
+    int64_t  u0;                       // first unit of this launch
+    uint64_t row_policy;
+    float    radius;
+    uint32_t a_id0, b_id0;             // global id of row 0 of A / of B
+    uint32_t a_seg0, b_seg0;           // pool segment of row 0 of A / of B
+    unsigned long long* cursor;        // pool entries reserved so far
+    uint64_t* keys;                    // [capacity] make_key(score, global id of the partner)
+    uint32_t* qidx;                    // [capacity] the segment of the row the entry belongs to
+    unsigned long long capacity;
+};
+
+// One CTA per unit.  The epilogue keeps (i, j) with i < n_a, j < n_b and score > radius -- the bounds are explicit
+// because the zero-filled rows past either end score 0, which exceeds a negative radius -- and appends two pool entries
+// per pair, one for each row, from one 64-bit cursor reservation per warp and 32-column chunk.  Entries at or past
+// `capacity` are dropped but counted.
+__global__ void __launch_bounds__(kSmallThreads, 1)
+search_mma_small_cross_join_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_a,
+                                   const SmallCrossParams p) {
+    extern __shared__ __align__(1024) uint8_t smem_raw[];
+    const SmallSmem sm(smem_raw, p.npad, p.kblocks, p.stages);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+    const int64_t u = p.u0 + blockIdx.x;
+    const int64_t s = u / p.nb, b = u - s * p.nb;
+    const int64_t jb = b * p.npad;                                     // first B row of the block
+    const int64_t t_end = (p.n_a + kSmallTileRows - 1) / kSmallTileRows;
+    const int64_t t0 = s * p.seg_tiles, t1 = t0 + p.seg_tiles < t_end ? t0 + p.seg_tiles : t_end;
+
+    small_setup(sm, &tmap_b, &tmap_a, p.stages, p.nbuf, warp, lane);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    uint32_t tmem_base;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(sm.tmem_slot()));
+
+    if (warp == 0 && lane == 0) {
+        small_produce_join(sm, &tmap_b, static_cast<int>(jb), &tmap_a, p.kblocks, p.stages, t0, t1, p.row_policy);
+    } else if (warp == 1 && lane == 0) {
+        small_mma(sm, tmem_base, p.npad, p.kblocks, p.stages, p.nbuf, p.buf_cols, t0, t1);
+    } else if (warp >= 2) {
+        // ============================ epilogue: the rectangle, fixed threshold ========
+        const int quarter = warp & 3;                              // the TMEM lanes this warp may read
+        int buf = 0; uint32_t bphase = 0;
+        for (int64_t t = t0; t < t1; ++t) {
+            const int64_t i = t * kSmallTileRows + quarter * 32 + lane;
+            mbar_wait(sm.tfull_bar(buf), bphase);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
+                                   static_cast<uint32_t>(buf * p.buf_cols);
+            for (int c0 = 0; c0 < p.npad; c0 += 32) {
+                uint32_t v[32];
+                if (p.npad - c0 >= 32) {
+                    tmem_ld_32x32(taddr + c0, v);
+                } else {                                            // npad is a multiple of 16: a 16-column tail
+#pragma unroll
+                    for (int k = 16; k < 32; ++k) v[k] = 0xff800000u;
+                    tmem_ld_32x16(taddr + c0, v);
+                }
+                tmem_wait_ld(v);
+                if (c0 + 32 >= p.npad) {                            // accumulator fully read: hand it back
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_local(sm.tempty_bar(buf));
+                }
+                unsigned m = 0;
+#pragma unroll
+                for (int k = 0; k < 32; ++k) m |= (__uint_as_float(v[k]) > p.radius ? 1u : 0u) << k;
+                // column k is B row j = jc + k: keep i < n_a and j < n_b
+                const int64_t jc = jb + c0;
+                const int64_t below = p.n_b - jc;                   // keep k < below
+                if (i >= p.n_a) m = 0;
+                m &= below >= 32 ? 0xffffffffu : (below <= 0 ? 0u : (1u << below) - 1u);
+                const int cnt = __popc(m);
+                int incl = cnt;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int x = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += x;
+                }
+                const int total = __shfl_sync(0xffffffffu, incl, 31);
+                if (total == 0) continue;                           // warp-uniform
+                unsigned long long slot = 0;
+                if (lane == 0) slot = atomicAdd(p.cursor, 2ull * static_cast<unsigned long long>(total));
+                slot = __shfl_sync(0xffffffffu, slot, 0) + 2ull * static_cast<unsigned long long>(incl - cnt);
+                const uint32_t id_i = p.a_id0 + static_cast<uint32_t>(i), seg_i = p.a_seg0 + static_cast<uint32_t>(i);
+#pragma unroll
+                for (int k = 0; k < 32; ++k) {
+                    if (!((m >> k) & 1u)) continue;
+                    const float sc = __uint_as_float(v[k]);
+                    const uint32_t j = static_cast<uint32_t>(jc + k);
+                    if (slot < p.capacity)     { p.keys[slot] = make_key(sc, p.b_id0 + j); p.qidx[slot] = seg_i; }
+                    if (slot + 1 < p.capacity) { p.keys[slot + 1] = make_key(sc, id_i); p.qidx[slot + 1] = p.b_seg0 + j; }
+                    slot += 2;
+                }
+            }
+            if (++buf == p.nbuf) { buf = 0; bphase ^= 1; }
+        }
+    }
+
+    // ------------------------------------------------------------------ teardown ----
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
+}
+
 // ------------------------------------------------------------------ host side ----
 struct SmallShape { int npad, stages, nbuf, buf_cols, C; size_t smem; };
 
@@ -937,6 +1054,56 @@ int search_mma_small_join(ivr_index* idx, float radius, unsigned long long* curs
                                   static_cast<int>(sh.smem)));
     search_mma_small_join_kernel<<<static_cast<unsigned>(units), kSmallThreads, sh.smem, st>>>(tmb, tmx, p);
     IVR_CUDA(cudaGetLastError());
+    return IVR_OK;
+}
+
+// The rectangle of the (windowed) index rows against `other` ([n_other, dpad] fp16 on the index's device).  The set
+// with the lower global ids is A, as i is in the self-join, so a pair's score has the bits the single-index join gives
+// it.  More units than one launch holds (2^31-1; IVR_JOIN_MAX_UNITS lowers the limit) are split into launches over
+// consecutive unit ranges.
+int search_mma_small_cross_join(ivr_index* idx, const __half* other, int64_t n_other, bool other_is_lower,
+                                uint32_t self_id0, uint32_t other_id0, float radius, unsigned long long* cursor,
+                                uint64_t* keys, uint32_t* qidx, int64_t capacity, cudaStream_t st) {
+    const int64_t n_self = idx->ntotal;
+    const int npad = small_range_chunk(idx);
+    SmallShape sh;
+    if (!pipe_shape(idx, npad, &sh)) {
+        set_error("range_cross_join: dim %d does not fit the small-batch kernel", idx->dim);
+        return IVR_EUNSUPPORTED;
+    }
+    SmallCrossParams p{};
+    p.n_a = other_is_lower ? n_other : n_self;
+    p.n_b = other_is_lower ? n_self : n_other;
+    p.npad = sh.npad;
+    p.kblocks = idx->dpad / kKBlock; p.stages = sh.stages; p.nbuf = sh.nbuf; p.buf_cols = sh.buf_cols;
+    p.seg_tiles = 40;                                                // ~40 row tiles per unit, as in the self-join
+    p.nb = (p.n_b + npad - 1) / npad;
+    p.row_policy = kL2EvictNormal;                                   // other CTAs re-read the same row tiles
+    p.radius = radius;
+    p.a_id0 = other_is_lower ? other_id0 : self_id0;
+    p.b_id0 = other_is_lower ? self_id0 : other_id0;
+    p.a_seg0 = other_is_lower ? static_cast<uint32_t>(n_self) : 0u;
+    p.b_seg0 = other_is_lower ? 0u : static_cast<uint32_t>(n_self);
+    p.cursor = cursor; p.keys = keys; p.qidx = qidx; p.capacity = static_cast<unsigned long long>(capacity);
+    const int64_t n_seg = ((p.n_a + kSmallTileRows - 1) / kSmallTileRows + p.seg_tiles - 1) / p.seg_tiles;
+    const int64_t units = n_seg * p.nb;
+    if (units == 0) return IVR_OK;
+    const CUtensorMap* cached;
+    IVR_TRY(row_tmap(idx, other_is_lower ? npad : kSmallTileRows, &cached));
+    const CUtensorMap tmi = *cached;
+    CUtensorMap tmo;
+    IVR_TRY(make_tmap(&tmo, other, n_other, idx->dpad, other_is_lower ? kSmallTileRows : npad));
+    const CUtensorMap& tma = other_is_lower ? tmo : tmi;
+    const CUtensorMap& tmb = other_is_lower ? tmi : tmo;
+    IVR_CUDA(cudaFuncSetAttribute(search_mma_small_cross_join_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(sh.smem)));
+    const int64_t max_units = std::max<int64_t>(1, std::min<int64_t>(INT_MAX, env_int("IVR_JOIN_MAX_UNITS", INT_MAX)));
+    for (int64_t u0 = 0; u0 < units; u0 += max_units) {
+        p.u0 = u0;
+        const int64_t grid = std::min(max_units, units - u0);
+        search_mma_small_cross_join_kernel<<<static_cast<unsigned>(grid), kSmallThreads, sh.smem, st>>>(tmb, tma, p);
+        IVR_CUDA(cudaGetLastError());
+    }
     return IVR_OK;
 }
 

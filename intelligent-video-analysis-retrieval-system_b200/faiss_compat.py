@@ -496,6 +496,76 @@ class IndexFlatIP:
                 return lims, D[:total], I[:total]
             cap = total
 
+    @property
+    def dpad(self) -> int:
+        """The storage dimension: d padded to a multiple of 64 (the row stride of ``rows_f16_tensor``)."""
+        return int(nat.lib.ivr_index_dpad(self._handle()))
+
+    def rows_f16_tensor(self, first: int, n: int):
+        """The stored fp16 rows [first, first + n) (whatever the search window) as a new CUDA float16 tensor
+        [n, dpad], copied on torch's current stream: the rows ``ShardedFlatIP.range_self_join`` sends to a peer."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        out = torch.empty((int(n), self.dpad), dtype=torch.float16, device=dev)
+        nat.check(nat.lib.ivr_index_rows_f16_device(self._handle(), int(first), int(n), out.data_ptr(),
+                                                    torch.cuda.current_stream(dev).cuda_stream))
+        return out
+
+    def range_self_join_keys_tensor(self, radius: float, id_offset: int = 0):
+        """``range_self_join_tensor`` with the hits left as packed 64-bit keys: CUDA int64 tensors (lims, keys), row
+        i's hits are ``keys[lims[i]:lims[i+1]]`` holding ``order_preserving(score) << 32 | ~(partner + id_offset)``
+        (partner = stored row), unsigned descending.  The diagonal step of ``ShardedFlatIP.range_self_join``; global
+        ids must stay below 2^32."""
+        import torch
+        radius = _radius(radius, "range_self_join")
+        n = self._join_rows()
+        dev = torch.device("cuda", self.device)
+        lims = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        cap = _join_capacity(n)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        while True:                                     # at most twice: the first call reports the exact total
+            keys = torch.empty(cap, dtype=torch.int64, device=dev)
+            nat.check(nat.lib.ivr_index_range_self_join_keys_device(self._handle(), radius, cap, lims.data_ptr(),
+                                                                    keys.data_ptr(), int(id_offset), st))
+            total = int(lims[n].item())
+            if total <= cap:
+                return lims, keys[:total]
+            cap = total
+
+    def range_cross_join_keys_tensor(self, other_rows, other_first_id: int, radius: float, other_is_lower: bool,
+                                     id_offset: int = 0):
+        """Every pair (row i of the search window, row j of ``other_rows``) whose inner product is strictly greater
+        than ``radius``, each pair scored once, as packed keys of GLOBAL ids: a window row's id is its stored row +
+        ``id_offset``, other row j's is ``other_first_id + j``.  ``other_rows``: CUDA float16 [n_other, dpad] on this
+        index's device (``rows_f16_tensor`` of another index).  ``other_is_lower``: the other rows' ids are below the
+        window's.  Returns (lims_self [n_self + 1], keys_self, lims_other [n_other + 1], keys_other), each row's hits
+        unsigned descending.  More than 2^31-1 hits in one call raise ``OverflowError``: split the other rows."""
+        import torch
+        radius = _radius(radius, "range_cross_join")
+        if other_rows.dim() != 2 or other_rows.dtype != torch.float16 or other_rows.shape[1] != self.dpad:
+            raise ValueError(f"other_rows: expected a float16 [n, {self.dpad}] tensor, got {other_rows.dtype} "
+                             f"{tuple(other_rows.shape)}")
+        other_rows = other_rows.contiguous()
+        _check_device(other_rows, self.device)
+        n, m = self._join_rows(), other_rows.shape[0]
+        dev = other_rows.device
+        lims = torch.zeros(n + m + 1, dtype=torch.int64, device=dev)
+        cap = _cross_capacity(n, m)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        while True:                                     # at most twice: the first call reports the exact total
+            keys = torch.empty(cap, dtype=torch.int64, device=dev)
+            nat.check(nat.lib.ivr_index_range_cross_join_keys_device(
+                self._handle(), other_rows.data_ptr(), m, int(other_first_id), int(bool(other_is_lower)), radius, cap,
+                lims.data_ptr(), keys.data_ptr(), int(id_offset), st))
+            total = int(lims[n + m].item())
+            if total <= cap:
+                break
+            if total > (1 << 31) - 1:
+                raise OverflowError(f"range_cross_join: {total} hits, more than one call holds (2^31-1)")
+            cap = total
+        mid = int(lims[n].item())
+        return lims[:n + 1], keys[:mid], lims[n:] - mid, keys[mid:total]
+
     def _selection(self, params):
         """The device selection of ``params.sel`` for this index's device and row count; None = unfiltered."""
         sel = getattr(params, "sel", None) if params is not None else None
@@ -680,6 +750,12 @@ def _join_capacity(n: int) -> int:
     pairs.  A near-duplicate radius finds a handful of copies per row, so one call usually suffices; a radius that
     finds more costs one retry with the exact total, not a pool sized for range search's 1024 hits per row."""
     return min(n * (n - 1), max(64 * n, 1 << 20), (1 << 31) - 1)
+
+
+def _cross_capacity(n: int, m: int) -> int:
+    """First guess of a cross join's pool size: 64 entries per row of either side (at least 1 M), never more than
+    the 2nm entries of every pair."""
+    return min(2 * n * m, max(64 * (n + m), 1 << 20), (1 << 31) - 1)
 
 
 def _is_cuda_tensor(x) -> bool:

@@ -51,6 +51,33 @@ def partition_rows(n_total: int, world_size: int, weights=None, align: int = 1) 
 
 
 MAX_SHARDED_ROWS = (1 << 32) - 1          # the exchange key holds a 32-bit global row id
+MAX_MERGE_PARTS = 64                      # runs one ivr_range_merge_keys_device call merges
+
+
+def join_schedule(bounds, rank: int) -> list:
+    """The work of rank ``rank`` in ``ShardedFlatIP.range_self_join`` (pure, the same answer on every rank).
+    ``bounds`` [world + 1]: the windows ``W_r = [bounds[r], bounds[r+1])``.  Returns tasks ``(a, b, peer, c, d)``:
+    score every pair of the rows ``[a, b)`` of this rank's window against the rows ``[c, d)`` of ``peer``'s.  Task 0 is
+    the diagonal (``peer == rank``, the self-join of ``W_rank``); then, for every step 1 <= delta with 2 delta < N,
+    the full block ``W_rank x W_(rank + delta) mod N``; and for an even N the block of the ranks r and r + N/2 split at
+    ``m = bounds[r] + n_r // 2``: rank r scores ``[bounds[r], m) x W_(r + N/2)``, rank r + N/2 scores
+    ``W_(r + N/2) x [m, bounds[r+1])``.  Every unordered pair of distinct rows is scored by exactly one rank, every
+    rank has N // 2 cross tasks, and with equal windows every rank scores the same number of pairs."""
+    b = [int(v) for v in np.asarray(bounds, dtype=np.int64)]
+    N = len(b) - 1
+    lo, hi = b[rank], b[rank + 1]
+    tasks = [(lo, hi, rank, lo, hi)]
+    for delta in range(1, (N + 1) // 2):
+        p = (rank + delta) % N
+        tasks.append((lo, hi, p, b[p], b[p + 1]))
+    if N % 2 == 0:
+        h = N // 2
+        if rank < h:
+            tasks.append((lo, lo + (hi - lo) // 2, rank + h, b[rank + h], b[rank + h + 1]))
+        else:
+            r = rank - h
+            tasks.append((lo, hi, r, b[r] + (b[r + 1] - b[r]) // 2, b[r + 1]))
+    return tasks
 
 
 def rebalance_bounds(bounds, times_ms, nominal, margin: int, gain: float = 0.7, align: int = 1024) -> np.ndarray:
@@ -230,7 +257,10 @@ class ShardedFlatIP:
     protocol: ``search_keys_tensor(q, k, id_offset, out)`` and ``merge(keys [world, nq, k], k)``; for
     ``range_search`` also ``range_search_tensor`` / ``range_search_keys_tensor(q, radius, id_offset)`` and
     ``range_merge(keys [world, stride], lims [world, nq + 1], total)``; for filtered searches the same calls with
-    ``params=`` holding a selector of stored rows, which must honour ``set_window``); by default they are the CUDA
+    ``params=`` holding a selector of stored rows, which must honour ``set_window``; for ``range_self_join``
+    ``dpad``, ``rows_f16_tensor(first, n)``, ``range_self_join_tensor(radius)``,
+    ``range_self_join_keys_tensor(radius, id_offset)`` and ``range_cross_join_keys_tensor(other_rows, other_first_id,
+    radius, other_is_lower, id_offset)``, the last two over the rows of the window); by default they are the CUDA
     index and the CUDA merge kernels and fail loudly without a GPU.
 
     FILTERED SEARCH (``params=SearchParameters(sel=...)``): ``sel`` selects GLOBAL ids.  Each rank searches the
@@ -559,6 +589,203 @@ class ShardedFlatIP:
                                    f"({self.world} x {stride} keys)")
             dist.all_gather_into_tensor(gathered.view(-1), mine, group=self.group)
         return self._range_merge(gathered, rows[:, :nq + 1].contiguous(), int(totals.sum()))
+
+    def range_self_join(self, radius: float, gather: bool = False):
+        """Exact range self-join over the rows of every rank: for every row, the other rows whose inner product with it
+        is strictly greater than ``radius``.  Returns tensors (lims int64 [n_local + 1], D float32, I int64 global ids)
+        for the rows of this rank's window (the current elastic boundaries, or its block), on the local index's
+        device: row i's hits are ``D[lims[i]:lims[i+1]]``, descending, ties -> lower id; the rows equal those of the
+        single-index ``range_self_join`` over all rows, bit for bit.  ``gather=True`` returns the whole result, every
+        row in global order, on every rank.  Collective: every rank must call it, with the same radius.
+
+        Each rank scores the tasks of ``join_schedule``: the self-join of its window, then one block of another rank's
+        rows per round, received through ``batch_isend_irecv`` and scored by the local cross join (the window's rows
+        against the received ones, each pair once).  The hits of the other side go back to their owner; every rank
+        merges the runs over its rows with ``range_merge``.  One all-gather before any row moves carries the radius and
+        the windows, one before any hit moves every run length and a status, so all ranks raise the same error when
+        one was called with another radius or one failed.  The join is not a timed search: ``balance_log``, the
+        search counter and the peer mailboxes are left alone; the window of the current boundaries is restored."""
+        import torch
+        import torch.distributed as dist
+        from .faiss_compat import _radius
+        radius = _radius(radius, "range_self_join")
+        if 1 + 2 * (self.world // 2) > MAX_MERGE_PARTS:  # the window's own join, then two runs per round
+            raise ValueError(f"range_self_join: {self.world} ranks give each rank {1 + 2 * (self.world // 2)} runs "
+                             f"to merge, more than the merge takes ({MAX_MERGE_PARTS})")
+        if self._bounds is not None:
+            self._set_window()
+        if self.world == 1:
+            lims, D, I = self.local.range_self_join_tensor(radius)
+            return lims, D, I + self.id_offset
+        dev = torch.device("cpu") if self.device is None else torch.device("cuda", self.device)
+        if self._bounds is not None:
+            lo, hi = int(self._bounds[self.rank]), int(self._bounds[self.rank + 1])
+        else:
+            lo, hi = self.id_offset, self.id_offset + self.local.ntotal
+        rbits = int(np.float32(radius).view(np.int32))
+        agree = torch.empty((self.world, 3), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(agree.view(-1), torch.tensor([rbits, lo, hi], dtype=torch.int64, device=dev),
+                                    group=self.group)
+        host = agree.cpu().numpy()
+        differ = np.nonzero(host[:, 0] != host[0, 0])[0]
+        if differ.size:
+            def rad(r):
+                return float(np.int32(host[r, 0]).view(np.float32))
+            raise ValueError(f"range_self_join: rank {int(differ[0])} was called with radius={rad(int(differ[0]))}, "
+                             f"rank 0 with radius={rad(0)}")
+        bounds = np.concatenate([host[:, 1], host[-1:, 2]])
+        if bounds[0] != 0 or bounds[-1] != self.ntotal_global or np.any(host[1:, 1] != host[:-1, 2]):
+            raise ValueError(f"range_self_join: the ranks' windows {host[:, 1:].tolist()} do not tile "
+                             f"[0, {self.ntotal_global})")
+        sched = [join_schedule(bounds, r) for r in range(self.world)]
+        mine, n_rounds = sched[self.rank], len(sched[self.rank]) - 1
+        parts, back, err = [], [], None                 # parts: runs (a, b, lims, keys) over this rank's rows [a, b)
+        try:
+            try:
+                self.local.set_window(lo - self.id_offset, hi - lo)
+                parts.append((lo, hi) + tuple(self.local.range_self_join_keys_tensor(radius, id_offset=self.id_offset)))
+            except Exception as e:                      # reported in the run-length all-gather
+                err = e
+            for k in range(n_rounds):
+                a, b, p, c, d = mine[k + 1]
+                needs = [(q,) + sched[q][k + 1][3:] for q in range(self.world) if sched[q][k + 1][2] == self.rank]
+                fail = self.world
+                try:
+                    recv = torch.empty((d - c, self.local.dpad), dtype=torch.float16, device=dev)
+                    sends = [(q, self.local.rows_f16_tensor(s - self.id_offset, e - s)) for q, s, e in needs]
+                except RuntimeError:                    # torch.OutOfMemoryError and the native errors included
+                    fail = self.rank
+                self._agree(fail, dev, "cannot allocate the row exchange buffers")
+                self._p2p([(dist.irecv, recv, p)] + [(dist.isend, t, q) for q, t in sends])
+                if err is not None:
+                    back.append((p, c, d, None, None))
+                    continue
+                try:
+                    self.local.set_window(a - self.id_offset, b - a)
+                    runs, lims_o, keys_o = self._cross_runs(recv, c, radius, c < a)
+                    parts += [(a, b, L, K) for L, K in runs]
+                    back.append((p, c, d, lims_o, keys_o))
+                except Exception as e:
+                    err = e
+                    back.append((p, c, d, None, None))
+                del recv, sends
+        finally:
+            if self._bounds is not None:
+                self._set_window()
+            else:
+                self.local.set_window()
+        # every run length before any hit moves: status, then the hits this rank sends back in each round
+        counts = [0 if err is None else 1] + [0 if L is None else int(K.numel()) for _, _, _, L, K in back]
+        allc = torch.empty((self.world, 1 + n_rounds), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(allc.view(-1), torch.tensor(counts, dtype=torch.int64, device=dev),
+                                    group=self.group)
+        allc = allc.cpu().numpy()
+        failed = np.nonzero(allc[:, 0])[0]
+        if failed.size:
+            raise RuntimeError(f"range_self_join failed on rank {int(failed[0])}") from err
+        for k in range(n_rounds):                       # the other side's runs go back to their owner
+            p, c, d, L, K = back[k]
+            needs = [(q,) + sched[q][k + 1][3:] for q in range(self.world) if sched[q][k + 1][2] == self.rank]
+            fail, recvs = self.world, []
+            try:
+                recvs = [(q, s, e, torch.empty(e - s + 1 + int(allc[q, 1 + k]), dtype=torch.int64, device=dev))
+                         for q, s, e in needs]
+                payload = torch.cat([L, K])
+            except RuntimeError:
+                fail = self.rank
+            self._agree(fail, dev, "cannot allocate the hit exchange buffers")
+            self._p2p([(dist.isend, payload, p)] + [(dist.irecv, t, q) for q, _, _, t in recvs])
+            parts += [(s, e, t[:e - s + 1], t[e - s + 1:]) for _, s, e, t in recvs]
+        # the merge can fail on one rank only (memory, or more runs than the merge takes after overflow splits):
+        # every rank learns it before any rank leaves or enters the gather
+        fail, err = self.world, None
+        try:
+            if len(parts) > MAX_MERGE_PARTS:
+                raise RuntimeError(f"{len(parts)} runs, more than the merge takes ({MAX_MERGE_PARTS})")
+            lims, D, I = self._merge_runs(parts, lo, hi, dev)
+        except RuntimeError as e:                       # torch.OutOfMemoryError and the native errors included
+            fail, err = self.rank, e
+        self._agree(fail, dev, "could not merge its runs", err)
+        return self._gather_join(lims, D, I, dev) if gather else (lims, D, I)
+
+    def _cross_runs(self, other, first: int, radius: float, lower: bool):
+        """The local cross join of the window against ``other`` (rows of global ids ``first + j``): (runs over the
+        window, lims over the other rows, their keys).  A call that would hold more than 2^31-1 hits is split over
+        halves of the other rows; each half adds one run over the window, and the halves' runs over the other rows
+        concatenate into one."""
+        try:
+            ls, ks, lo_, ko = self.local.range_cross_join_keys_tensor(other, first, radius, lower,
+                                                                      id_offset=self.id_offset)
+            return [(ls, ks)], lo_, ko
+        except OverflowError:
+            m = other.shape[0]
+            if m < 2:
+                raise
+            h = m // 2
+            r1, l1, k1 = self._cross_runs(other[:h], first, radius, lower)
+            r2, l2, k2 = self._cross_runs(other[h:], first + h, radius, lower)
+            import torch
+            return r1 + r2, torch.cat([l1[:-1], l2 + l1[-1]]), torch.cat([k1, k2])
+
+    def _agree(self, fail: int, dev, what: str, err=None) -> None:
+        """All ranks learn whether any failed a local step (``fail`` = this rank, else ``world``) and raise together,
+        naming the lowest such rank."""
+        import torch
+        import torch.distributed as dist
+        flag = torch.tensor([fail], dtype=torch.int64, device=dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
+        if int(flag.item()) < self.world:
+            raise RuntimeError(f"range_self_join: rank {int(flag.item())} {what}") from err
+
+    def _p2p(self, ops) -> None:
+        """One batch of point-to-point transfers (op, tensor, group rank); empty tensors are skipped (both sides
+        know every size)."""
+        import torch.distributed as dist
+        ops = [dist.P2POp(op, t, p if self.group is None else dist.get_global_rank(self.group, p), self.group)
+               for op, t, p in ops if t.numel() > 0]
+        if ops:
+            for w in dist.batch_isend_irecv(ops):
+                w.wait()
+
+    def _merge_runs(self, parts, lo: int, hi: int, dev):
+        """``range_merge`` of runs over sub-ranges of the rows [lo, hi): each run's lims embedded in [n + 1] entries,
+        zeros before its rows and its total after them, its keys padded to the longest run."""
+        import torch
+        n = hi - lo
+        stride = max([int(K.numel()) for _, _, _, K in parts] + [0])
+        keys_parts = torch.zeros((len(parts), stride), dtype=torch.int64, device=dev)
+        lims_parts = torch.zeros((len(parts), n + 1), dtype=torch.int64, device=dev)
+        total = 0
+        for i, (a, b, L, K) in enumerate(parts):
+            keys_parts[i, :K.numel()] = K
+            lims_parts[i, a - lo:b - lo + 1] = L
+            lims_parts[i, b - lo + 1:] = int(K.numel())
+            total += int(K.numel())
+        return self._range_merge(keys_parts, lims_parts, total)
+
+    def _gather_join(self, lims, D, I, dev):
+        """Every rank's (lims, D, I) on every rank, in rank (= global row) order."""
+        import torch
+        import torch.distributed as dist
+        sizes = torch.empty((self.world, 2), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(sizes.view(-1), torch.tensor([lims.numel() - 1, D.numel()], dtype=torch.int64,
+                                                                 device=dev), group=self.group)
+        sizes = sizes.cpu().numpy()
+        rmax, hmax = int(sizes[:, 0].max()) + 1, int(sizes[:, 1].max())
+        out = []
+        for t, m in ((lims, rmax), (D, hmax), (I, hmax)):
+            buf = torch.zeros(m, dtype=t.dtype, device=dev)
+            buf[:t.numel()] = t
+            allb = torch.empty((self.world, m), dtype=t.dtype, device=dev)
+            dist.all_gather_into_tensor(allb.view(-1), buf, group=self.group)
+            out.append(allb)
+        L_all, D_all, I_all = out
+        base = np.concatenate([[0], np.cumsum(sizes[:, 1])])
+        lims_g = torch.cat([L_all[r, :int(sizes[r, 0])] + int(base[r]) for r in range(self.world)] +
+                           [torch.tensor([int(base[-1])], dtype=torch.int64, device=dev)])
+        D_g = torch.cat([D_all[r, :int(sizes[r, 1])] for r in range(self.world)])
+        I_g = torch.cat([I_all[r, :int(sizes[r, 1])] for r in range(self.world)])
+        return lims_g, D_g, I_g
 
     # ---- peer-memory exchange (csrc/exchange.cu) ---------------------------
     def _ensure_mailbox(self, n_entries: int, device) -> bool:
